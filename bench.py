@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — BASELINE.json's metric on BASELINE.json's configs, measured on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload cfg2] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload cfg2] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
 
 Workloads (config.workload; SURVEY.md §8d).  The default, and the one the driver runs, is cfg2:
@@ -79,6 +79,47 @@ def _golden(name):
 
 def sha(b):
     return hashlib.sha256(b).hexdigest()
+
+
+# ------------------------------------------------------------------------------------------ --dump-outputs
+# What the timed path returned in its last step, written so that two builds run with the same arguments can be compared
+# output for output.  A chunk holds hundreds of MB, so each dumped chunk contributes its whole .alc header and a fixed,
+# seeded sample of its payload and decoded bytes; the samples depend only on the chunk, never on the batch size.
+DUMP_SEED = 20261020
+DUMP_SAMPLES = 1 << 19                  # decoded bytes per dumped chunk (cfg4: decoded samples per channel)
+DUMP_PAYLOAD_SAMPLES = 1 << 17          # payload bytes per dumped chunk (cfg4: per channel stream)
+DUMP_MAX_BYTES = 64 * 10**6
+ALC_HEADER_BYTES = 3138
+
+
+def dump_chunk_ids(n):
+    """Chunks 0-15 and every power of two below n: the same rows whatever batch size free memory allows."""
+    return sorted(set(range(min(n, 16))) | {1 << k for k in range(n.bit_length()) if (1 << k) < n})
+
+
+def dump_positions(n, count, key):
+    """`count` sorted positions in [0, n), drawn with replacement from a generator seeded by DUMP_SEED and `key`."""
+    import numpy as np
+    return np.sort(np.random.default_rng([DUMP_SEED, key]).integers(0, n, count))
+
+
+def payload_sample(blob, key):
+    """DUMP_PAYLOAD_SAMPLES bytes of an encoded stream at seeded positions, as float32."""
+    import numpy as np
+    a = np.frombuffer(blob, dtype=np.uint8)
+    return a[dump_positions(a.size, DUMP_PAYLOAD_SAMPLES, key)].astype(np.float32)
+
+
+def write_dump(out_dir, arrays):
+    """One DIR/<name>.npy per array (float32 or float64), DUMP_MAX_BYTES at most in all."""
+    import numpy as np
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_MAX_BYTES:
+        raise RuntimeError(f"--dump-outputs: {total} bytes exceed the {DUMP_MAX_BYTES}-byte limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 # ------------------------------------------------------------------------------------------ clocks
@@ -223,7 +264,14 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--verbose", action="store_true")
     ap.add_argument("--lib", default=None, help="experiment build of libalice_codec (debugging aid)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last step returned (rank 0's chunks: .alc lengths and "
+                         "headers, seeded samples of the payloads and of the decoded RGB) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl b200)")
     if args.warmup < 3:
         args.warmup = 3                      # timing rule: at least 3 warm-up steps
     wl = WORKLOADS[args.workload]
@@ -376,6 +424,17 @@ def main():
     if rank == 0 and g:
         alc = batch.get_chunk(0).to_bytes()
         bit_exact = (sha(alc) == g["sha256_alc"] and sha(bufs[1].cpu().numpy().tobytes()) == g["sha256_decoded"])
+    if rank == 0 and args.dump_outputs:
+        ids = dump_chunk_ids(B)
+        alcs = [batch.get_chunk(i).to_bytes() for i in ids]
+        decoded = [bufs[i + 1][torch.from_numpy(dump_positions(rgb_bytes, DUMP_SAMPLES, i)).cuda()] for i in ids]
+        write_dump(args.dump_outputs, {
+            "chunk_index": np.array(ids, dtype=np.float64),
+            "alc_len": np.array([len(a) for a in alcs], dtype=np.float64),
+            "alc_header": np.stack([np.frombuffer(a[:ALC_HEADER_BYTES], dtype=np.uint8) for a in alcs]).astype(np.float32),
+            "alc_payload_sample": np.stack([payload_sample(a[ALC_HEADER_BYTES:], i) for i, a in zip(ids, alcs)]),
+            "decoded_rgb_sample": torch.stack(decoded).float().cpu().numpy()})
+        del alcs, decoded
 
     # ---- rooflines, from the library's own CUDA events on the launch stream (averaged over the timed steps)
     peak, peak_src = _peaks()

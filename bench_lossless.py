@@ -57,6 +57,15 @@ def main(args, wl):
     ms_step = ev0.elapsed_time(ev1) / args.steps
     stage /= args.steps * nb                 # per frame set
     sampler.join(timeout=2)
+    if args.dump_outputs:                    # what the last step returned for its last frame set (nb - 1)
+        streams = [ls.stream(c) for c in range(3)]
+        inverse = ls.fetch("inverse")
+        B.write_dump(args.dump_outputs, {
+            "stream_len": np.array([len(s) for s in streams], dtype=np.float64),
+            "histogram": ls.fetch("hist").astype(np.float64),
+            "stream_sample": np.stack([B.payload_sample(s, c) for c, s in enumerate(streams)]),
+            "inverse_sample": np.stack([inverse[c][B.dump_positions(n, B.DUMP_SAMPLES, c)] for c in range(3)]).astype(np.float32)})
+        del streams, inverse
     # correctness of what was just timed: digests of every stage of set 0 against the oracle's (tests/golden)
     g = B._golden(wl["golden"])
     ls.encode_device(d_rgb[0].data_ptr())

@@ -77,12 +77,30 @@ def lossless_case(w, h, f, seed):
 
 
 LOSSLESS_CASES = {"cfg4_lossless_1080p64": (1920, 1080, 64, O.SEED)}
+BENCH_DUMP_OUT = os.path.join(os.path.dirname(OUT), "bench_dump_cfg2_chunk0.npz")
+
+
+def bench_dump_case():
+    """What `bench.py --dump-outputs` writes for chunk 0 of its default workload (cfg2), from the oracle, as uint8:
+    the .alc header, and the payload and decoded RGB bytes at the bench's seeded sample positions."""
+    import bench
+    kind, w, h, f, q, wv, seed = CASES["cfg2_cdf97_q80_1080p64"]
+    alc = O.encode(O.generate(kind, w, h, f, seed), w, h, f, q, wv)
+    dec = O.decode(alc)
+    payload = np.frombuffer(alc[bench.ALC_HEADER_BYTES:], dtype=np.uint8)
+    np.savez_compressed(BENCH_DUMP_OUT, alc_len=np.array([len(alc)]),
+                        alc_header=np.frombuffer(alc[:bench.ALC_HEADER_BYTES], dtype=np.uint8),
+                        alc_payload_sample=payload[bench.dump_positions(payload.size, bench.DUMP_PAYLOAD_SAMPLES, 0)],
+                        decoded_rgb_sample=dec[bench.dump_positions(dec.size, bench.DUMP_SAMPLES, 0)])
 
 
 def main():
-    names = sys.argv[1:] or list(CASES) + list(LOSSLESS_CASES)
+    names = sys.argv[1:] or list(CASES) + list(LOSSLESS_CASES) + ["bench_dump"]
     res = json.load(open(OUT)) if os.path.exists(OUT) else {}
     for name in names:
+        if name == "bench_dump":
+            bench_dump_case()
+            continue
         if name in LOSSLESS_CASES:
             res[name] = lossless_case(*LOSSLESS_CASES[name])
             print(name, res[name]["stream_lens"], res[name]["oracle_seconds"], flush=True)

@@ -6,6 +6,7 @@ bit-exact equality at every stage: wavelet coefficients, symbol planes, histogra
 streams, .alc bytes and decoded RGB (the path is integer/byte work throughout).
 """
 import hashlib
+import os
 
 import numpy as np
 
@@ -14,6 +15,13 @@ from __graft_entry__ import load_package
 
 pkg = load_package()
 WV = {0: "cdf53", 1: "cdf97", 2: "haar"}
+EMUL_BUILD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "emul", "_build")
+
+
+def device_of(api):
+    """torch device of the buffers that `api`'s device-pointer calls take.  The emulator builds (tests/emul/_build) run
+    their kernels on the host and treat host memory as device memory, also on a machine that has a GPU."""
+    return "cpu" if os.path.abspath(api.path).startswith(EMUL_BUILD + os.sep) else "cuda"
 
 
 def check_encode_decode(api, kind, w, h, f, quality, wavelet, seed=O.SEED, stages=True):
@@ -423,7 +431,7 @@ def check_shared_workspace_batch(api, shapes=((20, 12, 6), (21, 13, 5)), n=3):
             ws = batch.workspace_bytes()
             pw, ph, pf = O.padded_dims(w, h, f)
             assert ws == 3 * pw * ph * pf
-            dev = "cuda" if torch.cuda.is_available() else "cpu"        # the emulator treats host memory as device memory
+            dev = device_of(api)
             d_in = [torch.zeros(max(ws, r.size), dtype=torch.uint8, device=dev) for r in rgbs]
             for t, r in zip(d_in, rgbs):
                 t[:r.size] = torch.from_numpy(r).to(dev)
@@ -462,7 +470,7 @@ def check_payload_arena(api, w=48, h=20, f=8, n=4):
     (k_estimate_stream_bytes): with a budget just above the real payload everything fits, with a budget far below it the
     streams that find no room go through the worst-case retry -- the output is the oracle's either way."""
     import torch
-    dev = "cuda" if torch.cuda.is_available() else "cpu"        # the emulator treats host memory as device memory
+    dev = device_of(api)
     rgbs = [O.generate(O.G2 if i == 1 else O.G1, w, h, f, O.SEED + i) for i in range(n)]
     for q, wv in ((80, 1), (100, 0)):
         refs = [O.encode(r, w, h, f, q, wv) for r in rgbs]
@@ -513,7 +521,7 @@ def lossless_oracle(rgb, w, h, f):
 def check_lossless_set(api, shapes=((16, 6, 4), (21, 9, 3), (128, 8, 6))):
     """alice_codec_lossless_* against the oracle's stages (fast 2-D kernels and the step-by-step path)"""
     import torch
-    dev = "cuda" if torch.cuda.is_available() else "cpu"        # the emulator treats host memory as device memory
+    dev = device_of(api)
     for (w, h, f) in shapes:
         rgb = O.generate(O.G1, w, h, f)
         ref = lossless_oracle(rgb, w, h, f)
@@ -563,7 +571,7 @@ def check_shifted_in_place(api, shapes=((20, 12, 6), (96, 4, 64)), n=3):
     bufs[i] (the consumed input of chunk i - 1) and its decode lands back in bufs[i + 1] (the back-end runs the chunks in
     descending order).  Both fused kernels run in this plan (no buffer is read and written by the same launch)."""
     import torch
-    dev = "cuda" if torch.cuda.is_available() else "cpu"        # the emulator treats host memory as device memory
+    dev = device_of(api)
     for (w, h, f) in shapes:
         for q, wv in ((80, 1), (90, 0), (75, 2)):
             rgbs = [O.generate(O.G1, w, h, f, O.SEED + i) for i in range(n)]
@@ -591,8 +599,8 @@ def check_stream_device(api, shapes=((20, 12, 6), (96, 4, 64)), n=4):
     (submit_device) and ONE on the way out (decode_next_device); what stays per chunk is its symbol planes and payload.
     The decoded chunk is copied out on the same stream before the buffer is handed to the next chunk."""
     import torch
-    cuda = torch.cuda.is_available()
-    dev = "cuda" if cuda else "cpu"                            # the emulator treats host memory as device memory
+    dev = device_of(api)
+    cuda = dev == "cuda"
     for (w, h, f) in shapes:
         for q, wv, small in ((80, 1, False), (90, 0, True), (75, 2, False)):
             rgbs = [O.generate(O.G1, w, h, f, O.SEED + i) for i in range(n)]
