@@ -7,8 +7,9 @@ interface on top of that C ABI.  The directory name carries a hyphen, so import 
 """
 from . import _capi, sharding  # noqa: F401
 from .api import (Api, ChunkBatch, CodecError, EncodedChunk, FrameDecoder, FrameEncoder, LosslessSet, ReferenceAbi,  # noqa: F401
-                  SUBBANDS, WAVELET_BYTES, WAVELET_NAMES, default_api, rgb_to_ycocg_r_numpy, version,
-                  ycocg_r_to_rgb_numpy)
+                  SUBBANDS, WAVELET_BYTES, WAVELET_NAMES, default_api, quality_for_step, quality_to_step,
+                  rgb_to_ycocg_r_numpy, version, ycocg_r_to_rgb_numpy)
 
 __all__ = ["Api", "ChunkBatch", "CodecError", "EncodedChunk", "FrameDecoder", "FrameEncoder", "LosslessSet", "ReferenceAbi",
-           "default_api", "WAVELET_NAMES", "WAVELET_BYTES", "SUBBANDS", "rgb_to_ycocg_r_numpy", "ycocg_r_to_rgb_numpy", "version"]
+           "default_api", "WAVELET_NAMES", "WAVELET_BYTES", "SUBBANDS", "rgb_to_ycocg_r_numpy", "ycocg_r_to_rgb_numpy", "version",
+           "quality_to_step", "quality_for_step"]

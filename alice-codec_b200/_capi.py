@@ -112,6 +112,10 @@ SIGNATURES = {
     "alice_codec_batch_get_chunk": (vp, [vp, u32]),
     "alice_codec_batch_timings": (cint, [vp, C.POINTER(C.c_float)]),
     "alice_codec_batch_device_bytes": (u64, [vp]),
+    "alice_codec_rate_curve": (cint, [u8, u8p, u64, u32, u32, u32, u64p, u32p]),
+    "alice_codec_rate_curve_device": (cint, [u8, vp, u32, u32, u32, u64p, u32p, vp]),
+    "alice_codec_encode_to_size": (vp, [u8, u8p, u64, u32, u32, u32, u64, u8p]),
+    "alice_codec_batch_encode_host_to_size": (cint, [vp, C.POINTER(vp), u32, u64, C.POINTER(vp), u8p]),
     "alice_codec_synth_rgb_device": (cint, [cint, u32, u32, u32, u32, vp, vp]),
     "alice_codec_pinned_alloc": (vp, [u64]),
     "alice_codec_pinned_free": (None, [vp]),

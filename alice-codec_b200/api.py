@@ -33,6 +33,27 @@ class CodecError(ValueError):
         super().__init__(f"{self.kind}: {message}" if message else self.kind)
 
 
+RATE_STEPS = 64
+UINT64_MAX = (1 << 64) - 1
+
+
+def quality_to_step(quality: int) -> int:
+    """pipeline.rs:456-457: the quantiser step (1..64) of a quality byte"""
+    q = min(int(quality), 100)
+    return max(1, 64 - q * 63 // 100)
+
+
+def quality_for_step(step: int) -> int:
+    """the largest quality in 0..=100 whose quantiser step is `step` (1..64)"""
+    return max(q for q in range(101) if quality_to_step(q) == step)
+
+
+def _curve_dict(sizes):
+    """{quality: predicted .alc bytes} over the 64 steps (highest quality first); None where the reference aborts"""
+    return {quality_for_step(s): (None if int(sizes[s - 1]) == UINT64_MAX else int(sizes[s - 1]))
+            for s in range(1, RATE_STEPS + 1)}
+
+
 def _wavelet_byte(wavelet) -> int:
     if isinstance(wavelet, str):
         if wavelet not in WAVELET_NAMES:
@@ -436,6 +457,40 @@ class FrameEncoder:
             self._api._raise()
         return EncodedChunk(h, self._api), coeffs, syms
 
+    def rate_curve(self, rgb_frames, width: int, height: int, frames: int, with_hist: bool = False):
+        """Predicted .alc size of the chunk at every quantiser step, before any rANS work: {quality: bytes}, one entry per
+        step (the largest quality with that step), each an upper bound on len(encode at that quality).to_bytes(); None
+        where the reference aborts.  The encoder's wavelet is used, its quality is not.  with_hist=True also returns the
+        symbol histograms, uint32 [64][3][256] (row step - 1): what the headers of those encodes hold."""
+        a, pa = _u8(rgb_frames)
+        sizes = np.zeros(RATE_STEPS, np.uint64)
+        hist = np.zeros((RATE_STEPS, 3, 256), np.uint32) if with_hist else None
+        self._api._chk(self._api.lib.alice_codec_rate_curve(
+            self.wavelet, pa, a.size, width, height, frames, sizes.ctypes.data_as(_capi.u64p),
+            hist.ctypes.data_as(_capi.u32p) if with_hist else None))
+        return (_curve_dict(sizes), hist) if with_hist else _curve_dict(sizes)
+
+    def rate_curve_device(self, d_rgb: int, width: int, height: int, frames: int, stream: int = 0, with_hist: bool = False):
+        """rate_curve for RGB in device memory (raw device pointer); waits for the work enqueued on `stream` first"""
+        sizes = np.zeros(RATE_STEPS, np.uint64)
+        hist = np.zeros((RATE_STEPS, 3, 256), np.uint32) if with_hist else None
+        self._api._chk(self._api.lib.alice_codec_rate_curve_device(
+            self.wavelet, C.c_void_p(int(d_rgb)), width, height, frames, sizes.ctypes.data_as(_capi.u64p),
+            hist.ctypes.data_as(_capi.u32p) if with_hist else None, C.c_void_p(stream)))
+        return (_curve_dict(sizes), hist) if with_hist else _curve_dict(sizes)
+
+    def encode_to_size(self, rgb_frames, width: int, height: int, frames: int, max_bytes: int):
+        """The chunk at the highest quality whose .alc (to_bytes) is at most max_bytes: (EncodedChunk, quality), the
+        chunk byte-identical to FrameEncoder(quality, wavelet).encode.  The encoder's quality is not used.  Raises
+        CodecError InvalidBufferSize if no quality fits."""
+        a, pa = _u8(rgb_frames)
+        q = C.c_uint8()
+        h = self._api.lib.alice_codec_encode_to_size(self.wavelet, pa, a.size, width, height, frames, int(max_bytes),
+                                                     C.byref(q))
+        if not h:
+            self._api._raise()
+        return EncodedChunk(h, self._api), q.value
+
 
 class FrameDecoder:
     """python.rs:443-482: FrameDecoder().decode(chunk) -> 1-D uint8 RGB array."""
@@ -564,6 +619,17 @@ class ChunkBatch:
         out = (C.c_void_p * n)()
         self._api._chk(self._api.lib.alice_codec_batch_encode_host(self._h, arr, n, out))
         return [EncodedChunk(C.c_void_p(out[i]), self._api) for i in range(n)]
+
+    def encode_host_to_size(self, h_rgb_ptrs, max_bytes: int):
+        """encode_host with every chunk at the highest quality whose .alc fits max_bytes: (chunks, qualities).  The
+        batch's quality is not used."""
+        n = len(h_rgb_ptrs)
+        arr = self._ptr_array(h_rgb_ptrs)
+        out = (C.c_void_p * n)()
+        q = np.zeros(max(n, 1), np.uint8)
+        self._api._chk(self._api.lib.alice_codec_batch_encode_host_to_size(self._h, arr, n, int(max_bytes), out,
+                                                                           q.ctypes.data_as(_capi.u8p)))
+        return [EncodedChunk(C.c_void_p(out[i]), self._api) for i in range(n)], [int(x) for x in q[:n]]
 
     def submit_host(self, i, h_rgb_ptr):
         """chunk-at-a-time encode: enqueue the copy and the front-end of chunk i (submit 0, 1, ... in order)"""

@@ -16,7 +16,7 @@ from concurrent.futures import ThreadPoolExecutor
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
 CSRC = os.path.join(HERE, "csrc")
-SOURCES = ["k_forward.cu", "k_fwd_fused.cu", "k_inv_fused.cu", "k_inverse.cu", "k_rans.cu", "k_generic.cu", "k_wavelet_i32.cu", "k_rdo.cu", "k_synth.cu", "engine.cu", "lossless.cu", "capi.cu"]
+SOURCES = ["k_forward.cu", "k_fwd_fused.cu", "k_inv_fused.cu", "k_inverse.cu", "k_rans.cu", "k_generic.cu", "k_wavelet_i32.cu", "k_rdo.cu", "k_rate.cu", "k_synth.cu", "engine.cu", "lossless.cu", "capi.cu"]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "-Xcompiler", "-fPIC",
               "-Xcompiler", "-fvisibility=hidden", "--expt-relaxed-constexpr", "-cudart", "static"]

@@ -1,7 +1,9 @@
 """`alice-codec encode | decode | info` over the C ABI — same sub-commands, flags, messages and exit codes as the
 reference's CLI (src/bin/main.rs:36-196), plus multi-chunk streams (SURVEY.md §8f-1): with --chunk-frames N the input
 is cut into N-frame chunks, the chunks run as one batch (all rANS streams concurrently) and the output is the
-concatenation of self-delimiting .alc blobs; `decode` and `info` accept such streams.
+concatenation of self-delimiting .alc blobs; `decode` and `info` accept such streams.  With --max-bytes N every chunk
+(the whole input without --chunk-frames) is encoded at the highest quality whose .alc blob is at most N bytes; the chunk
+is byte-identical to an encode at that quality, and -q is not used.
 
     python -m alice_codec_b200.cli encode raw.rgb -W 1920 -H 1080 -f 64 -q 90 -w cdf53 -o out.alc
     (from the repo root: python alice-codec_b200/cli.py ...)
@@ -30,6 +32,16 @@ def cmd_encode(a) -> None:
         raise ValueError(f"unknown wavelet '{a.wavelet}'; expected cdf53, cdf97, or haar")     # main.rs:74-83
     rgb = np.fromfile(a.input, dtype=np.uint8)
     enc = pkg.FrameEncoder(a.quality, a.wavelet)
+    budget = a.max_bytes
+    qualities = []                                  # --max-bytes: the quality chosen for each chunk
+
+    def one(part, nf):
+        if budget is None:
+            return enc.encode(part, a.width, a.height, nf).to_bytes()
+        chunk, q = enc.encode_to_size(part, a.width, a.height, nf, budget)
+        qualities.append(q)
+        return chunk.to_bytes()
+
     if a.chunk_frames and a.frames > a.chunk_frames:
         per = a.width * a.height * 3
         if rgb.size != per * a.frames:
@@ -41,21 +53,28 @@ def cmd_encode(a) -> None:
             batch = pkg.ChunkBatch(a.quality, a.wavelet, a.width, a.height, a.chunk_frames, n_full)
             cb = per * a.chunk_frames
             parts = [np.ascontiguousarray(rgb[i * cb:(i + 1) * cb]) for i in range(n_full)]
-            blobs = [c.to_bytes() for c in batch.encode_host([p.ctypes.data for p in parts])]
+            if budget is None:
+                chunks = batch.encode_host([p.ctypes.data for p in parts])
+            else:
+                chunks, qs = batch.encode_host_to_size([p.ctypes.data for p in parts], budget)
+                qualities.extend(qs)
+            blobs = [c.to_bytes() for c in chunks]
             batch.close()
         else:
             n_full = 0
         for t0 in range(n_full * a.chunk_frames, a.frames, a.chunk_frames):
             nf = min(a.chunk_frames, a.frames - t0)
-            blobs.append(enc.encode(rgb[t0 * per:(t0 + nf) * per], a.width, a.height, nf).to_bytes())
+            blobs.append(one(rgb[t0 * per:(t0 + nf) * per], nf))
         data = sharding.concat_stream(blobs)
     else:
-        data = enc.encode(rgb, a.width, a.height, a.frames).to_bytes()
+        data = one(rgb, a.frames)
     with open(a.output, "wb") as f:
         f.write(data)
     ratio = len(data) / rgb.size if rgb.size else 0.0
+    setting = (f"quality={a.quality}" if budget is None else
+               f"max-bytes={budget} per chunk, quality={','.join(str(q) for q in qualities)}")
     sys.stderr.write(f"encoded {a.width}x{a.height}x{a.frames} ({rgb.size} bytes) -> {len(data)} bytes "
-                     f"({ratio * 100:.1f}% ratio, quality={a.quality}, wavelet={a.wavelet})\n")
+                     f"({ratio * 100:.1f}% ratio, {setting}, wavelet={a.wavelet})\n")
 
 
 def _blobs(data: bytes):
@@ -118,6 +137,8 @@ def main(argv=None) -> int:
     e.add_argument("-q", "--quality", type=int, default=90)
     e.add_argument("-w", "--wavelet", default="cdf53")
     e.add_argument("--chunk-frames", type=int, default=0, help="cut the input into chunks of this many frames (0 = one chunk)")
+    e.add_argument("--max-bytes", type=int, default=None,
+                   help="byte budget per chunk: encode each chunk at the highest quality whose .alc fits (-q is not used)")
     d = sub.add_parser("decode", help="Decode an .alc bitstream back to raw RGB")
     d.add_argument("input")
     d.add_argument("-o", "--output", required=True)

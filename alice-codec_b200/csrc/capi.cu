@@ -178,6 +178,129 @@ EncodedChunk *encode_impl(const FrameEncoder *enc, const uint8_t *rgb, uint64_t 
     return out;
 }
 
+// ------------------------------------------------------------------------------ rate control
+constexpr uint64_t kAlcHeaderBytes = kFixedHeaderBytes + 3 * kChannelHeaderBytes;   // 3138
+
+// the largest quality in 0..=100 whose step is s (every step has one: 63q/100 takes every integer 0..63)
+uint8_t quality_for_step(int s) {
+    for (int q = 100; q >= 0; q--)
+        if (quality_to_step((uint8_t)q) == s) return (uint8_t)q;
+    return 100;
+}
+
+// the smallest step >= first whose prediction fits max_bytes (the highest quality; sizes are not assumed monotone in the
+// step), 0 if there is none
+int pick_step(const uint64_t pred[kRateSteps], uint64_t max_bytes, int first) {
+    for (int s = first; s <= kRateSteps; s++)
+        if (pred[s - 1] != UINT64_MAX && pred[s - 1] <= max_bytes) return s;
+    return 0;
+}
+
+void set_no_fit_error(const uint64_t pred[kRateSteps], uint64_t max_bytes) {
+    uint64_t best = UINT64_MAX;
+    for (int i = 0; i < kRateSteps; i++) best = std::min(best, pred[i]);
+    set_error(kErrBufferSize, "no quality fits " + std::to_string(max_bytes) + " bytes: the smallest predicted size is " +
+                                  (best == UINT64_MAX ? std::string("unbounded (the reference aborts at every step)")
+                                                      : std::to_string(best) + " bytes"));
+}
+
+// Predicted .alc size of every step for one chunk whose RGB is on the host (device == false) or the device.
+int rate_curve_impl(uint8_t wavelet, const uint8_t *rgb, bool device, uint64_t rgb_len, uint32_t w, uint32_t h,
+                    uint32_t f, uint64_t *bytes64, uint32_t *hist_out, cudaStream_t user_st) {
+    set_error(0, "");
+    if (!bytes64) { set_error(kErrNull, "null output"); return kErrNull; }
+    if (wavelet > 2) { set_error(kErrBitstream, "unknown wavelet type byte"); return kErrBitstream; }
+    Dims d;
+    bool empty;
+    int rc = validate_encode(rgb_len, w, h, f, d, empty);
+    if (rc) return rc;
+    if (empty) {   // the empty chunk (three default headers) at every step
+        for (int i = 0; i < kRateSteps; i++) bytes64[i] = kAlcHeaderBytes;
+        if (hist_out) memset(hist_out, 0, (size_t)kRateSteps * 3 * 256 * sizeof(uint32_t));
+        return kOk;
+    }
+    if (!rgb) { set_error(kErrNull, "null argument"); return kErrNull; }
+    if (!cuda_ready()) return kErrCuda;
+    Engine *e = acquire_engine(d);
+    if (!e) return kErrCuda;
+    do {
+        const uint8_t *src = rgb;
+        if (device) {   // the engine's stream waits for the caller's work on the input
+            cudaEvent_t ev = nullptr;
+            if (cudaEventCreateWithFlags(&ev, cudaEventDisableTiming) != cudaSuccess) { cudaGetLastError(); set_error(kErrCuda, "event creation failed"); rc = kErrCuda; break; }
+            cudaError_t ce = cudaEventRecord(ev, user_st);
+            if (ce == cudaSuccess) ce = cudaStreamWaitEvent(e->stream(), ev, 0);
+            cudaEventDestroy(ev);
+            if (ce != cudaSuccess) { cudaGetLastError(); set_error(kErrCuda, "stream ordering failed"); rc = kErrCuda; break; }
+        } else {
+            uint8_t *stage = e->rgb_stage(0);
+            if (!stage) { rc = kErrCuda; break; }
+            if (cudaMemcpyAsync(stage, rgb, (size_t)rgb_len, cudaMemcpyHostToDevice, e->stream()) != cudaSuccess) {
+                set_error(kErrCuda, "H2D copy failed"); rc = kErrCuda; break;
+            }
+            src = stage;
+        }
+        rc = e->rate_curve(wavelet, src, bytes64, hist_out);
+    } while (0);
+    release_engine(e);
+    return rc;
+}
+
+// The highest quality whose chunk fits max_bytes, trying steps from first_step on: the rate curve picks the step, one
+// real encode checks it (an encode larger than its prediction, which the bound rules out, moves on to the next step).
+EncodedChunk *encode_to_size_impl(uint8_t wavelet, const uint8_t *rgb, uint64_t rgb_len, uint32_t w, uint32_t h,
+                                  uint32_t f, uint64_t max_bytes, int first_step, uint8_t *quality_out) {
+    set_error(0, "");
+    if (!rgb || !quality_out) { set_error(kErrNull, "null argument"); return nullptr; }
+    if (wavelet > 2) { set_error(kErrBitstream, "unknown wavelet type byte"); return nullptr; }
+    Dims d;
+    bool empty;
+    if (validate_encode(rgb_len, w, h, f, d, empty)) return nullptr;
+    if (empty) {
+        uint64_t pred[kRateSteps];
+        for (int i = 0; i < kRateSteps; i++) pred[i] = kAlcHeaderBytes;
+        if (max_bytes < kAlcHeaderBytes) { set_no_fit_error(pred, max_bytes); return nullptr; }
+        EncodedChunk *out = new (std::nothrow) EncodedChunk();
+        if (!out) return nullptr;
+        out->c.width = w; out->c.height = h; out->c.frames = f;
+        out->c.wavelet = wavelet;
+        *quality_out = 100;
+        return out;
+    }
+    if (!cuda_ready()) return nullptr;
+    Engine *e = acquire_engine(d);
+    if (!e) return nullptr;
+    EncodedChunk *out = nullptr;
+    do {
+        uint8_t *stage = e->rgb_stage(0);
+        if (!stage) break;
+        if (cudaMemcpyAsync(stage, rgb, (size_t)rgb_len, cudaMemcpyHostToDevice, e->stream()) != cudaSuccess) {
+            set_error(kErrCuda, "H2D copy failed"); break;
+        }
+        uint64_t pred[kRateSteps];
+        if (e->rate_curve(wavelet, stage, pred, nullptr)) break;
+        const uint8_t *ptrs[1] = {stage};
+        int step = pick_step(pred, max_bytes, first_step);
+        if (!step) { set_no_fit_error(pred, max_bytes); break; }
+        for (; step; step = pick_step(pred, max_bytes, step + 1)) {
+            out = new (std::nothrow) EncodedChunk();
+            if (!out) break;
+            if (e->encode_device(quality_for_step(step), wavelet, ptrs, 1, nullptr) || e->fetch_chunk(0, out->c)) {
+                delete out; out = nullptr;
+                break;
+            }
+            if (kAlcHeaderBytes + out->c.data.size() <= max_bytes) {
+                *quality_out = quality_for_step(step);
+                break;
+            }
+            delete out; out = nullptr;
+            set_error(kErrBufferSize, "no quality fits " + std::to_string(max_bytes) + " bytes");
+        }
+    } while (0);
+    release_engine(e);
+    return out;
+}
+
 uint8_t *decode_impl(const EncodedChunk *chunk, uint64_t *out_len, uint8_t *symbols_out) {
     set_error(0, "");
     if (!chunk || !out_len) { set_error(kErrNull, "null argument"); return nullptr; }
@@ -1173,6 +1296,77 @@ int alice_codec_batch_timings(AliceBatch *b, float *ms8) {
     return kOk;
 }
 uint64_t alice_codec_batch_device_bytes(const AliceBatch *b) { return b ? b->eng->device_bytes() : 0; }
+
+// ------------------------------------------------------------------------------ rate control
+int alice_codec_rate_curve(uint8_t wavelet, const uint8_t *rgb, uint64_t rgb_len, uint32_t width, uint32_t height,
+                           uint32_t frames, uint64_t *bytes64, uint32_t *hist_out) {
+    return rate_curve_impl(wavelet, rgb, false, rgb_len, width, height, frames, bytes64, hist_out, nullptr);
+}
+int alice_codec_rate_curve_device(uint8_t wavelet, const uint8_t *d_rgb, uint32_t width, uint32_t height,
+                                  uint32_t frames, uint64_t *bytes64, uint32_t *hist_out, void *cuda_stream) {
+    const unsigned __int128 len = (unsigned __int128)width * height * frames * 3;
+    if (len > (unsigned __int128)UINT64_MAX) { set_error(kErrOverflow, "dimensions overflow usize"); return kErrOverflow; }
+    return rate_curve_impl(wavelet, d_rgb, true, (uint64_t)len, width, height, frames, bytes64, hist_out,
+                           (cudaStream_t)cuda_stream);
+}
+EncodedChunk *alice_codec_encode_to_size(uint8_t wavelet, const uint8_t *rgb, uint64_t rgb_len, uint32_t width,
+                                         uint32_t height, uint32_t frames, uint64_t max_bytes, uint8_t *quality_out) {
+    return encode_to_size_impl(wavelet, rgb, rgb_len, width, height, frames, max_bytes, 1, quality_out);
+}
+// Per chunk, in stream order as alice_codec_batch_encode_host stages it: copy, rate curve, one host read of 64 sizes, the
+// front-end at the chosen step; then one table build and one rANS launch for the whole batch.
+int alice_codec_batch_encode_host_to_size(AliceBatch *b, const uint8_t *const *h_rgb, uint32_t n, uint64_t max_bytes,
+                                          EncodedChunk **out_chunks, uint8_t *qualities_out) {
+    set_error(0, "");
+    if (!b || !h_rgb || !out_chunks || !qualities_out) { set_error(kErrNull, "null argument"); return kErrNull; }
+    Engine *e = b->eng;
+    if (n > e->cap_chunks()) { set_error(kErrBufferSize, "batch larger than capacity"); return kErrBufferSize; }
+    const Dims &d = e->dims();
+    const size_t bytes = (size_t)d.n_pixels * 3;
+    const bool shared = e->shared_workspace();   // staging and workspaces as in alice_codec_batch_encode_host
+    std::vector<int> steps(n);
+    int rc = e->encode_begin(100, b->wavelet);    // the batch's quality is not used: every chunk names its step
+    for (uint32_t i = 0; i < n && !rc; i++) {
+        if (!h_rgb[i]) { set_error(kErrNull, "null chunk pointer"); return kErrNull; }
+        uint8_t *s = e->rgb_stage(shared ? i + 1 : 0);
+        uint8_t *work = shared ? e->rgb_stage(i) : nullptr;
+        if (!s || (shared && !work)) return kErrCuda;
+        CU_CHECK_RC(cudaMemcpyAsync(s, h_rgb[i], bytes, cudaMemcpyHostToDevice, e->stream()));
+        uint64_t pred[kRateSteps];
+        rc = e->rate_curve(b->wavelet, s, pred, nullptr, i, work);
+        if (rc) return rc;
+        steps[i] = pick_step(pred, max_bytes, 1);
+        if (!steps[i]) {
+            set_no_fit_error(pred, max_bytes);
+            set_error(kErrBufferSize, "chunk " + std::to_string(i) + ": " + last_error_msg());
+            return kErrBufferSize;
+        }
+        rc = e->encode_submit(i, s, work, steps[i]);
+    }
+    if (!rc) rc = e->encode_finish(n);
+    if (rc) return rc;
+    std::vector<Chunk *> cks(n);
+    for (uint32_t i = 0; i < n; i++) {
+        out_chunks[i] = new (std::nothrow) EncodedChunk();
+        if (!out_chunks[i]) { rc = kErrCuda; set_error(kErrCuda, "host allocation failed"); }
+        else cks[i] = &out_chunks[i]->c;
+    }
+    if (!rc) rc = e->fetch_chunks(n, cks.data());
+    for (uint32_t i = 0; i < n && !rc; i++) {
+        qualities_out[i] = quality_for_step(steps[i]);
+        if (kAlcHeaderBytes + out_chunks[i]->c.data.size() <= max_bytes) continue;
+        // larger than its prediction (the bound rules this out): this chunk alone, from the next step on
+        delete out_chunks[i];
+        out_chunks[i] = encode_to_size_impl(b->wavelet, h_rgb[i], bytes, d.w, d.h, d.f, max_bytes, steps[i] + 1,
+                                            &qualities_out[i]);
+        if (!out_chunks[i]) rc = last_error_code() ? last_error_code() : kErrCuda;
+    }
+    if (rc) {
+        for (uint32_t k = 0; k < n; k++) { delete out_chunks[k]; out_chunks[k] = nullptr; }
+        return rc;
+    }
+    return kOk;
+}
 
 int alice_codec_synth_rgb_device(int kind, uint32_t seed, uint32_t w, uint32_t h, uint32_t f, uint8_t *d_rgb,
                                  void *cuda_stream) {

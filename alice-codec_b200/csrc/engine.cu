@@ -254,6 +254,7 @@ Engine::Engine(const Dims &d, uint32_t cap_chunks, uint64_t payload_cap, cudaStr
     stream_off_.assign(S, 0);
     stream_len_.assign(S, 0);
     stream_base_.assign(S, nullptr);
+    chunk_step_.assign(cap_, 1);
     ok_ = true;
 }
 
@@ -272,6 +273,9 @@ Engine::~Engine() {
     if (h_inv_jobs_) cudaFreeHost(h_inv_jobs_);
     cudaFree(d_fwd_jobs_);
     cudaFree(d_inv_jobs_);
+    cudaFree(d_coef_); cudaFree(d_vhist_); cudaFree(d_rate_hist_); cudaFree(d_rate_enc_); cudaFree(d_rate_lut_);
+    cudaFree(d_rate_aux_); cudaFree(d_rate_est_); cudaFree(d_rate_out_);
+    if (h_rate_out_) cudaFreeHost(h_rate_out_);
     for (auto &e : ev_) if (e) cudaEventDestroy(e);
     if (st_ && own_stream_) cudaStreamDestroy(st_);
     cudaGetLastError();
@@ -375,7 +379,7 @@ int Engine::encode_device(uint8_t quality, uint8_t wavelet, const uint8_t *const
     const size_t N = (size_t)d_.padded;
     const int step = quality_to_step(quality);
     last_wavelet = wavelet;
-    last_step = step;
+    for (uint32_t c = 0; c < n; c++) chunk_step_[c] = step;
     last_n = n;
     resident_decoded_ = 0;
     CU_TRY(cudaMemsetAsync(d_hist_, 0, (size_t)n * 3 * 256 * sizeof(unsigned), st_));
@@ -428,20 +432,22 @@ int Engine::encode_device(uint8_t quality, uint8_t wavelet, const uint8_t *const
 // one chunk and returns at once), then encode_finish(n): tables, all 3n rANS streams, one synchronisation.
 int Engine::encode_begin(uint8_t quality, uint8_t wavelet) {
     last_wavelet = wavelet;
-    last_step = quality_to_step(quality);
+    begin_step_ = quality_to_step(quality);
     last_n = 0;
     submitted_ = 0;
     resident_decoded_ = 0;
     CU_TRY(cudaEventRecord(ev_[0], st_));
     return kOk;
 }
-int Engine::encode_submit(uint32_t c, const uint8_t *d_rgb, uint8_t *d_work) {
+int Engine::encode_submit(uint32_t c, const uint8_t *d_rgb, uint8_t *d_work, int step) {
     if (c >= cap_ || c != submitted_) { set_error(kErrBufferSize, "chunks must be submitted in index order, below the batch capacity"); return kErrBufferSize; }
     if (shared_ws_) {
         if (!d_work) { set_error(kErrNull, "shared-workspace batch: workspace pointer required"); return kErrNull; }
         sym_ptr_[c] = d_work;
     }
     const size_t N = (size_t)d_.padded;
+    if (step <= 0) step = begin_step_;
+    chunk_step_[c] = step;
     auto overlaps = [&](const uint8_t *a, size_t na, const uint8_t *b, size_t nb) { return a < b + nb && b < a + na; };
     unsigned *hist = d_hist_ + (size_t)c * 3 * 256;
     CU_TRY(cudaMemsetAsync(hist, 0, 3 * 256 * sizeof(unsigned), st_));
@@ -450,10 +456,10 @@ int Engine::encode_submit(uint32_t c, const uint8_t *d_rgb, uint8_t *d_work) {
     if (fused) {
         h_fwd_jobs_[c] = FwdFusedJob{d_rgb, sym_ptr_[c], hist, nullptr};
         CU_TRY(cudaMemcpyAsync(d_fwd_jobs_ + c, h_fwd_jobs_ + c, sizeof(FwdFusedJob), cudaMemcpyHostToDevice, st_));
-        forward_frontend_fused(last_wavelet, d_fwd_jobs_ + c, 1, false, hist, (int)d_.w, (int)d_.h, last_step, device_sm_count(), st_);
+        forward_frontend_fused(last_wavelet, d_fwd_jobs_ + c, 1, false, hist, (int)d_.w, (int)d_.h, step, device_sm_count(), st_);
     } else {
         forward_frontend(last_wavelet, d_rgb, reinterpret_cast<int16_t *>(d_scratch_), sym_ptr_[c], hist, (int)d_.w, (int)d_.h,
-                         (int)d_.f, (int)d_.pw, (int)d_.ph, (int)d_.pf, last_step, nullptr, st_);
+                         (int)d_.f, (int)d_.pw, (int)d_.ph, (int)d_.pf, step, nullptr, st_);
     }
     submitted_ = c + 1;
     return kOk;
@@ -481,8 +487,8 @@ int Engine::fetch_enqueue(uint32_t i, Chunk &out, bool &direct) {
         const uint32_t s = i * 3 + c;
         ChannelHeader &h = out.ch[c];
         h.compressed_len = (uint32_t)stream_len_[s];
-        h.quant_step = last_step;
-        h.quant_dead_zone = last_step;          // Quantizer::new: dead_zone = step (quant.rs:70-75)
+        h.quant_step = chunk_step_[i];
+        h.quant_dead_zone = chunk_step_[i];     // Quantizer::new: dead_zone = step (quant.rs:70-75)
         h.num_symbols = (uint32_t)d_.padded;    // `as u32`, pipeline.rs:492
         memcpy(h.histogram, h_hist_ + (size_t)s * 256, 256 * sizeof(uint32_t));
         total += stream_len_[s];
@@ -617,7 +623,8 @@ int Engine::decode_resident_begin(uint32_t n) {
 int Engine::decode_resident_next(uint32_t c, uint8_t *d_rgb_out) {
     if (c >= resident_decoded_) { set_error(kErrBufferSize, "decode_next: chunk index beyond the last decode_begin"); return kErrBufferSize; }
     if (!d_rgb_out) { set_error(kErrNull, "null output pointer"); return kErrNull; }
-    int rc = backend_one(c, BackendHeader{last_wavelet, {last_step, last_step, last_step}}, d_rgb_out);
+    const int step = chunk_step_[c];
+    int rc = backend_one(c, BackendHeader{last_wavelet, {step, step, step}}, d_rgb_out);
     if (rc) return rc;
     CU_TRY(cudaGetLastError());
     return kOk;
@@ -653,7 +660,7 @@ int Engine::decode_device_resident(uint8_t *const *d_rgb_out, uint32_t n) {
     CU_TRY(cudaEventRecord(ev_[6], st_));
     {
         std::vector<BackendHeader> hdr(n);
-        for (uint32_t c = 0; c < n; c++) hdr[c] = BackendHeader{last_wavelet, {last_step, last_step, last_step}};
+        for (uint32_t c = 0; c < n; c++) hdr[c] = BackendHeader{last_wavelet, {chunk_step_[c], chunk_step_[c], chunk_step_[c]}};
         int rc = run_backend(n, hdr.data(), d_rgb_out);
         if (rc) return rc;
     }
@@ -769,6 +776,82 @@ int Engine::decode_chunks(const Chunk *const *chunks, uint32_t n, uint8_t *const
     cudaEventElapsedTime(&timings.ms[3], ev_[4], ev_[5]);
     cudaEventElapsedTime(&timings.ms[4], ev_[5], ev_[6]);
     cudaEventElapsedTime(&timings.ms[5], ev_[6], ev_[7]);
+    return kOk;
+}
+
+// ------------------------------------------------------------------------------ rate curve
+bool Engine::ensure_rate_buffers() {
+    if (d_coef_) return true;
+    const size_t N = (size_t)d_.padded;
+    const size_t S = (size_t)kRateSteps * 3;
+    int bound = 0;
+    for (int wv = 0; wv < 3; wv++) bound = std::max(bound, rate_value_bound(wv));
+    bool a = true;
+    a = a && dev_alloc(d_coef_, 3 * N * sizeof(int32_t), dev_bytes_);
+    a = a && dev_alloc(d_vhist_, 3 * (2 * (size_t)bound + 1) * sizeof(unsigned), dev_bytes_);
+    a = a && dev_alloc(d_rate_hist_, S * 256 * sizeof(unsigned), dev_bytes_);
+    a = a && dev_alloc(d_rate_enc_, S * 256 * sizeof(EncSym), dev_bytes_);
+    a = a && dev_alloc(d_rate_lut_, S * kDecLutEntries * sizeof(uint32_t), dev_bytes_);
+    a = a && dev_alloc(d_rate_aux_, S * sizeof(DecAux), dev_bytes_);
+    a = a && dev_alloc(d_rate_est_, S * sizeof(unsigned long long), dev_bytes_);
+    a = a && dev_alloc(d_rate_out_, (kRateSteps + 1) * sizeof(unsigned long long), dev_bytes_);
+    a = a && cudaMallocHost((void **)&h_rate_out_, (kRateSteps + 1) * sizeof(unsigned long long)) == cudaSuccess;
+    if (!a) {
+        cudaGetLastError();
+        // leave the engine as it was: a later call retries
+        cudaFree(d_coef_); cudaFree(d_vhist_); cudaFree(d_rate_hist_); cudaFree(d_rate_enc_); cudaFree(d_rate_lut_);
+        cudaFree(d_rate_aux_); cudaFree(d_rate_est_); cudaFree(d_rate_out_);
+        if (h_rate_out_) cudaFreeHost(h_rate_out_);
+        d_coef_ = nullptr; d_vhist_ = nullptr; d_rate_hist_ = nullptr; d_rate_enc_ = nullptr; d_rate_lut_ = nullptr;
+        d_rate_aux_ = nullptr; d_rate_est_ = nullptr; d_rate_out_ = nullptr; h_rate_out_ = nullptr;
+        set_error(kErrCuda, "device or pinned memory allocation failed (rate curve)");
+        return false;
+    }
+    return true;
+}
+
+int Engine::rate_curve(uint8_t wavelet, const uint8_t *d_rgb, uint64_t bytes[kRateSteps], unsigned *h_hist_out,
+                       uint32_t slot, uint8_t *d_work) {
+    if (slot >= cap_) { set_error(kErrBufferSize, "rate curve: chunk slot beyond the engine capacity"); return kErrBufferSize; }
+    uint8_t *sym = d_work ? d_work : sym_ptr_[slot];
+    if (!sym) { set_error(kErrNull, "shared-workspace engine: workspace pointer required"); return kErrNull; }
+    const uint64_t dev_before = dev_bytes_;
+    if (!ensure_rate_buffers()) { dev_bytes_ = dev_before; return kErrCuda; }
+    const size_t N = (size_t)d_.padded;
+    unsigned *hist = d_hist_ + (size_t)slot * 3 * 256;
+    CU_TRY(cudaMemsetAsync(hist, 0, 3 * 256 * sizeof(unsigned), st_));
+    // front-end at any step (step 1) with the coefficient dump; the same kernel choice as encode_submit
+    auto overlaps = [&](const uint8_t *a, size_t na, const uint8_t *b, size_t nb) { return a < b + nb && b < a + na; };
+    const bool fused = !small_smem_ && forward_fused_eligible(d_rgb, (int)d_.w, (int)d_.h, (int)d_.f) &&
+                       (reinterpret_cast<uintptr_t>(sym) & 3) == 0 && !overlaps(sym, 3 * N, d_rgb, 3 * (size_t)d_.n_pixels);
+    if (fused) {
+        h_fwd_jobs_[slot] = FwdFusedJob{d_rgb, sym, hist, d_coef_};
+        CU_TRY(cudaMemcpyAsync(d_fwd_jobs_ + slot, h_fwd_jobs_ + slot, sizeof(FwdFusedJob), cudaMemcpyHostToDevice, st_));
+        forward_frontend_fused(wavelet, d_fwd_jobs_ + slot, 1, true, hist, (int)d_.w, (int)d_.h, 1, device_sm_count(), st_);
+    } else {
+        // the dump covers the padded volume [3][pf][ph][pw] (pf = f + 1 for odd f, 2 for f == 1) = [3][N]
+        forward_frontend(wavelet, d_rgb, reinterpret_cast<int16_t *>(d_scratch_), sym, hist, (int)d_.w, (int)d_.h,
+                         (int)d_.f, (int)d_.pw, (int)d_.ph, (int)d_.pf, 1, d_coef_, st_);
+    }
+    const int bound = rate_value_bound(wavelet);
+    CU_TRY(cudaMemsetAsync(d_vhist_, 0, 3 * (2 * (size_t)bound + 1) * sizeof(unsigned), st_));
+    CU_TRY(cudaMemsetAsync(d_rate_out_ + kRateSteps, 0, sizeof(unsigned long long), st_));
+    coef_value_hist(d_coef_, N, bound, d_vhist_, d_rate_out_ + kRateSteps, st_);
+    step_hists(d_vhist_, bound, N, d_rate_hist_, st_);
+    build_tables(d_rate_hist_, kRateSteps * 3, 256, d_rate_enc_, d_rate_lut_, d_rate_aux_, nullptr, nullptr, nullptr, st_);
+    estimate_stream_bytes(d_rate_hist_, d_rate_enc_, kRateSteps * 3, N, d_rate_est_, st_);
+    rate_sizes(d_rate_hist_, d_rate_enc_, d_rate_est_, N, kFixedHeaderBytes + 3 * kChannelHeaderBytes, d_rate_out_, st_);
+    CU_TRY(cudaMemcpyAsync(h_rate_out_, d_rate_out_, (kRateSteps + 1) * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st_));
+    if (h_hist_out)
+        CU_TRY(cudaMemcpyAsync(h_hist_out, d_rate_hist_, (size_t)kRateSteps * 3 * 256 * sizeof(unsigned), cudaMemcpyDeviceToHost, st_));
+    CU_TRY(cudaStreamSynchronize(st_));
+    CU_TRY(cudaGetLastError());
+    if (h_rate_out_[kRateSteps]) {
+        set_error(kErrPanic, "rate curve: " + std::to_string(h_rate_out_[kRateSteps]) +
+                                 " coefficients outside the derived value range");
+        return kErrPanic;
+    }
+    for (int i = 0; i < kRateSteps; i++) bytes[i] = h_rate_out_[i];
     return kOk;
 }
 

@@ -106,8 +106,9 @@ public:
                       int32_t *d_coef_dump, uint8_t *const *d_work = nullptr);
     // The same encode, one chunk at a time: begin, submit chunk 0, 1, ... (each call enqueues that chunk's front-end on the
     // stream and returns), finish(n) = tables + all rANS streams + one synchronisation.  d_work as in encode_device.
+    // step > 0: chunk c's quantiser step instead of the one encode_begin's quality gives (rate-controlled batches)
     int encode_begin(uint8_t quality, uint8_t wavelet);
-    int encode_submit(uint32_t c, const uint8_t *d_rgb, uint8_t *d_work);
+    int encode_submit(uint32_t c, const uint8_t *d_rgb, uint8_t *d_work, int step = 0);
     int encode_finish(uint32_t n);
     // Fill a Chunk (headers + payload copied to the host) from the last encode_device.
     int fetch_chunk(uint32_t i, Chunk &out);
@@ -129,13 +130,21 @@ public:
     int decode_chunks(const Chunk *const *chunks, uint32_t n, uint8_t *const *d_rgb_out, uint8_t *const *d_work = nullptr,
                       uint8_t *const *h_rgb_out = nullptr);
 
+    // Rate curve of one chunk (k_rate.cu): bytes[i] = an upper bound on the .alc length an encode at step i + 1 gives
+    // (UINT64_MAX where the reference aborts), h_hist_out (host, optional) = the symbol histograms [64][3][256] of every
+    // step.  Runs the front-end with the coefficient dump into chunk slot `slot` (its histogram and symbol planes, or
+    // d_work for shared-workspace engines, are scratch until that chunk's real front-end), then the value histogram,
+    // the step histograms, the table build and the estimate; one synchronisation.  The buffers it needs (12 B per padded
+    // pixel of coefficients + the tables of 192 pseudo-streams) are allocated on the first call.
+    int rate_curve(uint8_t wavelet, const uint8_t *d_rgb, uint64_t bytes[kRateSteps], unsigned *h_hist_out,
+                   uint32_t slot = 0, uint8_t *d_work = nullptr);
+
     // staging buffers for host-pointer entry points
     uint8_t *rgb_stage(uint32_t slot);          // device buffer of 3*n_pixels bytes, slot in [0, n_stage)
     uint32_t n_stage() const { return (uint32_t)rgb_stage_.size(); }
     const uint8_t *symbols_dev(uint32_t chunk) const { return sym_ptr_[chunk]; }
     EngineTimings timings;
     uint8_t last_wavelet = 0;
-    int last_step = 1;
     uint32_t last_n = 0;
     uint32_t submitted_ = 0;
 
@@ -173,6 +182,18 @@ private:
     uint8_t *h_pay_ = nullptr;                 // pinned staging for one chunk's payload (host <-> device)
     size_t h_pay_cap_ = 0;
     bool ensure_pinned_payload(size_t bytes);
+    std::vector<int> chunk_step_;              // quantiser step of every chunk of the last encode
+    int begin_step_ = 1;                       // encode_begin's step, for submits that name none
+    // rate curve (allocated by the first rate_curve call)
+    bool ensure_rate_buffers();
+    int32_t *d_coef_ = nullptr;                // i32 [3][N] coefficients
+    unsigned *d_vhist_ = nullptr;              // [3][2*bound+1] value histogram (largest bound of the three wavelets)
+    unsigned *d_rate_hist_ = nullptr;          // [64][3][256]
+    EncSym *d_rate_enc_ = nullptr;             // [192][256]
+    uint32_t *d_rate_lut_ = nullptr;           // [192][4096] (built, not read)
+    DecAux *d_rate_aux_ = nullptr;             // [192]
+    unsigned long long *d_rate_est_ = nullptr; // [192]
+    unsigned long long *d_rate_out_ = nullptr, *h_rate_out_ = nullptr;   // [64] sizes + [1] out-of-range count
     // pinned host mirrors
     unsigned long long *h_results_ = nullptr;
     unsigned *h_hist_ = nullptr;

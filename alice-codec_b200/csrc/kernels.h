@@ -88,6 +88,21 @@ struct RansDecJob {
 void rans_decode(const RansDecJob *d_jobs, const uint32_t *d_dec_lut, const DecAux *d_aux, int n_streams,
                  cudaStream_t st, bool shared_gpu = false);
 
+// ---- rate curve (k_rate.cu): the symbol histograms of every quantiser step from one histogram of coefficient values
+constexpr int kRateSteps = 64;   // quantiser steps 1..64 (quality_to_step)
+// largest |coefficient| of the pipeline's 3-D transform of u8 RGB for this wavelet (derivation in k_rate.cu)
+int rate_value_bound(int wavelet);
+// coef: i32 [3][n] (n a multiple of 8); vhist: u32 [3][2*bound+1] (zeroed by caller), bin v + bound = count of v, v != 0;
+// *out_of_range (zeroed by caller) += number of coefficients with |v| > bound
+void coef_value_hist(const int32_t *d_coef, unsigned long long n, int bound, unsigned *d_vhist,
+                     unsigned long long *d_out_of_range, cudaStream_t st);
+// hist [kRateSteps][3][256]: row (step-1)*3 + channel = the symbol histogram a front-end at that step would produce
+void step_hists(const unsigned *d_vhist, int bound, unsigned long long n, unsigned *d_hist, cudaStream_t st);
+// bytes[kRateSteps] = header_bytes + predicted stream bytes of the three channels (from estimate_stream_bytes' est),
+// UINT64_MAX where a used symbol has frequency 0
+void rate_sizes(const unsigned *d_hist, const EncSym *d_enc, const unsigned long long *d_est, unsigned long long n,
+                unsigned long long header_bytes, unsigned long long *d_bytes, cudaStream_t st);
+
 // ---- generic element-wise / line kernels behind the public stage API (k_generic.cu) -----
 void lift_axis(int32_t *d_data, int32_t *d_tmp, int wavelet, bool inverse, int axis, long long w, long long h,
                long long d, cudaStream_t st);  // one 1-D transform along `axis` (0=x,1=y,2=t) of every line

@@ -12,7 +12,7 @@ struct QuantDev {
     uint32_t magic;  // ceil(2^32 / step) for step >= 2
 };
 
-inline QuantDev make_quant_dev(int step) {
+ALICE_HD QuantDev make_quant_dev(int step) {
     QuantDev q;
     q.step = step;
     q.dz = step;

@@ -273,6 +273,28 @@ int alice_codec_batch_timings(AliceBatch *b, float *ms8);
 /* bytes of device memory the batch holds */
 uint64_t alice_codec_batch_device_bytes(const AliceBatch *b);
 
+/* ---- Byte-budget encoding.  Quality q maps to quantiser step 64 - 63q/100 (1..64); a step's chunk size is bounded
+ * before any rANS work from one transform pass and one histogram of the coefficient values (the symbol histogram of
+ * every step follows from it, and the table build's size estimate bounds every stream).  The .alc format is unchanged:
+ * a rate-controlled chunk is byte-identical to alice_codec_encode at the quality it reports, which is the largest
+ * quality with that step.  An empty input (a zero dimension) is the 3138-byte empty chunk at every step. */
+/* predicted .alc size of every quantiser step (index i = step i+1), UINT64_MAX where the reference would abort;
+ * hist_out (u32 [64][3][256]) may be null */
+int alice_codec_rate_curve(uint8_t wavelet, const uint8_t *rgb, uint64_t rgb_len, uint32_t width, uint32_t height,
+                           uint32_t frames, uint64_t *bytes64, uint32_t *hist_out);
+/* the same for RGB in device memory; the call waits for the work enqueued on cuda_stream before it reads d_rgb */
+int alice_codec_rate_curve_device(uint8_t wavelet, const uint8_t *d_rgb, uint32_t width, uint32_t height,
+                                  uint32_t frames, uint64_t *bytes64, uint32_t *hist_out, void *cuda_stream);
+/* the highest quality whose chunk fits max_bytes; identical to alice_codec_encode at *quality_out.  No quality fits:
+ * null, ALICE_ERR_BUFFER_SIZE, and the message names the smallest predicted size */
+EncodedChunk *alice_codec_encode_to_size(uint8_t wavelet, const uint8_t *rgb, uint64_t rgb_len, uint32_t width,
+                                         uint32_t height, uint32_t frames, uint64_t max_bytes, uint8_t *quality_out);
+/* host-buffer batch, every chunk with its own quality under the same per-chunk budget; all 3n rANS streams run
+ * concurrently as in alice_codec_batch_encode_host.  The batch's own quality is not used.  The first rate call on a
+ * batch allocates 12 B per padded pixel of coefficients plus ~4 MB of tables (alice_codec_batch_device_bytes grows). */
+int alice_codec_batch_encode_host_to_size(AliceBatch *b, const uint8_t *const *h_rgb, uint32_t n, uint64_t max_bytes,
+                                          EncodedChunk **out_chunks, uint8_t *qualities_out);
+
 /* synthetic RGB volumes generated on the device (SURVEY.md Appendix D): kind 0=G0, 1=G1, 2=G2 */
 int alice_codec_synth_rgb_device(int kind, uint32_t seed, uint32_t width, uint32_t height, uint32_t frames,
                                  uint8_t *d_rgb, void *cuda_stream);
