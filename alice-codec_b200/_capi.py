@@ -51,6 +51,7 @@ SIGNATURES = {
     "alice_codec_last_error": (i32, []),
     "alice_codec_last_error_message": (C.c_char_p, []),
     "alice_codec_encoder_create_with_wavelet": (vp, [u8, u8]),
+    "alice_codec_encoder_create_ex": (vp, [u8, u8, u32]),
     "alice_codec_chunk_wavelet": (u8, [vp]),
     "alice_codec_chunk_compressed_size": (u64, [vp]),
     "alice_codec_chunk_channel_header": (cint, [vp, u32, u32p, i32p, i32p, u32p, u32p]),
@@ -115,6 +116,9 @@ SIGNATURES = {
     "alice_codec_rate_curve": (cint, [u8, u8p, u64, u32, u32, u32, u64p, u32p]),
     "alice_codec_rate_curve_device": (cint, [u8, vp, u32, u32, u32, u64p, u32p, vp]),
     "alice_codec_encode_to_size": (vp, [u8, u8p, u64, u32, u32, u32, u64, u8p]),
+    "alice_codec_rate_curve_ex": (cint, [u8, u8p, u64, u32, u32, u32, u64p, u32p, u32]),
+    "alice_codec_rate_curve_device_ex": (cint, [u8, vp, u32, u32, u32, u64p, u32p, vp, u32]),
+    "alice_codec_encode_to_size_ex": (vp, [u8, u8p, u64, u32, u32, u32, u64, u8p, u32]),
     "alice_codec_batch_encode_host_to_size": (cint, [vp, C.POINTER(vp), u32, u64, C.POINTER(vp), u8p]),
     "alice_codec_synth_rgb_device": (cint, [cint, u32, u32, u32, u32, vp, vp]),
     "alice_codec_pinned_alloc": (vp, [u64]),

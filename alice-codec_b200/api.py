@@ -416,15 +416,25 @@ class EncodedChunk:
         return f"EncodedChunk({self.width}x{self.height}x{self.frames}, {self.compressed_size} bytes, {self.wavelet})"
 
 
-class FrameEncoder:
-    """python.rs:365-435: FrameEncoder(quality=90, wavelet="cdf53").encode(rgb_frames, width, height, frames)."""
+ENCODE_WELL_FORMED_TABLES = 1   # ALICE_ENCODE_WELL_FORMED_TABLES
+BATCH_WELL_FORMED_TABLES = 4    # ALICE_BATCH_WELL_FORMED_TABLES
 
-    def __init__(self, quality: int = 90, wavelet="cdf53", api: Api | None = None):
+
+class FrameEncoder:
+    """python.rs:365-435: FrameEncoder(quality=90, wavelet="cdf53").encode(rgb_frames, width, height, frames).
+
+    well_formed_tables=True: every encode (and rate_curve / encode_to_size) stores, per channel, a histogram whose
+    rANS table keeps every used symbol inside [0, 4096), so that the chunk decodes to exactly what was encoded on any
+    decoder of the format (DESIGN.md 4.8).  The header histogram is then a table specification, not symbol counts."""
+
+    def __init__(self, quality: int = 90, wavelet="cdf53", api: Api | None = None, well_formed_tables: bool = False):
         if not 0 <= int(quality) <= 255:
             raise OverflowError("quality must fit in u8")
         self._api = api or default_api()
         self.quality, self.wavelet = int(quality), _wavelet_byte(wavelet)
-        self._h = self._api.lib.alice_codec_encoder_create_with_wavelet(self.quality, self.wavelet)
+        self.well_formed_tables = bool(well_formed_tables)
+        self._flags = ENCODE_WELL_FORMED_TABLES if self.well_formed_tables else 0
+        self._h = self._api.lib.alice_codec_encoder_create_ex(self.quality, self.wavelet, self._flags)
         if not self._h:
             self._api._raise()
 
@@ -460,33 +470,34 @@ class FrameEncoder:
     def rate_curve(self, rgb_frames, width: int, height: int, frames: int, with_hist: bool = False):
         """Predicted .alc size of the chunk at every quantiser step, before any rANS work: {quality: bytes}, one entry per
         step (the largest quality with that step), each an upper bound on len(encode at that quality).to_bytes(); None
-        where the reference aborts.  The encoder's wavelet is used, its quality is not.  with_hist=True also returns the
-        symbol histograms, uint32 [64][3][256] (row step - 1): what the headers of those encodes hold."""
+        where the reference aborts.  The encoder's wavelet and table mode are used, its quality is not.  with_hist=True
+        also returns the symbol histograms, uint32 [64][3][256] (row step - 1): what the headers of default encodes hold.
+        With well_formed_tables the sizes bound the well-formed encodes, and no step is None."""
         a, pa = _u8(rgb_frames)
         sizes = np.zeros(RATE_STEPS, np.uint64)
         hist = np.zeros((RATE_STEPS, 3, 256), np.uint32) if with_hist else None
-        self._api._chk(self._api.lib.alice_codec_rate_curve(
+        self._api._chk(self._api.lib.alice_codec_rate_curve_ex(
             self.wavelet, pa, a.size, width, height, frames, sizes.ctypes.data_as(_capi.u64p),
-            hist.ctypes.data_as(_capi.u32p) if with_hist else None))
+            hist.ctypes.data_as(_capi.u32p) if with_hist else None, self._flags))
         return (_curve_dict(sizes), hist) if with_hist else _curve_dict(sizes)
 
     def rate_curve_device(self, d_rgb: int, width: int, height: int, frames: int, stream: int = 0, with_hist: bool = False):
         """rate_curve for RGB in device memory (raw device pointer); waits for the work enqueued on `stream` first"""
         sizes = np.zeros(RATE_STEPS, np.uint64)
         hist = np.zeros((RATE_STEPS, 3, 256), np.uint32) if with_hist else None
-        self._api._chk(self._api.lib.alice_codec_rate_curve_device(
+        self._api._chk(self._api.lib.alice_codec_rate_curve_device_ex(
             self.wavelet, C.c_void_p(int(d_rgb)), width, height, frames, sizes.ctypes.data_as(_capi.u64p),
-            hist.ctypes.data_as(_capi.u32p) if with_hist else None, C.c_void_p(stream)))
+            hist.ctypes.data_as(_capi.u32p) if with_hist else None, C.c_void_p(stream), self._flags))
         return (_curve_dict(sizes), hist) if with_hist else _curve_dict(sizes)
 
     def encode_to_size(self, rgb_frames, width: int, height: int, frames: int, max_bytes: int):
         """The chunk at the highest quality whose .alc (to_bytes) is at most max_bytes: (EncodedChunk, quality), the
-        chunk byte-identical to FrameEncoder(quality, wavelet).encode.  The encoder's quality is not used.  Raises
-        CodecError InvalidBufferSize if no quality fits."""
+        chunk byte-identical to FrameEncoder(quality, wavelet, well_formed_tables=...).encode.  The encoder's quality is
+        not used.  Raises CodecError InvalidBufferSize if no quality fits."""
         a, pa = _u8(rgb_frames)
         q = C.c_uint8()
-        h = self._api.lib.alice_codec_encode_to_size(self.wavelet, pa, a.size, width, height, frames, int(max_bytes),
-                                                     C.byref(q))
+        h = self._api.lib.alice_codec_encode_to_size_ex(self.wavelet, pa, a.size, width, height, frames, int(max_bytes),
+                                                        C.byref(q), self._flags)
         if not h:
             self._api._raise()
         return EncodedChunk(h, self._api), q.value
@@ -569,17 +580,22 @@ class ReferenceAbi:
 class ChunkBatch:
     """Many independent chunks of one shape in flight on one GPU (the throughput path):
     wraps the alice_codec_batch_* entry points.  Device pointers are plain integers
-    (e.g. torch.Tensor.data_ptr()); `stream` is a cudaStream_t value (0 = default stream)."""
+    (e.g. torch.Tensor.data_ptr()); `stream` is a cudaStream_t value (0 = default stream).
+    well_formed_tables=True: every encode of the batch stores well-formed table specifications, as
+    FrameEncoder(..., well_formed_tables=True) does."""
 
     def __init__(self, quality, wavelet, width, height, frames, n_chunks, stream: int = 0, api: Api | None = None,
-                 shared_workspace: bool = False, payload_bytes_per_chunk: int = 0, small_smem_kernels: bool = False):
+                 shared_workspace: bool = False, payload_bytes_per_chunk: int = 0, small_smem_kernels: bool = False,
+                 well_formed_tables: bool = False):
         self._api = api or default_api()
         self.n_chunks = n_chunks
         self.shape = (width, height, frames)
         self.shared_workspace = shared_workspace
+        self.well_formed_tables = bool(well_formed_tables)
+        flags = ((1 if shared_workspace else 0) | (2 if small_smem_kernels else 0) |
+                 (BATCH_WELL_FORMED_TABLES if well_formed_tables else 0))
         self._h = self._api.lib.alice_codec_batch_create_ex2(int(quality), _wavelet_byte(wavelet), width, height, frames,
-                                                             n_chunks, C.c_void_p(stream),
-                                                             (1 if shared_workspace else 0) | (2 if small_smem_kernels else 0),
+                                                             n_chunks, C.c_void_p(stream), flags,
                                                              int(payload_bytes_per_chunk))
         if not self._h:
             self._api._raise()

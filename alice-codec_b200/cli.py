@@ -3,7 +3,8 @@ reference's CLI (src/bin/main.rs:36-196), plus multi-chunk streams (SURVEY.md §
 is cut into N-frame chunks, the chunks run as one batch (all rANS streams concurrently) and the output is the
 concatenation of self-delimiting .alc blobs; `decode` and `info` accept such streams.  With --max-bytes N every chunk
 (the whole input without --chunk-frames) is encoded at the highest quality whose .alc blob is at most N bytes; the chunk
-is byte-identical to an encode at that quality, and -q is not used.
+is byte-identical to an encode at that quality, and -q is not used.  With --well-formed-tables every chunk stores
+rANS tables that decode exactly on any decoder of the format (DESIGN.md 4.8); without it the output is the reference's.
 
     python -m alice_codec_b200.cli encode raw.rgb -W 1920 -H 1080 -f 64 -q 90 -w cdf53 -o out.alc
     (from the repo root: python alice-codec_b200/cli.py ...)
@@ -31,7 +32,7 @@ def cmd_encode(a) -> None:
     if a.wavelet not in pkg.WAVELET_NAMES:
         raise ValueError(f"unknown wavelet '{a.wavelet}'; expected cdf53, cdf97, or haar")     # main.rs:74-83
     rgb = np.fromfile(a.input, dtype=np.uint8)
-    enc = pkg.FrameEncoder(a.quality, a.wavelet)
+    enc = pkg.FrameEncoder(a.quality, a.wavelet, well_formed_tables=a.well_formed_tables)
     budget = a.max_bytes
     qualities = []                                  # --max-bytes: the quality chosen for each chunk
 
@@ -50,7 +51,8 @@ def cmd_encode(a) -> None:
         n_full, rest = divmod(a.frames, a.chunk_frames)
         blobs = []
         if n_full >= 2:
-            batch = pkg.ChunkBatch(a.quality, a.wavelet, a.width, a.height, a.chunk_frames, n_full)
+            batch = pkg.ChunkBatch(a.quality, a.wavelet, a.width, a.height, a.chunk_frames, n_full,
+                                   well_formed_tables=a.well_formed_tables)
             cb = per * a.chunk_frames
             parts = [np.ascontiguousarray(rgb[i * cb:(i + 1) * cb]) for i in range(n_full)]
             if budget is None:
@@ -73,8 +75,9 @@ def cmd_encode(a) -> None:
     ratio = len(data) / rgb.size if rgb.size else 0.0
     setting = (f"quality={a.quality}" if budget is None else
                f"max-bytes={budget} per chunk, quality={','.join(str(q) for q in qualities)}")
+    tables = ", tables=well-formed" if a.well_formed_tables else ""
     sys.stderr.write(f"encoded {a.width}x{a.height}x{a.frames} ({rgb.size} bytes) -> {len(data)} bytes "
-                     f"({ratio * 100:.1f}% ratio, {setting}, wavelet={a.wavelet})\n")
+                     f"({ratio * 100:.1f}% ratio, {setting}, wavelet={a.wavelet}{tables})\n")
 
 
 def _blobs(data: bytes):
@@ -139,6 +142,9 @@ def main(argv=None) -> int:
     e.add_argument("--chunk-frames", type=int, default=0, help="cut the input into chunks of this many frames (0 = one chunk)")
     e.add_argument("--max-bytes", type=int, default=None,
                    help="byte budget per chunk: encode each chunk at the highest quality whose .alc fits (-q is not used)")
+    e.add_argument("--well-formed-tables", action="store_true",
+                   help="store rANS tables that every .alc decoder decodes exactly (the header histograms become table "
+                        "specifications instead of symbol counts)")
     d = sub.add_parser("decode", help="Decode an .alc bitstream back to raw RGB")
     d.add_argument("input")
     d.add_argument("-o", "--output", required=True)

@@ -13,7 +13,7 @@
 using namespace alice;
 
 struct Wavelet1D { int kind; };                       // wavelet.rs:47-50 (step list chosen by kind)
-struct FrameEncoder { uint8_t quality; uint8_t wavelet; };   // pipeline.rs:335-340
+struct FrameEncoder { uint8_t quality; uint8_t wavelet; bool well_formed = false; };   // pipeline.rs:335-340
 struct EncodedChunk { Chunk c; };
 struct AliceBatch {
     Engine *eng = nullptr;
@@ -150,7 +150,7 @@ EncodedChunk *encode_impl(const FrameEncoder *enc, const uint8_t *rgb, uint64_t 
     out->c.wavelet = enc->wavelet;
     if (empty) return out;  // three default headers, empty payload (pipeline.rs:391-412)
     if (!cuda_ready()) { delete out; return nullptr; }
-    Engine *e = acquire_engine(d);
+    Engine *e = acquire_engine(d, enc->well_formed);
     if (!e) { delete out; return nullptr; }
     int rc = kOk;
     DevBuf coef;
@@ -204,12 +204,18 @@ void set_no_fit_error(const uint64_t pred[kRateSteps], uint64_t max_bytes) {
                                                       : std::to_string(best) + " bytes"));
 }
 
+bool encode_flags_ok(uint32_t flags) {
+    if (flags & ~(uint32_t)ALICE_ENCODE_WELL_FORMED_TABLES) { set_error(kErrDimensions, "unknown encode flag"); return false; }
+    return true;
+}
+
 // Predicted .alc size of every step for one chunk whose RGB is on the host (device == false) or the device.
 int rate_curve_impl(uint8_t wavelet, const uint8_t *rgb, bool device, uint64_t rgb_len, uint32_t w, uint32_t h,
-                    uint32_t f, uint64_t *bytes64, uint32_t *hist_out, cudaStream_t user_st) {
+                    uint32_t f, uint64_t *bytes64, uint32_t *hist_out, cudaStream_t user_st, uint32_t flags) {
     set_error(0, "");
     if (!bytes64) { set_error(kErrNull, "null output"); return kErrNull; }
     if (wavelet > 2) { set_error(kErrBitstream, "unknown wavelet type byte"); return kErrBitstream; }
+    if (!encode_flags_ok(flags)) return kErrDimensions;
     Dims d;
     bool empty;
     int rc = validate_encode(rgb_len, w, h, f, d, empty);
@@ -221,7 +227,7 @@ int rate_curve_impl(uint8_t wavelet, const uint8_t *rgb, bool device, uint64_t r
     }
     if (!rgb) { set_error(kErrNull, "null argument"); return kErrNull; }
     if (!cuda_ready()) return kErrCuda;
-    Engine *e = acquire_engine(d);
+    Engine *e = acquire_engine(d, (flags & ALICE_ENCODE_WELL_FORMED_TABLES) != 0);
     if (!e) return kErrCuda;
     do {
         const uint8_t *src = rgb;
@@ -249,10 +255,11 @@ int rate_curve_impl(uint8_t wavelet, const uint8_t *rgb, bool device, uint64_t r
 // The highest quality whose chunk fits max_bytes, trying steps from first_step on: the rate curve picks the step, one
 // real encode checks it (an encode larger than its prediction, which the bound rules out, moves on to the next step).
 EncodedChunk *encode_to_size_impl(uint8_t wavelet, const uint8_t *rgb, uint64_t rgb_len, uint32_t w, uint32_t h,
-                                  uint32_t f, uint64_t max_bytes, int first_step, uint8_t *quality_out) {
+                                  uint32_t f, uint64_t max_bytes, int first_step, uint8_t *quality_out, uint32_t flags) {
     set_error(0, "");
     if (!rgb || !quality_out) { set_error(kErrNull, "null argument"); return nullptr; }
     if (wavelet > 2) { set_error(kErrBitstream, "unknown wavelet type byte"); return nullptr; }
+    if (!encode_flags_ok(flags)) return nullptr;
     Dims d;
     bool empty;
     if (validate_encode(rgb_len, w, h, f, d, empty)) return nullptr;
@@ -268,7 +275,7 @@ EncodedChunk *encode_to_size_impl(uint8_t wavelet, const uint8_t *rgb, uint64_t 
         return out;
     }
     if (!cuda_ready()) return nullptr;
-    Engine *e = acquire_engine(d);
+    Engine *e = acquire_engine(d, (flags & ALICE_ENCODE_WELL_FORMED_TABLES) != 0);
     if (!e) return nullptr;
     EncodedChunk *out = nullptr;
     do {
@@ -425,6 +432,12 @@ const char *alice_codec_last_error_message(void) { return last_error_msg(); }
 FrameEncoder *alice_codec_encoder_create_with_wavelet(uint8_t quality, uint8_t wavelet) {
     if (wavelet > 2) { set_error(kErrBitstream, "unknown wavelet type byte"); return nullptr; }
     return new (std::nothrow) FrameEncoder{quality, wavelet};
+}
+FrameEncoder *alice_codec_encoder_create_ex(uint8_t quality, uint8_t wavelet, uint32_t flags) {
+    set_error(0, "");
+    if (wavelet > 2) { set_error(kErrBitstream, "unknown wavelet type byte"); return nullptr; }
+    if (!encode_flags_ok(flags)) return nullptr;
+    return new (std::nothrow) FrameEncoder{quality, wavelet, (flags & ALICE_ENCODE_WELL_FORMED_TABLES) != 0};
 }
 uint8_t alice_codec_chunk_wavelet(const EncodedChunk *c) { return c ? c->c.wavelet : 0; }
 uint64_t alice_codec_chunk_compressed_size(const EncodedChunk *c) { return c ? c->c.data.size() : 0; }
@@ -1094,7 +1107,8 @@ AliceBatch *alice_codec_batch_create_ex2(uint8_t quality, uint8_t wavelet, uint3
     uint64_t cap = n_chunks == 1 ? 0 : d.padded / 3 + 65536;
     if (payload_bytes_per_chunk) cap = payload_bytes_per_chunk / 3 + 16;
     b->eng = new (std::nothrow) Engine(d, n_chunks, cap, (cudaStream_t)cuda_stream, false,
-                                       (flags & ALICE_BATCH_SHARED_WORKSPACE) != 0);
+                                       (flags & ALICE_BATCH_SHARED_WORKSPACE) != 0,
+                                       (flags & ALICE_BATCH_WELL_FORMED_TABLES) != 0);
     if (!b->eng || !b->eng->ok()) { delete b->eng; delete b; return nullptr; }
     b->eng->set_prefer_small_smem((flags & ALICE_BATCH_SMALL_SMEM_KERNELS) != 0);
     b->quality = quality;
@@ -1300,18 +1314,32 @@ uint64_t alice_codec_batch_device_bytes(const AliceBatch *b) { return b ? b->eng
 // ------------------------------------------------------------------------------ rate control
 int alice_codec_rate_curve(uint8_t wavelet, const uint8_t *rgb, uint64_t rgb_len, uint32_t width, uint32_t height,
                            uint32_t frames, uint64_t *bytes64, uint32_t *hist_out) {
-    return rate_curve_impl(wavelet, rgb, false, rgb_len, width, height, frames, bytes64, hist_out, nullptr);
+    return alice_codec_rate_curve_ex(wavelet, rgb, rgb_len, width, height, frames, bytes64, hist_out, 0);
+}
+int alice_codec_rate_curve_ex(uint8_t wavelet, const uint8_t *rgb, uint64_t rgb_len, uint32_t width, uint32_t height,
+                              uint32_t frames, uint64_t *bytes64, uint32_t *hist_out, uint32_t flags) {
+    return rate_curve_impl(wavelet, rgb, false, rgb_len, width, height, frames, bytes64, hist_out, nullptr, flags);
 }
 int alice_codec_rate_curve_device(uint8_t wavelet, const uint8_t *d_rgb, uint32_t width, uint32_t height,
                                   uint32_t frames, uint64_t *bytes64, uint32_t *hist_out, void *cuda_stream) {
+    return alice_codec_rate_curve_device_ex(wavelet, d_rgb, width, height, frames, bytes64, hist_out, cuda_stream, 0);
+}
+int alice_codec_rate_curve_device_ex(uint8_t wavelet, const uint8_t *d_rgb, uint32_t width, uint32_t height,
+                                     uint32_t frames, uint64_t *bytes64, uint32_t *hist_out, void *cuda_stream,
+                                     uint32_t flags) {
     const unsigned __int128 len = (unsigned __int128)width * height * frames * 3;
     if (len > (unsigned __int128)UINT64_MAX) { set_error(kErrOverflow, "dimensions overflow usize"); return kErrOverflow; }
     return rate_curve_impl(wavelet, d_rgb, true, (uint64_t)len, width, height, frames, bytes64, hist_out,
-                           (cudaStream_t)cuda_stream);
+                           (cudaStream_t)cuda_stream, flags);
 }
 EncodedChunk *alice_codec_encode_to_size(uint8_t wavelet, const uint8_t *rgb, uint64_t rgb_len, uint32_t width,
                                          uint32_t height, uint32_t frames, uint64_t max_bytes, uint8_t *quality_out) {
-    return encode_to_size_impl(wavelet, rgb, rgb_len, width, height, frames, max_bytes, 1, quality_out);
+    return alice_codec_encode_to_size_ex(wavelet, rgb, rgb_len, width, height, frames, max_bytes, quality_out, 0);
+}
+EncodedChunk *alice_codec_encode_to_size_ex(uint8_t wavelet, const uint8_t *rgb, uint64_t rgb_len, uint32_t width,
+                                            uint32_t height, uint32_t frames, uint64_t max_bytes, uint8_t *quality_out,
+                                            uint32_t flags) {
+    return encode_to_size_impl(wavelet, rgb, rgb_len, width, height, frames, max_bytes, 1, quality_out, flags);
 }
 // Per chunk, in stream order as alice_codec_batch_encode_host stages it: copy, rate curve, one host read of 64 sizes, the
 // front-end at the chosen step; then one table build and one rANS launch for the whole batch.
@@ -1358,7 +1386,8 @@ int alice_codec_batch_encode_host_to_size(AliceBatch *b, const uint8_t *const *h
         // larger than its prediction (the bound rules this out): this chunk alone, from the next step on
         delete out_chunks[i];
         out_chunks[i] = encode_to_size_impl(b->wavelet, h_rgb[i], bytes, d.w, d.h, d.f, max_bytes, steps[i] + 1,
-                                            &qualities_out[i]);
+                                            &qualities_out[i],
+                                            e->well_formed_tables() ? (uint32_t)ALICE_ENCODE_WELL_FORMED_TABLES : 0u);
         if (!out_chunks[i]) rc = last_error_code() ? last_error_code() : kErrCuda;
     }
     if (rc) {

@@ -217,8 +217,8 @@ template <class T> static bool dev_alloc(T *&p, size_t bytes, uint64_t &acc) {
 static size_t round_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
 Engine::Engine(const Dims &d, uint32_t cap_chunks, uint64_t payload_cap, cudaStream_t user_stream, bool own_stream,
-               bool shared_workspace)
-    : d_(d), cap_(cap_chunks), own_stream_(own_stream), shared_ws_(shared_workspace) {
+               bool shared_workspace, bool well_formed_tables)
+    : d_(d), cap_(cap_chunks), own_stream_(own_stream), shared_ws_(shared_workspace), well_formed_(well_formed_tables) {
     const size_t N = (size_t)d_.padded;
     const size_t vol = (size_t)d_.f * d_.ph * d_.pw;
     pay_cap_ = payload_cap ? round_up((size_t)payload_cap, 16) : rans_enc_worst_case(N);
@@ -230,6 +230,8 @@ Engine::Engine(const Dims &d, uint32_t cap_chunks, uint64_t payload_cap, cudaStr
     a = a && dev_alloc(d_scratch_, vol * 3 * 4, dev_bytes_);
     if (!shared_ws_) a = a && dev_alloc(d_symbols_, S * N, dev_bytes_);
     a = a && dev_alloc(d_hist_, S * 256 * sizeof(unsigned), dev_bytes_);
+    if (well_formed_) a = a && dev_alloc(d_wf_hist_, S * 256 * sizeof(unsigned), dev_bytes_);
+    d_tab_hist_ = well_formed_ ? d_wf_hist_ : d_hist_;
     a = a && dev_alloc(d_enc_, S * 256 * sizeof(EncSym), dev_bytes_);
     a = a && dev_alloc(d_dec_lut_, S * kDecLutEntries * sizeof(uint32_t), dev_bytes_);
     a = a && dev_alloc(d_aux_, S * sizeof(DecAux), dev_bytes_);
@@ -260,7 +262,7 @@ Engine::Engine(const Dims &d, uint32_t cap_chunks, uint64_t payload_cap, cudaStr
 
 Engine::~Engine() {
     if (st_ && own_stream_) cudaStreamSynchronize(st_);
-    cudaFree(d_scratch_); cudaFree(d_symbols_); cudaFree(d_hist_); cudaFree(d_enc_); cudaFree(d_dec_lut_);
+    cudaFree(d_scratch_); cudaFree(d_symbols_); cudaFree(d_hist_); cudaFree(d_wf_hist_); cudaFree(d_enc_); cudaFree(d_dec_lut_);
     cudaFree(d_aux_); cudaFree(d_payload_); cudaFree(d_enc_jobs_); cudaFree(d_dec_jobs_); cudaFree(d_results_);
     for (uint8_t *p : rgb_stage_) cudaFree(p);
     for (uint8_t *p : overflow_bufs_) if (p) cudaFree(p);
@@ -273,8 +275,8 @@ Engine::~Engine() {
     if (h_inv_jobs_) cudaFreeHost(h_inv_jobs_);
     cudaFree(d_fwd_jobs_);
     cudaFree(d_inv_jobs_);
-    cudaFree(d_coef_); cudaFree(d_vhist_); cudaFree(d_rate_hist_); cudaFree(d_rate_enc_); cudaFree(d_rate_lut_);
-    cudaFree(d_rate_aux_); cudaFree(d_rate_est_); cudaFree(d_rate_out_);
+    cudaFree(d_coef_); cudaFree(d_vhist_); cudaFree(d_rate_hist_); cudaFree(d_rate_wf_hist_); cudaFree(d_rate_enc_);
+    cudaFree(d_rate_lut_); cudaFree(d_rate_aux_); cudaFree(d_rate_est_); cudaFree(d_rate_out_);
     if (h_rate_out_) cudaFreeHost(h_rate_out_);
     for (auto &e : ev_) if (e) cudaEventDestroy(e);
     if (st_ && own_stream_) cudaStreamDestroy(st_);
@@ -312,7 +314,7 @@ int Engine::run_rans_encode(uint32_t n) {
     // Payload placement: the streams go back to back into the engine's payload arena (cap_ * 3 * pay_cap_ bytes), each with
     // the upper bound that its histogram and table give (k_estimate_stream_bytes) instead of a fixed slot, so the arena
     // only has to hold what the batch really produces (+ 0.03 %).  A stream that does not fit any more gets no room at all
-    // and goes through the overflow path below.
+    // and goes through the overflow path below.  The estimate takes the symbol counts, whatever table they are coded with.
     estimate_stream_bytes(d_hist_, d_enc_, (int)S, N, d_results_, st_);
     CU_TRY(cudaMemcpyAsync(h_results_, d_results_, S * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st_));
     CU_TRY(cudaStreamSynchronize(st_));
@@ -332,7 +334,7 @@ int Engine::run_rans_encode(uint32_t n) {
     rans_encode(d_enc_jobs_, d_enc_, d_hist_, d_results_, (int)S, st_, small_smem_);
     CU_TRY(cudaEventRecord(ev_[3], st_));
     CU_TRY(cudaMemcpyAsync(h_results_, d_results_, S * 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st_));
-    CU_TRY(cudaMemcpyAsync(h_hist_, d_hist_, (size_t)S * 256 * sizeof(unsigned), cudaMemcpyDeviceToHost, st_));
+    CU_TRY(cudaMemcpyAsync(h_hist_, d_tab_hist_, (size_t)S * 256 * sizeof(unsigned), cudaMemcpyDeviceToHost, st_));
     CU_TRY(cudaStreamSynchronize(st_));
     CU_TRY(cudaGetLastError());
     for (uint32_t s = 0; s < S; s++) {
@@ -364,6 +366,12 @@ int Engine::run_rans_encode(uint32_t n) {
         stream_off_[s] = h_enc_jobs_[s].cap - stream_len_[s];
     }
     return kOk;
+}
+
+// symbol counts of n chunks -> the headers' histograms (well-formed engines) -> the rANS tables
+void Engine::build_encode_tables(uint32_t n) {
+    if (well_formed_) well_formed_hists(d_hist_, (int)n * 3, d_wf_hist_, st_);
+    build_tables(d_tab_hist_, (int)n * 3, 256, d_enc_, d_dec_lut_, d_aux_, nullptr, nullptr, nullptr, st_);
 }
 
 int Engine::encode_device(uint8_t quality, uint8_t wavelet, const uint8_t *const *d_rgb, uint32_t n,
@@ -417,7 +425,7 @@ int Engine::encode_device(uint8_t quality, uint8_t wavelet, const uint8_t *const
         c += m;
     }
     CU_TRY(cudaEventRecord(ev_[1], st_));
-    build_tables(d_hist_, (int)n * 3, 256, d_enc_, d_dec_lut_, d_aux_, nullptr, nullptr, nullptr, st_);
+    build_encode_tables(n);
     CU_TRY(cudaEventRecord(ev_[2], st_));
     int rc = run_rans_encode(n);
     if (rc) return rc;
@@ -468,7 +476,7 @@ int Engine::encode_finish(uint32_t n) {
     if (n != submitted_) { set_error(kErrBufferSize, "collect: chunk count differs from the chunks submitted"); return kErrBufferSize; }
     last_n = n;
     CU_TRY(cudaEventRecord(ev_[1], st_));
-    build_tables(d_hist_, (int)n * 3, 256, d_enc_, d_dec_lut_, d_aux_, nullptr, nullptr, nullptr, st_);
+    build_encode_tables(n);
     CU_TRY(cudaEventRecord(ev_[2], st_));
     int rc = run_rans_encode(n);
     if (rc) { last_n = 0; return rc; }
@@ -604,7 +612,7 @@ int Engine::decode_resident_begin(uint32_t n) {
     const uint32_t S = n * 3;
     resident_decoded_ = 0;
     CU_TRY(cudaEventRecord(ev_[4], st_));
-    build_tables(d_hist_, (int)S, 256, d_enc_, d_dec_lut_, d_aux_, nullptr, nullptr, nullptr, st_);
+    build_tables(d_tab_hist_, (int)S, 256, d_enc_, d_dec_lut_, d_aux_, nullptr, nullptr, nullptr, st_);
     CU_TRY(cudaEventRecord(ev_[5], st_));
     for (uint32_t s = 0; s < S; s++) {
         h_dec_jobs_[s].in = stream_base_[s] + stream_off_[s];
@@ -647,7 +655,7 @@ int Engine::decode_device_resident(uint8_t *const *d_rgb_out, uint32_t n) {
     const size_t N = (size_t)d_.padded;
     const uint32_t S = n * 3;
     CU_TRY(cudaEventRecord(ev_[4], st_));
-    build_tables(d_hist_, (int)S, 256, d_enc_, d_dec_lut_, d_aux_, nullptr, nullptr, nullptr, st_);
+    build_tables(d_tab_hist_, (int)S, 256, d_enc_, d_dec_lut_, d_aux_, nullptr, nullptr, nullptr, st_);
     CU_TRY(cudaEventRecord(ev_[5], st_));
     for (uint32_t s = 0; s < S; s++) {
         h_dec_jobs_[s].in = stream_base_[s] + stream_off_[s];
@@ -790,6 +798,7 @@ bool Engine::ensure_rate_buffers() {
     a = a && dev_alloc(d_coef_, 3 * N * sizeof(int32_t), dev_bytes_);
     a = a && dev_alloc(d_vhist_, 3 * (2 * (size_t)bound + 1) * sizeof(unsigned), dev_bytes_);
     a = a && dev_alloc(d_rate_hist_, S * 256 * sizeof(unsigned), dev_bytes_);
+    if (well_formed_) a = a && dev_alloc(d_rate_wf_hist_, S * 256 * sizeof(unsigned), dev_bytes_);
     a = a && dev_alloc(d_rate_enc_, S * 256 * sizeof(EncSym), dev_bytes_);
     a = a && dev_alloc(d_rate_lut_, S * kDecLutEntries * sizeof(uint32_t), dev_bytes_);
     a = a && dev_alloc(d_rate_aux_, S * sizeof(DecAux), dev_bytes_);
@@ -799,11 +808,11 @@ bool Engine::ensure_rate_buffers() {
     if (!a) {
         cudaGetLastError();
         // leave the engine as it was: a later call retries
-        cudaFree(d_coef_); cudaFree(d_vhist_); cudaFree(d_rate_hist_); cudaFree(d_rate_enc_); cudaFree(d_rate_lut_);
-        cudaFree(d_rate_aux_); cudaFree(d_rate_est_); cudaFree(d_rate_out_);
+        cudaFree(d_coef_); cudaFree(d_vhist_); cudaFree(d_rate_hist_); cudaFree(d_rate_wf_hist_); cudaFree(d_rate_enc_);
+        cudaFree(d_rate_lut_); cudaFree(d_rate_aux_); cudaFree(d_rate_est_); cudaFree(d_rate_out_);
         if (h_rate_out_) cudaFreeHost(h_rate_out_);
-        d_coef_ = nullptr; d_vhist_ = nullptr; d_rate_hist_ = nullptr; d_rate_enc_ = nullptr; d_rate_lut_ = nullptr;
-        d_rate_aux_ = nullptr; d_rate_est_ = nullptr; d_rate_out_ = nullptr; h_rate_out_ = nullptr;
+        d_coef_ = nullptr; d_vhist_ = nullptr; d_rate_hist_ = nullptr; d_rate_wf_hist_ = nullptr; d_rate_enc_ = nullptr;
+        d_rate_lut_ = nullptr; d_rate_aux_ = nullptr; d_rate_est_ = nullptr; d_rate_out_ = nullptr; h_rate_out_ = nullptr;
         set_error(kErrCuda, "device or pinned memory allocation failed (rate curve)");
         return false;
     }
@@ -838,7 +847,10 @@ int Engine::rate_curve(uint8_t wavelet, const uint8_t *d_rgb, uint64_t bytes[kRa
     CU_TRY(cudaMemsetAsync(d_rate_out_ + kRateSteps, 0, sizeof(unsigned long long), st_));
     coef_value_hist(d_coef_, N, bound, d_vhist_, d_rate_out_ + kRateSteps, st_);
     step_hists(d_vhist_, bound, N, d_rate_hist_, st_);
-    build_tables(d_rate_hist_, kRateSteps * 3, 256, d_rate_enc_, d_rate_lut_, d_rate_aux_, nullptr, nullptr, nullptr, st_);
+    // the tables the encode at each step would use; the estimate and the zero-frequency check take the symbol counts
+    if (well_formed_) well_formed_hists(d_rate_hist_, kRateSteps * 3, d_rate_wf_hist_, st_);
+    build_tables(well_formed_ ? d_rate_wf_hist_ : d_rate_hist_, kRateSteps * 3, 256, d_rate_enc_, d_rate_lut_, d_rate_aux_,
+                 nullptr, nullptr, nullptr, st_);
     estimate_stream_bytes(d_rate_hist_, d_rate_enc_, kRateSteps * 3, N, d_rate_est_, st_);
     rate_sizes(d_rate_hist_, d_rate_enc_, d_rate_est_, N, kFixedHeaderBytes + 3 * kChannelHeaderBytes, d_rate_out_, st_);
     CU_TRY(cudaMemcpyAsync(h_rate_out_, d_rate_out_, (kRateSteps + 1) * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st_));
@@ -869,12 +881,13 @@ uint64_t g_stamp = 0;
 constexpr size_t kMaxIdleEngines = 2;
 }  // namespace
 
-Engine *acquire_engine(const Dims &d) {
+Engine *acquire_engine(const Dims &d, bool well_formed_tables) {
     int dev = 0;
     cudaGetDevice(&dev);
     std::lock_guard<std::mutex> lk(g_pool_mu);
     for (PoolEntry &p : g_pool)
-        if (!p.busy && p.device == dev && p.eng->dims().w == d.w && p.eng->dims().h == d.h && p.eng->dims().f == d.f) {
+        if (!p.busy && p.device == dev && p.eng->dims().w == d.w && p.eng->dims().h == d.h && p.eng->dims().f == d.f &&
+            p.eng->well_formed_tables() == well_formed_tables) {
             p.busy = true;
             p.stamp = ++g_stamp;
             return p.eng.get();
@@ -890,12 +903,12 @@ Engine *acquire_engine(const Dims &d) {
         if (idle < kMaxIdleEngines || oldest == g_pool.size()) break;
         g_pool.erase(g_pool.begin() + (long)oldest);
     }
-    std::unique_ptr<Engine> e(new Engine(d, 1, 0, nullptr, true));
+    std::unique_ptr<Engine> e(new Engine(d, 1, 0, nullptr, true, false, well_formed_tables));
     if (!e->ok()) {
         // out of memory: release every idle engine and retry once
         for (size_t i = g_pool.size(); i-- > 0;)
             if (!g_pool[i].busy) g_pool.erase(g_pool.begin() + (long)i);
-        e.reset(new Engine(d, 1, 0, nullptr, true));
+        e.reset(new Engine(d, 1, 0, nullptr, true, false, well_formed_tables));
         if (!e->ok()) return nullptr;
     }
     PoolEntry p;

@@ -84,8 +84,11 @@ public:
     // shared_workspace: the engine owns no symbol planes; every chunk's planes live in a caller-provided buffer of
     // workspace_bytes() (device-pointer calls; it may be the buffer the chunk is later decoded into) or in the
     // chunk's RGB staging buffer (host-pointer calls)
+    // well_formed_tables: every encode stores, instead of a channel's symbol counts, the table specification that
+    // well_formed_hists derives from them (DESIGN.md 4.8), and builds its rANS tables from that; the rate curve bounds
+    // those encodes.  A property of the engine: the decode paths read whatever the headers hold.
     Engine(const Dims &d, uint32_t cap_chunks, uint64_t payload_cap_per_stream, cudaStream_t user_stream,
-           bool own_stream, bool shared_workspace = false);
+           bool own_stream, bool shared_workspace = false, bool well_formed_tables = false);
     // prefer_small_smem: take the two-kernel front-end / back-end (k_forward.cu / k_inverse.cu: no shared memory to speak
     // of) instead of the fused kernels (one 106-210 KB block per SM).  For batches that run NEXT TO other batches' rANS
     // launches: a fused block cannot start on an SM whose shared memory is held by eight resident rANS streams and waits
@@ -93,6 +96,7 @@ public:
     void set_prefer_small_smem(bool v) { small_smem_ = v; }
     uint64_t workspace_bytes() const { return 3 * d_.padded; }
     bool shared_workspace() const { return shared_ws_; }
+    bool well_formed_tables() const { return well_formed_; }
     ~Engine();
     bool ok() const { return ok_; }
     const Dims &dims() const { return d_; }
@@ -131,7 +135,7 @@ public:
                       uint8_t *const *h_rgb_out = nullptr);
 
     // Rate curve of one chunk (k_rate.cu): bytes[i] = an upper bound on the .alc length an encode at step i + 1 gives
-    // (UINT64_MAX where the reference aborts), h_hist_out (host, optional) = the symbol histograms [64][3][256] of every
+    // (UINT64_MAX where the reference aborts; never for well-formed-tables engines), h_hist_out (host, optional) = the symbol histograms [64][3][256] of every
     // step.  Runs the front-end with the coefficient dump into chunk slot `slot` (its histogram and symbol planes, or
     // d_work for shared-workspace engines, are scratch until that chunk's real front-end), then the value histogram,
     // the step histograms, the table build and the estimate; one synchronisation.  The buffers it needs (12 B per padded
@@ -150,6 +154,7 @@ public:
 
 private:
     int run_rans_encode(uint32_t n);
+    void build_encode_tables(uint32_t n);
     struct BackendHeader { uint8_t wavelet; int steps[3]; };   // what the back-end needs from a chunk's headers
     int run_backend(uint32_t n, const BackendHeader *hdr, uint8_t *const *d_rgb_out);
     int backend_one(uint32_t c, const BackendHeader &hdr, uint8_t *d_rgb_out);
@@ -167,7 +172,10 @@ private:
     std::vector<uint8_t *> sym_ptr_;  // per chunk: where its symbol planes [3][N] live
     bool shared_ws_ = false;
     bool small_smem_ = false;
-    unsigned *d_hist_ = nullptr;      // [cap][3][256]
+    unsigned *d_hist_ = nullptr;      // [cap][3][256] symbol counts
+    bool well_formed_ = false;
+    unsigned *d_wf_hist_ = nullptr;   // [cap][3][256] table specifications (well-formed engines only)
+    unsigned *d_tab_hist_ = nullptr;  // what encode tables are built from and headers store: d_wf_hist_ or d_hist_
     EncSym *d_enc_ = nullptr;         // [cap*3][256]
     uint32_t *d_dec_lut_ = nullptr;   // [cap*3][4096]
     DecAux *d_aux_ = nullptr;         // [cap*3]
@@ -189,6 +197,7 @@ private:
     int32_t *d_coef_ = nullptr;                // i32 [3][N] coefficients
     unsigned *d_vhist_ = nullptr;              // [3][2*bound+1] value histogram (largest bound of the three wavelets)
     unsigned *d_rate_hist_ = nullptr;          // [64][3][256]
+    unsigned *d_rate_wf_hist_ = nullptr;       // [64][3][256] table specifications (well-formed engines only)
     EncSym *d_rate_enc_ = nullptr;             // [192][256]
     uint32_t *d_rate_lut_ = nullptr;           // [192][4096] (built, not read)
     DecAux *d_rate_aux_ = nullptr;             // [192]
@@ -206,7 +215,8 @@ private:
 };
 
 // Pool of single-chunk engines behind the reference-ABI entry points (alice_codec_encode / _decode).
-Engine *acquire_engine(const Dims &d);
+// A well-formed-tables engine only ever serves well_formed_tables calls, and the reverse.
+Engine *acquire_engine(const Dims &d, bool well_formed_tables = false);
 void release_engine(Engine *e);
 bool cuda_ready();   // a device is present and usable; sets the CUDA error otherwise
 void trim_pinned_pool();   // release the idle page-locked payload buffers (ByteBuf pool)

@@ -55,6 +55,40 @@ ALICE_D uint32_t pack_dec(uint32_t sym, uint32_t freq, uint32_t bias) {
     return sym | (fm1 << 8) | (bias << 20);
 }
 
+// FrequencyTable::from_histogram of one stream (rans.rs:102-125; uniform, rans.rs:158-189, for an all-zero histogram):
+// freq / cum of symbols [0, n), 0 above.  The normalisation is a serial running sum in the reference; 256 entries are
+// cheap enough to do exactly that on one thread.
+ALICE_D void normalise_table(const unsigned *h, int n, uint32_t *s_freq, uint32_t *s_cum) {
+    unsigned long long total = 0;
+    for (int i = 0; i < n; i++) total += h[i];
+    if (total == 0) {
+        // u16 arithmetic
+        uint16_t fps = (uint16_t)(kProbScale / (uint32_t)n);
+        uint16_t cum = 0;
+        for (int i = 0; i < n; i++) { s_cum[i] = cum; s_freq[i] = fps; cum = (uint16_t)(cum + fps); }
+        s_freq[n - 1] = (uint16_t)((uint16_t)kProbScale - (uint16_t)s_cum[n - 1]);
+    } else {
+        uint32_t cum = 0, norm = 0;
+        for (int i = 0; i < n; i++) {
+            uint32_t c = h[i];
+            uint32_t fr = 1;
+            if (c != 0) {
+                unsigned long long t = ((unsigned long long)c * kProbScale) / total;
+                fr = t < 1 ? 1u : (uint32_t)t;
+            }
+            norm += fr;
+            s_cum[i] = (uint16_t)cum;
+            s_freq[i] = (uint16_t)fr;
+            cum += fr;
+        }
+        if (norm != kProbScale) {
+            int diff = (int)kProbScale - (int)norm;
+            s_freq[n - 1] = (uint16_t)((int)s_freq[n - 1] + diff);
+        }
+    }
+    for (int i = n; i < 256; i++) { s_freq[i] = 0; s_cum[i] = 0; }
+}
+
 __global__ void ALICE_LAUNCH_BOUNDS(256, 1)
 k_build_tables(const unsigned *__restrict__ hist, int n_symbols, EncSym *__restrict__ enc,
                uint32_t *__restrict__ dec_lut, DecAux *__restrict__ aux, uint16_t *__restrict__ freq_out,
@@ -66,37 +100,8 @@ k_build_tables(const unsigned *__restrict__ hist, int n_symbols, EncSym *__restr
     const unsigned *h = hist + (size_t)stream * 256;
     const int n = n_symbols;
 
-    // The normalisation is a serial running sum in the reference (rans.rs:113-125); 256 entries
-    // are cheap enough to do exactly that on one thread.
     if (tid == 0) {
-        unsigned long long total = 0;
-        for (int i = 0; i < n; i++) total += h[i];
-        if (total == 0) {
-            // FrequencyTable::uniform (rans.rs:158-189), u16 arithmetic
-            uint16_t fps = (uint16_t)(kProbScale / (uint32_t)n);
-            uint16_t cum = 0;
-            for (int i = 0; i < n; i++) { s_cum[i] = cum; s_freq[i] = fps; cum = (uint16_t)(cum + fps); }
-            s_freq[n - 1] = (uint16_t)((uint16_t)kProbScale - (uint16_t)s_cum[n - 1]);
-        } else {
-            uint32_t cum = 0, norm = 0;
-            for (int i = 0; i < n; i++) {
-                uint32_t c = h[i];
-                uint32_t fr = 1;
-                if (c != 0) {
-                    unsigned long long t = ((unsigned long long)c * kProbScale) / total;
-                    fr = t < 1 ? 1u : (uint32_t)t;
-                }
-                norm += fr;
-                s_cum[i] = (uint16_t)cum;
-                s_freq[i] = (uint16_t)fr;
-                cum += fr;
-            }
-            if (norm != kProbScale) {
-                int diff = (int)kProbScale - (int)norm;
-                s_freq[n - 1] = (uint16_t)((int)s_freq[n - 1] + diff);
-            }
-        }
-        for (int i = n; i < 256; i++) { s_freq[i] = 0; s_cum[i] = 0; }
+        normalise_table(h, n, s_freq, s_cum);
         const uint32_t fl = s_freq[n - 1];
         const bool last_wide = !(fl >= 1 && fl <= kProbScale);
         DecAux a;
@@ -159,6 +164,90 @@ void build_tables(const unsigned *d_hist, int n_streams, int n_symbols, EncSym *
     if (n_streams <= 0) return;
     ALICE_LAUNCH(k_build_tables, dim3(n_streams), dim3(256), 0, st, d_hist, n_symbols, d_enc, d_dec_lut, d_aux,
                  d_freq, d_cum, d_lut8);
+}
+
+// ------------------------------------------------------------------ well-formed table specification
+// The histogram a well-formed-tables encode stores in a channel header (DESIGN.md 4.8), from the stream's symbol
+// counts c (N = sum c, used = c > 0):
+//   1. from_histogram(c) already gives every used symbol 1 <= f <= 4096 and cum + f <= 4096: H' = c.
+//   2. otherwise, with Z = empty bins among 0..254 and S = 4096 - Z: F[j] = max(1, c[j] * S / N) for used j, D = S - sum F;
+//      D > 0: +1 for the D used symbols with the largest c[j] * S mod N (ties to the lower index); D < 0: -1 from the
+//      used symbol with the largest F > 1 (ties to the lower index), -D times.  H'[j] = F[j] for used j < 255, 0 for
+//      empty j < 255, H'[255] = 4096 - sum of F[j] over used j < 255.
+// H' sums to 4096, so from_histogram(H') gives every used j < 255 exactly F[j], every empty bin 1 and symbol 255 the
+// rest: every used range lies inside [0, 4096), and every decoder of the format decodes the stream exactly.
+__global__ void ALICE_LAUNCH_BOUNDS(256, 1)
+k_well_formed_hists(const unsigned *__restrict__ counts, unsigned *__restrict__ out) {
+    __shared__ uint32_t s_freq[256];
+    __shared__ uint32_t s_cum[256];
+    __shared__ unsigned long long s_rem[256];
+    __shared__ unsigned long long s_total;
+    __shared__ int s_clean, s_empty, s_d;
+    __shared__ uint32_t s_head;          // sum of F over symbols 0..254
+    const int stream = blockIdx.x, tid = threadIdx.x;
+    const unsigned *c = counts + (size_t)stream * 256;
+    unsigned *o = out + (size_t)stream * 256;
+    const unsigned cj = c[tid];
+    if (tid == 0) {
+        normalise_table(c, 256, s_freq, s_cum);
+        unsigned long long total = 0;
+        int clean = 1, empty = 0;
+        for (int i = 0; i < 256; i++) {
+            total += c[i];
+            if (c[i]) clean &= (s_freq[i] >= 1 && s_freq[i] <= kProbScale && s_cum[i] + s_freq[i] <= kProbScale);
+            else if (i < 255) empty++;
+        }
+        s_total = total;
+        s_clean = clean;
+        s_empty = empty;
+    }
+    __syncthreads();
+    if (s_clean) { o[tid] = cj; return; }    // block-uniform; also every all-zero histogram (no used symbol)
+    const unsigned long long n = s_total, scale = kProbScale - (unsigned long long)s_empty;
+    const unsigned long long prod = (unsigned long long)cj * scale;
+    const unsigned long long q = prod / n;
+    uint32_t f = cj ? (q < 1 ? 1u : (uint32_t)q) : 0u;   // f > 0 marks a used symbol below
+    s_freq[tid] = f;
+    s_rem[tid] = prod % n;
+    __syncthreads();
+    if (tid == 0) {
+        long long sum = 0;
+        for (int i = 0; i < 256; i++) sum += s_freq[i];
+        s_d = (int)((long long)scale - sum);
+    }
+    __syncthreads();
+    const int d = s_d;
+    if (d > 0 && cj) {   // rank among the used symbols by (remainder descending, index ascending)
+        const unsigned long long r = s_rem[tid];
+        int rank = 0;
+        for (int k = 0; k < 256; k++) {
+            const unsigned long long rk = s_rem[k];
+            rank += (s_freq[k] != 0 && (rk > r || (rk == r && k < tid))) ? 1 : 0;
+        }
+        if (rank < d) f++;
+    }
+    __syncthreads();
+    s_freq[tid] = f;
+    __syncthreads();
+    if (tid == 0) {
+        // at most one step per symbol that max(1, .) raised; some used symbol keeps F > 1 since used <= S
+        for (int k = d; k < 0; k++) {
+            int best = -1;
+            for (int i = 0; i < 256; i++)
+                if (s_freq[i] > 1 && (best < 0 || s_freq[i] > s_freq[best])) best = i;
+            s_freq[best]--;
+        }
+        uint32_t head = 0;
+        for (int i = 0; i < 255; i++) head += s_freq[i];
+        s_head = head;
+    }
+    __syncthreads();
+    o[tid] = tid < 255 ? s_freq[tid] : kProbScale - s_head;
+}
+
+void well_formed_hists(const unsigned *d_counts, int n_streams, unsigned *d_out, cudaStream_t st) {
+    if (n_streams <= 0) return;
+    ALICE_LAUNCH(k_well_formed_hists, dim3(n_streams), dim3(256), 0, st, d_counts, d_out);
 }
 
 // ------------------------------------------------------------------- stream size estimate

@@ -64,6 +64,10 @@ constexpr int kDecLutEntries = 4096;
 void build_tables(const unsigned *d_hist, int n_streams, int n_symbols, EncSym *d_enc, uint32_t *d_dec_lut,
                   DecAux *d_aux, uint16_t *d_freq, uint16_t *d_cum, uint8_t *d_lut8, cudaStream_t st);
 
+// out [n_streams][256] = the well-formed table specification of each stream's symbol counts (rule in k_rans.cu,
+// DESIGN.md 4.8): a histogram whose from_histogram table keeps every used symbol's range inside [0, 4096)
+void well_formed_hists(const unsigned *d_counts, int n_streams, unsigned *d_out, cudaStream_t st);
+
 // est[i] = upper bound on the bytes stream i will take (multiple of 16, includes the encoder's slack), from hist + enc
 void estimate_stream_bytes(const unsigned *d_hist, const EncSym *d_enc, int n_streams, unsigned long long n_symbols,
                            unsigned long long *d_est, cudaStream_t st);

@@ -85,6 +85,18 @@ enum { ALICE_WAVELET_CDF53 = 0, ALICE_WAVELET_CDF97 = 1, ALICE_WAVELET_HAAR = 2 
 
 /* FrameEncoder::with_wavelet (pipeline.rs:356); null if wavelet > 2 */
 FrameEncoder *alice_codec_encoder_create_with_wavelet(uint8_t quality, uint8_t wavelet);
+/* ALICE_ENCODE_WELL_FORMED_TABLES — encodes whose chunks decode exactly on every decoder of the format.  The default
+ * encode stores each channel's symbol counts, and the table FrequencyTable::from_histogram derives from them gives
+ * every empty bin a frequency of 1; where empty bins lie below used symbols, the ranges of the high symbols run past
+ * 4096 and the stream does not decode to what was encoded (SURVEY.md 0.7).  In this mode the 256-bin histogram of a
+ * channel header is a TABLE SPECIFICATION that sums to 4096, not the symbol counts: the counts themselves where their
+ * table is already well formed (the chunk is then byte-identical to the default encode), otherwise the counts scaled
+ * to the 4096 - (empty bins among 0..254) slots left by the empty bins, with the rest on symbol 255 (DESIGN.md 4.8).
+ * The .alc format and every decoder, including the reference's, are unchanged; where the rule rescales, a chunk costs a
+ * few percent more bytes than the default encode.  Unknown flag bits: null, ALICE_ERR_DIMENSIONS. */
+enum { ALICE_ENCODE_WELL_FORMED_TABLES = 1 };
+/* with_wavelet + flags; alice_codec_encode and alice_codec_encode_stages honour the encoder's flags */
+FrameEncoder *alice_codec_encoder_create_ex(uint8_t quality, uint8_t wavelet, uint32_t flags);
 uint8_t alice_codec_chunk_wavelet(const EncodedChunk *chunk);                  /* EncodedChunk::wavelet_type */
 uint64_t alice_codec_chunk_compressed_size(const EncodedChunk *chunk);         /* pipeline.rs:190 */
 /* per-channel header fields (pipeline.rs:123-134); hist256 may be null */
@@ -213,7 +225,10 @@ AliceBatch *alice_codec_batch_create(uint8_t quality, uint8_t wavelet, uint32_t 
  * of the fused kernels (one 106-210 KB block per SM).  For batches that run NEXT TO other batches' rANS launches (several
  * host threads, one batch each): a fused block cannot start on an SM whose shared memory is held by resident rANS streams
  * and would wait for a whole rANS launch to end; the small kernels slip in beside them.  Same results. */
-enum { ALICE_BATCH_SHARED_WORKSPACE = 1, ALICE_BATCH_SMALL_SMEM_KERNELS = 2 };
+/* ALICE_BATCH_WELL_FORMED_TABLES — every encode of the batch (encode_host_to_size included) stores well-formed table
+ * specifications as ALICE_ENCODE_WELL_FORMED_TABLES does; alice_codec_batch_decode_device builds its tables from them.
+ * Costs 3 KiB per chunk of device memory. */
+enum { ALICE_BATCH_SHARED_WORKSPACE = 1, ALICE_BATCH_SMALL_SMEM_KERNELS = 2, ALICE_BATCH_WELL_FORMED_TABLES = 4 };
 AliceBatch *alice_codec_batch_create_ex(uint8_t quality, uint8_t wavelet, uint32_t width, uint32_t height,
                                         uint32_t frames, uint32_t n_chunks, void *cuda_stream, uint32_t flags);
 /* payload_bytes_per_chunk: device memory reserved for the encoded payload, per chunk on average (0 = the default, one
@@ -289,6 +304,16 @@ int alice_codec_rate_curve_device(uint8_t wavelet, const uint8_t *d_rgb, uint32_
  * null, ALICE_ERR_BUFFER_SIZE, and the message names the smallest predicted size */
 EncodedChunk *alice_codec_encode_to_size(uint8_t wavelet, const uint8_t *rgb, uint64_t rgb_len, uint32_t width,
                                          uint32_t height, uint32_t frames, uint64_t max_bytes, uint8_t *quality_out);
+/* the three calls above for encodes with ALICE_ENCODE_WELL_FORMED_TABLES flags (0 = the calls above): the curve then
+ * bounds the well-formed encode at every step and has no UINT64_MAX entry; hist_out still holds the symbol counts */
+int alice_codec_rate_curve_ex(uint8_t wavelet, const uint8_t *rgb, uint64_t rgb_len, uint32_t width, uint32_t height,
+                              uint32_t frames, uint64_t *bytes64, uint32_t *hist_out, uint32_t flags);
+int alice_codec_rate_curve_device_ex(uint8_t wavelet, const uint8_t *d_rgb, uint32_t width, uint32_t height,
+                                     uint32_t frames, uint64_t *bytes64, uint32_t *hist_out, void *cuda_stream,
+                                     uint32_t flags);
+EncodedChunk *alice_codec_encode_to_size_ex(uint8_t wavelet, const uint8_t *rgb, uint64_t rgb_len, uint32_t width,
+                                            uint32_t height, uint32_t frames, uint64_t max_bytes, uint8_t *quality_out,
+                                            uint32_t flags);
 /* host-buffer batch, every chunk with its own quality under the same per-chunk budget; all 3n rANS streams run
  * concurrently as in alice_codec_batch_encode_host.  The batch's own quality is not used.  The first rate call on a
  * batch allocates 12 B per padded pixel of coefficients plus ~4 MB of tables (alice_codec_batch_device_bytes grows). */
