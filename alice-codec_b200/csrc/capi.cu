@@ -137,6 +137,17 @@ int validate_encode(uint64_t rgb_len, uint32_t w, uint32_t h, uint32_t f, Dims &
     return kOk;
 }
 
+// Stage 0 of a pooled single-chunk engine, with the copy of the host chunk `rgb` enqueued on the engine's stream; null
+// (error set) on failure.
+const uint8_t *stage_host_chunk(Engine *e, const uint8_t *rgb, uint64_t rgb_len) {
+    uint8_t *stage = e->rgb_stage(0);
+    if (stage && cudaMemcpyAsync(stage, rgb, (size_t)rgb_len, cudaMemcpyHostToDevice, e->stream()) != cudaSuccess) {
+        set_error(kErrCuda, "H2D copy failed");
+        return nullptr;
+    }
+    return stage;
+}
+
 EncodedChunk *encode_impl(const FrameEncoder *enc, const uint8_t *rgb, uint64_t rgb_len, uint32_t w, uint32_t h,
                           uint32_t f, int32_t *coeffs_out, uint8_t *symbols_out) {
     set_error(0, "");
@@ -155,11 +166,8 @@ EncodedChunk *encode_impl(const FrameEncoder *enc, const uint8_t *rgb, uint64_t 
     int rc = kOk;
     DevBuf coef;
     do {
-        uint8_t *stage = e->rgb_stage(0);
+        const uint8_t *stage = stage_host_chunk(e, rgb, rgb_len);
         if (!stage) { rc = kErrCuda; break; }
-        if (cudaMemcpyAsync(stage, rgb, (size_t)rgb_len, cudaMemcpyHostToDevice, e->stream()) != cudaSuccess) {
-            set_error(kErrCuda, "H2D copy failed"); rc = kErrCuda; break;
-        }
         if (coeffs_out && !coef.alloc((size_t)d.padded * 3 * 4)) { rc = kErrCuda; break; }
         const uint8_t *ptrs[1] = {stage};
         rc = e->encode_device(enc->quality, enc->wavelet, ptrs, 1, coef.as<int32_t>());
@@ -239,12 +247,8 @@ int rate_curve_impl(uint8_t wavelet, const uint8_t *rgb, bool device, uint64_t r
             cudaEventDestroy(ev);
             if (ce != cudaSuccess) { cudaGetLastError(); set_error(kErrCuda, "stream ordering failed"); rc = kErrCuda; break; }
         } else {
-            uint8_t *stage = e->rgb_stage(0);
-            if (!stage) { rc = kErrCuda; break; }
-            if (cudaMemcpyAsync(stage, rgb, (size_t)rgb_len, cudaMemcpyHostToDevice, e->stream()) != cudaSuccess) {
-                set_error(kErrCuda, "H2D copy failed"); rc = kErrCuda; break;
-            }
-            src = stage;
+            src = stage_host_chunk(e, rgb, rgb_len);
+            if (!src) { rc = kErrCuda; break; }
         }
         rc = e->rate_curve(wavelet, src, bytes64, hist_out);
     } while (0);
@@ -279,11 +283,8 @@ EncodedChunk *encode_to_size_impl(uint8_t wavelet, const uint8_t *rgb, uint64_t 
     if (!e) return nullptr;
     EncodedChunk *out = nullptr;
     do {
-        uint8_t *stage = e->rgb_stage(0);
+        const uint8_t *stage = stage_host_chunk(e, rgb, rgb_len);
         if (!stage) break;
-        if (cudaMemcpyAsync(stage, rgb, (size_t)rgb_len, cudaMemcpyHostToDevice, e->stream()) != cudaSuccess) {
-            set_error(kErrCuda, "H2D copy failed"); break;
-        }
         uint64_t pred[kRateSteps];
         if (e->rate_curve(wavelet, stage, pred, nullptr)) break;
         const uint8_t *ptrs[1] = {stage};
@@ -1081,6 +1082,38 @@ uint8_t *alice_codec_decode_stages(const EncodedChunk *chunk, uint64_t *out_len,
 }
 
 // ------------------------------------------------------------------------------ batch API
+namespace {
+// Host staging of chunk i of a batch: `rgb` receives its RGB, `work` its symbol planes (null: the engine's own).
+// Shared-workspace batches keep the symbol planes of chunk i in the RGB staging buffer of chunk i - 1 (chunk 0: one spare
+// buffer): the front-end of chunk i runs after that of chunk i - 1 has consumed its RGB, and a workspace that is not the
+// chunk's own RGB lets the fused kernels run.  A decode writes chunk i's RGB over the planes of chunk i + 1, which the
+// back-end's descending order has consumed by then (Engine::run_backend).
+// Batches that own their symbol planes need ONE staging buffer: copy, front-end, next chunk, all in stream order, so a
+// chunk in flight costs 3 B/px (its symbol planes) + its payload, not 3 B/px more for its RGB.
+bool host_stage(Engine *e, uint32_t i, uint8_t *&rgb, uint8_t *&work) {
+    const bool shared = e->shared_workspace();
+    rgb = e->rgb_stage(shared ? i + 1 : 0);
+    work = shared ? e->rgb_stage(i) : nullptr;
+    return rgb && (work || !shared);
+}
+
+// n new chunks filled from the engine's last encode (every payload copy enqueued, one synchronisation); on failure none
+// is left allocated
+int fetch_new_chunks(Engine *e, uint32_t n, EncodedChunk **out_chunks) {
+    int rc = kOk;
+    std::vector<Chunk *> cks(n);
+    for (uint32_t i = 0; i < n; i++) {
+        out_chunks[i] = new (std::nothrow) EncodedChunk();
+        if (!out_chunks[i]) { rc = kErrCuda; set_error(kErrCuda, "host allocation failed"); }
+        else cks[i] = &out_chunks[i]->c;
+    }
+    if (!rc) rc = e->fetch_chunks(n, cks.data());
+    if (rc)
+        for (uint32_t k = 0; k < n; k++) { delete out_chunks[k]; out_chunks[k] = nullptr; }
+    return rc;
+}
+}  // namespace
+
 AliceBatch *alice_codec_batch_create(uint8_t quality, uint8_t wavelet, uint32_t w, uint32_t h, uint32_t f,
                                      uint32_t n_chunks, void *cuda_stream) {
     return alice_codec_batch_create_ex(quality, wavelet, w, h, f, n_chunks, cuda_stream, 0);
@@ -1149,52 +1182,11 @@ EncodedChunk *alice_codec_batch_get_chunk(AliceBatch *b, uint32_t i) {
 int alice_codec_batch_encode_host(AliceBatch *b, const uint8_t *const *h_rgb, uint32_t n, EncodedChunk **out_chunks) {
     set_error(0, "");
     if (!b || !h_rgb || !out_chunks) { set_error(kErrNull, "null argument"); return kErrNull; }
-    Engine *e = b->eng;
-    if (n > e->cap_chunks()) { set_error(kErrBufferSize, "batch larger than capacity"); return kErrBufferSize; }
-    const size_t bytes = (size_t)e->dims().n_pixels * 3;
-    // Shared-workspace batches keep the symbol planes of chunk i in the RGB staging buffer of chunk i - 1 (chunk 0: one
-    // spare buffer): the front-end of chunk i runs after that of chunk i - 1 has consumed its RGB, and a workspace that is
-    // not the chunk's own RGB lets the fused front-end kernel run (Engine::encode_device).
-    // Batches that own their symbol planes need ONE staging buffer: copy, front-end, next chunk, all in stream order, so a
-    // chunk in flight costs 3 B/px (its symbol planes) + its payload, not 3 B/px more for its RGB.
-    const bool shared = e->shared_workspace();
-    int rc = kOk;
-    if (!shared) {
-        uint8_t *s = e->rgb_stage(0);
-        if (!s) return kErrCuda;
-        rc = e->encode_begin(b->quality, b->wavelet);
-        for (uint32_t i = 0; i < n && !rc; i++) {
-            if (!h_rgb[i]) { set_error(kErrNull, "null chunk pointer"); return kErrNull; }
-            CU_CHECK_RC(cudaMemcpyAsync(s, h_rgb[i], bytes, cudaMemcpyHostToDevice, e->stream()));
-            rc = e->encode_submit(i, s, nullptr);
-        }
-        if (!rc) rc = e->encode_finish(n);
-        if (rc) return rc;
-    } else {
-        b->stage_ptrs.resize(n);
-        b->work_ptrs.resize(n);
-        for (uint32_t i = 0; i < n; i++) {
-            uint8_t *s = e->rgb_stage(i + 1);
-            if (!s || !e->rgb_stage(i)) return kErrCuda;
-            b->stage_ptrs[i] = s;
-            b->work_ptrs[i] = e->rgb_stage(i);
-            CU_CHECK_RC(cudaMemcpyAsync(s, h_rgb[i], bytes, cudaMemcpyHostToDevice, e->stream()));
-        }
-        rc = e->encode_device(b->quality, b->wavelet, b->stage_ptrs.data(), n, nullptr, b->work_ptrs.data());
-        if (rc) return rc;
-    }
-    std::vector<Chunk *> cks(n);
-    for (uint32_t i = 0; i < n; i++) {
-        out_chunks[i] = new (std::nothrow) EncodedChunk();
-        if (!out_chunks[i]) { rc = kErrCuda; set_error(kErrCuda, "host allocation failed"); }
-        else cks[i] = &out_chunks[i]->c;
-    }
-    if (!rc) rc = e->fetch_chunks(n, cks.data());     // every payload copy enqueued, one synchronisation
-    if (rc) {
-        for (uint32_t k = 0; k < n; k++) { delete out_chunks[k]; out_chunks[k] = nullptr; }
-        return rc;
-    }
-    return kOk;
+    if (n > b->eng->cap_chunks()) { set_error(kErrBufferSize, "batch larger than capacity"); return kErrBufferSize; }
+    // submit_host begins the encode at chunk 0; an empty batch begins it here, so that collect finds 0 chunks submitted
+    int rc = n ? kOk : b->eng->encode_begin(b->quality, b->wavelet);
+    for (uint32_t i = 0; i < n && !rc; i++) rc = alice_codec_batch_submit_host(b, i, h_rgb[i]);
+    return rc ? rc : alice_codec_batch_collect(b, n, out_chunks);
 }
 // Chunk-at-a-time form of alice_codec_batch_encode_host: submit chunk 0, 1, ... as they arrive (the host -> device copy
 // and the front-end of that chunk are enqueued and the call returns at once), then collect.  The host does not have to
@@ -1204,16 +1196,14 @@ int alice_codec_batch_submit_host(AliceBatch *b, uint32_t i, const uint8_t *h_rg
     if (!b || !h_rgb) { set_error(kErrNull, "null argument"); return kErrNull; }
     Engine *e = b->eng;
     if (i >= e->cap_chunks()) { set_error(kErrBufferSize, "chunk index beyond the batch capacity"); return kErrBufferSize; }
-    const size_t bytes = (size_t)e->dims().n_pixels * 3;
-    const bool shared = e->shared_workspace();
     if (i == 0) {
         int rc = e->encode_begin(b->quality, b->wavelet);
         if (rc) return rc;
     }
-    uint8_t *s = e->rgb_stage(shared ? i + 1 : 0);     // engine-owned symbol planes: one staging buffer for every chunk
-    if (!s || (shared && !e->rgb_stage(i))) return kErrCuda;
-    CU_CHECK_RC(cudaMemcpyAsync(s, h_rgb, bytes, cudaMemcpyHostToDevice, e->stream()));
-    return e->encode_submit(i, s, shared ? e->rgb_stage(i) : nullptr);
+    uint8_t *s, *work;
+    if (!host_stage(e, i, s, work)) return kErrCuda;
+    CU_CHECK_RC(cudaMemcpyAsync(s, h_rgb, (size_t)e->dims().n_pixels * 3, cudaMemcpyHostToDevice, e->stream()));
+    return e->encode_submit(i, s, work);
 }
 // Device-pointer form of submit / collect: chunk i's RGB is already on the device (d_workspace as in
 // alice_codec_batch_encode_device_ws, null for batches that own their symbol planes).  Work is enqueued on the batch's stream
@@ -1252,21 +1242,8 @@ int alice_codec_batch_decode_end(AliceBatch *b) {
 int alice_codec_batch_collect(AliceBatch *b, uint32_t n, EncodedChunk **out_chunks) {
     set_error(0, "");
     if (!b || !out_chunks) { set_error(kErrNull, "null argument"); return kErrNull; }
-    Engine *e = b->eng;
-    int rc = e->encode_finish(n);
-    if (rc) return rc;
-    std::vector<Chunk *> cks(n);
-    for (uint32_t i = 0; i < n; i++) {
-        out_chunks[i] = new (std::nothrow) EncodedChunk();
-        if (!out_chunks[i]) { rc = kErrCuda; set_error(kErrCuda, "host allocation failed"); }
-        else cks[i] = &out_chunks[i]->c;
-    }
-    if (!rc) rc = e->fetch_chunks(n, cks.data());
-    if (rc) {
-        for (uint32_t k = 0; k < n; k++) { delete out_chunks[k]; out_chunks[k] = nullptr; }
-        return rc;
-    }
-    return kOk;
+    int rc = b->eng->encode_finish(n);
+    return rc ? rc : fetch_new_chunks(b->eng, n, out_chunks);
 }
 int alice_codec_batch_decode_host(AliceBatch *b, const EncodedChunk *const *chunks, uint32_t n,
                                   uint8_t *const *h_rgb_out) {
@@ -1274,9 +1251,6 @@ int alice_codec_batch_decode_host(AliceBatch *b, const EncodedChunk *const *chun
     if (!b || !chunks || !h_rgb_out) { set_error(kErrNull, "null argument"); return kErrNull; }
     Engine *e = b->eng;
     if (n > e->cap_chunks()) { set_error(kErrBufferSize, "batch larger than capacity"); return kErrBufferSize; }
-    const size_t bytes = (size_t)e->dims().n_pixels * 3;
-    // shared-workspace batches: chunk i's symbol planes go to staging buffer i, its RGB to staging buffer i + 1 (the
-    // back-end runs the chunks in descending order, so that buffer's planes have been consumed: Engine::run_backend)
     const bool shared = e->shared_workspace();
     std::vector<const Chunk *> cks(n);
     b->stage_ptrs.resize(n);
@@ -1284,17 +1258,14 @@ int alice_codec_batch_decode_host(AliceBatch *b, const EncodedChunk *const *chun
     for (uint32_t i = 0; i < n; i++) {
         if (!chunks[i] || !h_rgb_out[i]) { set_error(kErrNull, "null chunk or output pointer"); return kErrNull; }
         cks[i] = &chunks[i]->c;
-        uint8_t *s = e->rgb_stage(shared ? i + 1 : 0);   // engine-owned symbol planes: one staging buffer, see encode_host
-        if (!s || (shared && !e->rgb_stage(i))) return kErrCuda;
-        b->stage_ptrs[i] = s;
-        b->work_ptrs[i] = shared ? e->rgb_stage(i) : nullptr;
+        if (!host_stage(e, i, b->stage_ptrs[i], b->work_ptrs[i])) return kErrCuda;
     }
-    if (!shared)     // back-end and device -> host copy chunk by chunk (Engine::decode_chunks synchronises at the end)
-        return e->decode_chunks(cks.data(), n, b->stage_ptrs.data(), nullptr, h_rgb_out);
-    int rc = e->decode_chunks(cks.data(), n, b->stage_ptrs.data(), b->work_ptrs.data());
-    if (rc) return rc;
+    // engine-owned symbol planes: back-end and device -> host copy chunk by chunk (Engine::decode_chunks synchronises)
+    int rc = e->decode_chunks(cks.data(), n, b->stage_ptrs.data(), b->work_ptrs.data(), shared ? nullptr : h_rgb_out);
+    if (rc || !shared) return rc;
     for (uint32_t i = 0; i < n; i++)
-        CU_CHECK_RC(cudaMemcpyAsync(h_rgb_out[i], b->stage_ptrs[i], bytes, cudaMemcpyDeviceToHost, e->stream()));
+        CU_CHECK_RC(cudaMemcpyAsync(h_rgb_out[i], b->stage_ptrs[i], (size_t)e->dims().n_pixels * 3, cudaMemcpyDeviceToHost,
+                                    e->stream()));
     CU_CHECK_RC(cudaStreamSynchronize(e->stream()));
     return kOk;
 }
@@ -1351,14 +1322,12 @@ int alice_codec_batch_encode_host_to_size(AliceBatch *b, const uint8_t *const *h
     if (n > e->cap_chunks()) { set_error(kErrBufferSize, "batch larger than capacity"); return kErrBufferSize; }
     const Dims &d = e->dims();
     const size_t bytes = (size_t)d.n_pixels * 3;
-    const bool shared = e->shared_workspace();   // staging and workspaces as in alice_codec_batch_encode_host
     std::vector<int> steps(n);
     int rc = e->encode_begin(100, b->wavelet);    // the batch's quality is not used: every chunk names its step
     for (uint32_t i = 0; i < n && !rc; i++) {
         if (!h_rgb[i]) { set_error(kErrNull, "null chunk pointer"); return kErrNull; }
-        uint8_t *s = e->rgb_stage(shared ? i + 1 : 0);
-        uint8_t *work = shared ? e->rgb_stage(i) : nullptr;
-        if (!s || (shared && !work)) return kErrCuda;
+        uint8_t *s, *work;
+        if (!host_stage(e, i, s, work)) return kErrCuda;
         CU_CHECK_RC(cudaMemcpyAsync(s, h_rgb[i], bytes, cudaMemcpyHostToDevice, e->stream()));
         uint64_t pred[kRateSteps];
         rc = e->rate_curve(b->wavelet, s, pred, nullptr, i, work);
@@ -1372,14 +1341,8 @@ int alice_codec_batch_encode_host_to_size(AliceBatch *b, const uint8_t *const *h
         rc = e->encode_submit(i, s, work, steps[i]);
     }
     if (!rc) rc = e->encode_finish(n);
+    if (!rc) rc = fetch_new_chunks(e, n, out_chunks);
     if (rc) return rc;
-    std::vector<Chunk *> cks(n);
-    for (uint32_t i = 0; i < n; i++) {
-        out_chunks[i] = new (std::nothrow) EncodedChunk();
-        if (!out_chunks[i]) { rc = kErrCuda; set_error(kErrCuda, "host allocation failed"); }
-        else cks[i] = &out_chunks[i]->c;
-    }
-    if (!rc) rc = e->fetch_chunks(n, cks.data());
     for (uint32_t i = 0; i < n && !rc; i++) {
         qualities_out[i] = quality_for_step(steps[i]);
         if (kAlcHeaderBytes + out_chunks[i]->c.data.size() <= max_bytes) continue;

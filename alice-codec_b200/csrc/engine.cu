@@ -374,9 +374,41 @@ void Engine::build_encode_tables(uint32_t n) {
     build_tables(d_tab_hist_, (int)n * 3, 256, d_enc_, d_dec_lut_, d_aux_, nullptr, nullptr, nullptr, st_);
 }
 
+// whether a chunk's symbol planes [3][N] and an RGB buffer of one chunk share bytes
+bool Engine::overlaps(const uint8_t *sym, const uint8_t *rgb) const {
+    return sym < rgb + 3 * (size_t)d_.n_pixels && rgb < sym + 3 * (size_t)d_.padded;
+}
+
+// The fused front-end (k_fwd_fused.cu) takes 64-frame chunks of even height and a width that is a multiple of 16.  It
+// reads RGB and writes symbols in the same launch, so a chunk whose symbol planes overlap its own RGB takes the
+// two-kernel path, which finishes reading the RGB before the first symbol is written.
+bool Engine::fused_frontend_ok(const uint8_t *d_rgb, const uint8_t *sym) const {
+    return !small_smem_ && forward_fused_eligible(d_rgb, (int)d_.w, (int)d_.h, (int)d_.f) &&
+           (reinterpret_cast<uintptr_t>(sym) & 3) == 0 && !overlaps(sym, d_rgb);
+}
+
+// One chunk's front-end on the stream (no synchronisation) into the symbol planes `sym` and chunk slot c's histogram, which
+// the caller has zeroed.  coef_dump: optional device i32 [3][N], the coefficients of the padded volume [3][pf][ph][pw]
+// (pf = f + 1 for odd f, 2 for f == 1).
+int Engine::frontend_one(uint32_t c, uint8_t wavelet, const uint8_t *d_rgb, uint8_t *sym, int step, int32_t *coef_dump) {
+    unsigned *hist = d_hist_ + (size_t)c * 3 * 256;
+    if (fused_frontend_ok(d_rgb, sym)) {
+        h_fwd_jobs_[c] = FwdFusedJob{d_rgb, sym, hist, coef_dump};
+        CU_TRY(cudaMemcpyAsync(d_fwd_jobs_ + c, h_fwd_jobs_ + c, sizeof(FwdFusedJob), cudaMemcpyHostToDevice, st_));
+        forward_frontend_fused(wavelet, d_fwd_jobs_ + c, 1, coef_dump != nullptr, hist, (int)d_.w, (int)d_.h, step,
+                               device_sm_count(), st_);
+    } else {
+        forward_frontend(wavelet, d_rgb, reinterpret_cast<int16_t *>(d_scratch_), sym, hist, (int)d_.w, (int)d_.h,
+                         (int)d_.f, (int)d_.pw, (int)d_.ph, (int)d_.pf, step, coef_dump, st_);
+    }
+    return kOk;
+}
+
 int Engine::encode_device(uint8_t quality, uint8_t wavelet, const uint8_t *const *d_rgb, uint32_t n,
                           int32_t *d_coef_dump, uint8_t *const *d_work) {
     if (n > cap_) { set_error(kErrBufferSize, "batch larger than engine capacity"); return kErrBufferSize; }
+    int rc = encode_begin(quality, wavelet);
+    if (rc) return rc;
     if (shared_ws_) {
         if (!d_work) { set_error(kErrNull, "shared-workspace batch: workspace pointers required"); return kErrNull; }
         for (uint32_t c = 0; c < n; c++) {
@@ -384,58 +416,33 @@ int Engine::encode_device(uint8_t quality, uint8_t wavelet, const uint8_t *const
             sym_ptr_[c] = d_work[c];
         }
     }
-    const size_t N = (size_t)d_.padded;
-    const int step = quality_to_step(quality);
-    last_wavelet = wavelet;
-    for (uint32_t c = 0; c < n; c++) chunk_step_[c] = step;
-    last_n = n;
-    resident_decoded_ = 0;
+    const int step = begin_step_;
     CU_TRY(cudaMemsetAsync(d_hist_, 0, (size_t)n * 3 * 256 * sizeof(unsigned), st_));
-    CU_TRY(cudaEventRecord(ev_[0], st_));
-    // Front-end.  64-frame chunks of even height and a width that is a multiple of 16 take the fused kernel
-    // (k_fwd_fused.cu), which reads RGB and writes symbols in the same launch: a chunk whose symbol workspace overlaps the
-    // RGB of a chunk of the same launch cannot use it.  Engine-owned symbol planes: one launch for the whole batch.
-    // Caller-provided workspaces (shared-workspace batches): one launch per chunk, in index order, so workspace i may be
-    // the RGB buffer of any chunk j < i (already consumed); a workspace that overlaps its own chunk's RGB falls back to
-    // the two-kernel path, which finishes reading the RGB before the first symbol is written.
-    auto overlaps = [&](const uint8_t *a, size_t na, const uint8_t *b, size_t nb) { return a < b + nb && b < a + na; };
-    bool all_fused = !small_smem_;
-    for (uint32_t c = 0; c < n; c++)
-        all_fused = all_fused && forward_fused_eligible(d_rgb[c], (int)d_.w, (int)d_.h, (int)d_.f) &&
-                    (reinterpret_cast<uintptr_t>(sym_ptr_[c]) & 3) == 0;
-    if (all_fused) {
+    // Engine-owned symbol planes: one fused launch for the whole batch.  Caller-provided workspaces (shared-workspace
+    // batches): one launch per chunk, in index order, so workspace i may be the RGB buffer of any chunk j < i (already
+    // consumed).
+    bool batch_fused = !shared_ws_;
+    for (uint32_t c = 0; c < n; c++) {
+        chunk_step_[c] = step;
+        batch_fused = batch_fused && fused_frontend_ok(d_rgb[c], sym_ptr_[c]);
+    }
+    if (batch_fused) {
         for (uint32_t c = 0; c < n; c++)
             h_fwd_jobs_[c] = FwdFusedJob{d_rgb[c], sym_ptr_[c], d_hist_ + (size_t)c * 3 * 256, c == 0 ? d_coef_dump : nullptr};
         CU_TRY(cudaMemcpyAsync(d_fwd_jobs_, h_fwd_jobs_, n * sizeof(FwdFusedJob), cudaMemcpyHostToDevice, st_));
+        const uint32_t m = (d_coef_dump && n) ? 1 : 0;   // chunk 0 alone when its coefficients are dumped (parity tests)
+        if (m) forward_frontend_fused(wavelet, d_fwd_jobs_, 1, true, d_hist_, (int)d_.w, (int)d_.h, step, device_sm_count(), st_);
+        forward_frontend_fused(wavelet, d_fwd_jobs_ + m, (int)(n - m), false, d_hist_ + (size_t)m * 3 * 256, (int)d_.w,
+                               (int)d_.h, step, device_sm_count(), st_);
+    } else {
+        for (uint32_t c = 0; c < n && !rc; c++)
+            rc = frontend_one(c, wavelet, d_rgb[c], sym_ptr_[c], step, c == 0 ? d_coef_dump : nullptr);
+        if (rc) return rc;
     }
-    const int n_sms = device_sm_count();
-    for (uint32_t c = 0; c < n;) {
-        if (!all_fused || (shared_ws_ && overlaps(sym_ptr_[c], 3 * N, d_rgb[c], 3 * (size_t)d_.n_pixels))) {
-            forward_frontend(wavelet, d_rgb[c], reinterpret_cast<int16_t *>(d_scratch_), sym_ptr_[c],
-                             d_hist_ + (size_t)c * 3 * 256, (int)d_.w, (int)d_.h, (int)d_.f, (int)d_.pw, (int)d_.ph,
-                             (int)d_.pf, step, c == 0 ? d_coef_dump : nullptr, st_);
-            c++;
-            continue;
-        }
-        // a run of chunks for one launch: the whole rest of an engine-owned batch, a single chunk otherwise (or chunk 0
-        // alone when its coefficients are dumped for the parity tests)
-        uint32_t m = (shared_ws_ || (c == 0 && d_coef_dump)) ? 1 : n - c;
-        forward_frontend_fused(wavelet, d_fwd_jobs_ + c, (int)m, c == 0 && d_coef_dump != nullptr,
-                               d_hist_ + (size_t)c * 3 * 256, (int)d_.w, (int)d_.h, step, n_sms, st_);
-        c += m;
-    }
-    CU_TRY(cudaEventRecord(ev_[1], st_));
-    build_encode_tables(n);
-    CU_TRY(cudaEventRecord(ev_[2], st_));
-    int rc = run_rans_encode(n);
-    if (rc) return rc;
-    cudaEventElapsedTime(&timings.ms[0], ev_[0], ev_[1]);
-    cudaEventElapsedTime(&timings.ms[1], ev_[1], ev_[2]);
-    cudaEventElapsedTime(&timings.ms[2], ev_[2], ev_[3]);
-    return kOk;
+    submitted_ = n;
+    return encode_finish(n);
 }
 
-// headers of chunk i + the device->host copies of its payload, enqueued on the engine's stream (no synchronisation)
 // ---- chunk-at-a-time encode: encode_begin, then encode_submit(c) for c = 0, 1, ... in order (each enqueues the front-end of
 // one chunk and returns at once), then encode_finish(n): tables, all 3n rANS streams, one synchronisation.
 int Engine::encode_begin(uint8_t quality, uint8_t wavelet) {
@@ -453,22 +460,11 @@ int Engine::encode_submit(uint32_t c, const uint8_t *d_rgb, uint8_t *d_work, int
         if (!d_work) { set_error(kErrNull, "shared-workspace batch: workspace pointer required"); return kErrNull; }
         sym_ptr_[c] = d_work;
     }
-    const size_t N = (size_t)d_.padded;
     if (step <= 0) step = begin_step_;
     chunk_step_[c] = step;
-    auto overlaps = [&](const uint8_t *a, size_t na, const uint8_t *b, size_t nb) { return a < b + nb && b < a + na; };
-    unsigned *hist = d_hist_ + (size_t)c * 3 * 256;
-    CU_TRY(cudaMemsetAsync(hist, 0, 3 * 256 * sizeof(unsigned), st_));
-    const bool fused = !small_smem_ && forward_fused_eligible(d_rgb, (int)d_.w, (int)d_.h, (int)d_.f) && (reinterpret_cast<uintptr_t>(sym_ptr_[c]) & 3) == 0 &&
-                       !overlaps(sym_ptr_[c], 3 * N, d_rgb, 3 * (size_t)d_.n_pixels);
-    if (fused) {
-        h_fwd_jobs_[c] = FwdFusedJob{d_rgb, sym_ptr_[c], hist, nullptr};
-        CU_TRY(cudaMemcpyAsync(d_fwd_jobs_ + c, h_fwd_jobs_ + c, sizeof(FwdFusedJob), cudaMemcpyHostToDevice, st_));
-        forward_frontend_fused(last_wavelet, d_fwd_jobs_ + c, 1, false, hist, (int)d_.w, (int)d_.h, step, device_sm_count(), st_);
-    } else {
-        forward_frontend(last_wavelet, d_rgb, reinterpret_cast<int16_t *>(d_scratch_), sym_ptr_[c], hist, (int)d_.w, (int)d_.h,
-                         (int)d_.f, (int)d_.pw, (int)d_.ph, (int)d_.pf, step, nullptr, st_);
-    }
+    CU_TRY(cudaMemsetAsync(d_hist_ + (size_t)c * 3 * 256, 0, 3 * 256 * sizeof(unsigned), st_));
+    int rc = frontend_one(c, last_wavelet, d_rgb, sym_ptr_[c], step, nullptr);
+    if (rc) return rc;
     submitted_ = c + 1;
     return kOk;
 }
@@ -486,6 +482,7 @@ int Engine::encode_finish(uint32_t n) {
     return kOk;
 }
 
+// headers of chunk i + the device->host copies of its payload, enqueued on the engine's stream (no synchronisation)
 int Engine::fetch_enqueue(uint32_t i, Chunk &out, bool &direct) {
     if (i >= last_n) { set_error(kErrBufferSize, "chunk index out of range"); return kErrBufferSize; }
     out.width = d_.w; out.height = d_.h; out.frames = d_.f;
@@ -551,51 +548,41 @@ int Engine::fetch_chunks(uint32_t n, Chunk *const *out) {
     return kOk;
 }
 
-// Back-end of n chunks whose symbol planes are in sym_ptr_[c]: RGB into d_rgb_out[c].  Chunks of the fused kernel's shape
-// whose headers stay within its arithmetic bound take k_inv_fused, which reads symbols and writes RGB in the same launch:
-//   * engine-owned symbol planes, one header for the whole batch: one launch;
-//   * caller-provided workspaces (shared-workspace batches): one launch per chunk in DESCENDING index order, so the output
-//     of chunk i may be the workspace of any chunk j > i (already consumed); an output that overlaps its own chunk's
-//     symbol planes falls back to the two-kernel path, which finishes reading the planes before it writes RGB.
-int Engine::run_backend(uint32_t n, const BackendHeader *hdr, uint8_t *const *d_rgb_out) {
-    const size_t N = (size_t)d_.padded;
-    auto overlaps = [&](const uint8_t *a, size_t na, const uint8_t *b, size_t nb) { return a < b + nb && b < a + na; };
-    const int n_sms = device_sm_count();
-    std::vector<char> fused(n, 0);
-    bool any = false, uniform = true;
-    for (uint32_t c = 0; c < n; c++) {
-        fused[c] = !small_smem_ && inverse_fused_eligible(sym_ptr_[c], d_rgb_out[c], (int)d_.w, (int)d_.h, (int)d_.f, hdr[c].steps) &&
-                   !overlaps(sym_ptr_[c], 3 * N, d_rgb_out[c], 3 * (size_t)d_.n_pixels);
-        any = any || fused[c];
-        uniform = uniform && fused[c] && hdr[c].wavelet == hdr[0].wavelet && hdr[c].steps[0] == hdr[0].steps[0] &&
-                  hdr[c].steps[1] == hdr[0].steps[1] && hdr[c].steps[2] == hdr[0].steps[2];
-    }
-    if (any) {
-        for (uint32_t c = 0; c < n; c++) h_inv_jobs_[c] = InvFusedJob{sym_ptr_[c], d_rgb_out[c]};
-        CU_TRY(cudaMemcpyAsync(d_inv_jobs_, h_inv_jobs_, n * sizeof(InvFusedJob), cudaMemcpyHostToDevice, st_));
-    }
-    if (uniform && !shared_ws_) {
-        inverse_backend_fused(hdr[0].wavelet, d_inv_jobs_, (int)n, (int)d_.w, (int)d_.h, hdr[0].steps, n_sms, st_);
-        return kOk;
-    }
-    for (uint32_t k = 0; k < n; k++) {
-        const uint32_t c = shared_ws_ ? n - 1 - k : k;
-        if (fused[c])
-            inverse_backend_fused(hdr[c].wavelet, d_inv_jobs_ + c, 1, (int)d_.w, (int)d_.h, hdr[c].steps, n_sms, st_);
-        else
-            inverse_backend(hdr[c].wavelet, sym_ptr_[c], reinterpret_cast<int32_t *>(d_scratch_), d_rgb_out[c], (int)d_.w,
-                            (int)d_.h, (int)d_.f, (int)d_.pw, (int)d_.ph, (int)d_.pf, hdr[c].steps, st_);
-    }
-    return kOk;
+// The fused back-end (k_inv_fused.cu) takes chunks of the fused front-end's shape whose headers stay within its arithmetic
+// bound.  It reads symbols and writes RGB in the same launch, so an output that overlaps its own chunk's symbol planes
+// takes the two-kernel path, which finishes reading the planes before it writes RGB.
+bool Engine::fused_backend_ok(const uint8_t *sym, const uint8_t *d_rgb, const BackendHeader &hdr) const {
+    return !small_smem_ && inverse_fused_eligible(sym, d_rgb, (int)d_.w, (int)d_.h, (int)d_.f, hdr.steps) &&
+           !overlaps(sym, d_rgb);
 }
 
-// One chunk's back-end on the stream (no synchronisation): the fused kernel when the shape, the header and the buffers allow.
+// Back-end of n chunks whose symbol planes are in sym_ptr_[c]: RGB into d_rgb_out[c].
+//   * engine-owned symbol planes, every chunk fused with one header: one launch;
+//   * otherwise one chunk at a time (backend_one); caller-provided workspaces (shared-workspace batches) in DESCENDING
+//     index order, so the output of chunk i may be the workspace of any chunk j > i (already consumed).  The host
+//     staging layout of the batch calls (host_stage in capi.cu) relies on this order.
+int Engine::run_backend(uint32_t n, const BackendHeader *hdr, uint8_t *const *d_rgb_out) {
+    bool uniform = !shared_ws_ && n > 0;
+    for (uint32_t c = 0; c < n && uniform; c++)
+        uniform = fused_backend_ok(sym_ptr_[c], d_rgb_out[c], hdr[c]) && hdr[c].wavelet == hdr[0].wavelet &&
+                  hdr[c].steps[0] == hdr[0].steps[0] && hdr[c].steps[1] == hdr[0].steps[1] && hdr[c].steps[2] == hdr[0].steps[2];
+    if (uniform) {
+        for (uint32_t c = 0; c < n; c++) h_inv_jobs_[c] = InvFusedJob{sym_ptr_[c], d_rgb_out[c]};
+        CU_TRY(cudaMemcpyAsync(d_inv_jobs_, h_inv_jobs_, n * sizeof(InvFusedJob), cudaMemcpyHostToDevice, st_));
+        inverse_backend_fused(hdr[0].wavelet, d_inv_jobs_, (int)n, (int)d_.w, (int)d_.h, hdr[0].steps, device_sm_count(), st_);
+        return kOk;
+    }
+    int rc = kOk;
+    for (uint32_t k = 0; k < n && !rc; k++) {
+        const uint32_t c = shared_ws_ ? n - 1 - k : k;
+        rc = backend_one(c, hdr[c], d_rgb_out[c]);
+    }
+    return rc;
+}
+
+// One chunk's back-end on the stream (no synchronisation).
 int Engine::backend_one(uint32_t c, const BackendHeader &hdr, uint8_t *d_rgb_out) {
-    const size_t N = (size_t)d_.padded;
-    auto overlaps = [&](const uint8_t *a, size_t na, const uint8_t *b, size_t nb) { return a < b + nb && b < a + na; };
-    const bool fused = !small_smem_ && inverse_fused_eligible(sym_ptr_[c], d_rgb_out, (int)d_.w, (int)d_.h, (int)d_.f, hdr.steps) &&
-                       !overlaps(sym_ptr_[c], 3 * N, d_rgb_out, 3 * (size_t)d_.n_pixels);
-    if (fused) {
+    if (fused_backend_ok(sym_ptr_[c], d_rgb_out, hdr)) {
         h_inv_jobs_[c] = InvFusedJob{sym_ptr_[c], d_rgb_out};
         CU_TRY(cudaMemcpyAsync(d_inv_jobs_ + c, h_inv_jobs_ + c, sizeof(InvFusedJob), cudaMemcpyHostToDevice, st_));
         inverse_backend_fused(hdr.wavelet, d_inv_jobs_ + c, 1, (int)d_.w, (int)d_.h, hdr.steps, device_sm_count(), st_);
@@ -607,7 +594,7 @@ int Engine::backend_one(uint32_t c, const BackendHeader &hdr, uint8_t *d_rgb_out
 }
 
 int Engine::decode_resident_begin(uint32_t n) {
-    if (n > last_n) { set_error(kErrBufferSize, "decode_begin: more chunks than the last encode"); return kErrBufferSize; }
+    if (n > last_n) { set_error(kErrBufferSize, "decode: more chunks than the last encode"); return kErrBufferSize; }
     const size_t N = (size_t)d_.padded;
     const uint32_t S = n * 3;
     resident_decoded_ = 0;
@@ -651,34 +638,12 @@ int Engine::decode_resident_end() {
 }
 
 int Engine::decode_device_resident(uint8_t *const *d_rgb_out, uint32_t n) {
-    if (n > last_n) { set_error(kErrBufferSize, "decode_device: more chunks than the last encode"); return kErrBufferSize; }
-    const size_t N = (size_t)d_.padded;
-    const uint32_t S = n * 3;
-    CU_TRY(cudaEventRecord(ev_[4], st_));
-    build_tables(d_tab_hist_, (int)S, 256, d_enc_, d_dec_lut_, d_aux_, nullptr, nullptr, nullptr, st_);
-    CU_TRY(cudaEventRecord(ev_[5], st_));
-    for (uint32_t s = 0; s < S; s++) {
-        h_dec_jobs_[s].in = stream_base_[s] + stream_off_[s];
-        h_dec_jobs_[s].len = stream_len_[s];
-        h_dec_jobs_[s].symbols = sym_ptr_[s / 3] + (size_t)(s % 3) * N;
-        h_dec_jobs_[s].n = N;
-    }
-    CU_TRY(cudaMemcpyAsync(d_dec_jobs_, h_dec_jobs_, S * sizeof(RansDecJob), cudaMemcpyHostToDevice, st_));
-    rans_decode(d_dec_jobs_, d_dec_lut_, d_aux_, (int)S, st_, small_smem_);
-    CU_TRY(cudaEventRecord(ev_[6], st_));
-    {
-        std::vector<BackendHeader> hdr(n);
-        for (uint32_t c = 0; c < n; c++) hdr[c] = BackendHeader{last_wavelet, {chunk_step_[c], chunk_step_[c], chunk_step_[c]}};
-        int rc = run_backend(n, hdr.data(), d_rgb_out);
-        if (rc) return rc;
-    }
-    CU_TRY(cudaEventRecord(ev_[7], st_));
-    CU_TRY(cudaStreamSynchronize(st_));
-    CU_TRY(cudaGetLastError());
-    cudaEventElapsedTime(&timings.ms[3], ev_[4], ev_[5]);
-    cudaEventElapsedTime(&timings.ms[4], ev_[5], ev_[6]);
-    cudaEventElapsedTime(&timings.ms[5], ev_[6], ev_[7]);
-    return kOk;
+    int rc = decode_resident_begin(n);
+    if (rc) return rc;
+    std::vector<BackendHeader> hdr(n);
+    for (uint32_t c = 0; c < n; c++) hdr[c] = BackendHeader{last_wavelet, {chunk_step_[c], chunk_step_[c], chunk_step_[c]}};
+    rc = run_backend(n, hdr.data(), d_rgb_out);
+    return rc ? rc : decode_resident_end();
 }
 
 int Engine::decode_chunks(const Chunk *const *chunks, uint32_t n, uint8_t *const *d_rgb_out, uint8_t *const *d_work,
@@ -827,21 +792,9 @@ int Engine::rate_curve(uint8_t wavelet, const uint8_t *d_rgb, uint64_t bytes[kRa
     const uint64_t dev_before = dev_bytes_;
     if (!ensure_rate_buffers()) { dev_bytes_ = dev_before; return kErrCuda; }
     const size_t N = (size_t)d_.padded;
-    unsigned *hist = d_hist_ + (size_t)slot * 3 * 256;
-    CU_TRY(cudaMemsetAsync(hist, 0, 3 * 256 * sizeof(unsigned), st_));
-    // front-end at any step (step 1) with the coefficient dump; the same kernel choice as encode_submit
-    auto overlaps = [&](const uint8_t *a, size_t na, const uint8_t *b, size_t nb) { return a < b + nb && b < a + na; };
-    const bool fused = !small_smem_ && forward_fused_eligible(d_rgb, (int)d_.w, (int)d_.h, (int)d_.f) &&
-                       (reinterpret_cast<uintptr_t>(sym) & 3) == 0 && !overlaps(sym, 3 * N, d_rgb, 3 * (size_t)d_.n_pixels);
-    if (fused) {
-        h_fwd_jobs_[slot] = FwdFusedJob{d_rgb, sym, hist, d_coef_};
-        CU_TRY(cudaMemcpyAsync(d_fwd_jobs_ + slot, h_fwd_jobs_ + slot, sizeof(FwdFusedJob), cudaMemcpyHostToDevice, st_));
-        forward_frontend_fused(wavelet, d_fwd_jobs_ + slot, 1, true, hist, (int)d_.w, (int)d_.h, 1, device_sm_count(), st_);
-    } else {
-        // the dump covers the padded volume [3][pf][ph][pw] (pf = f + 1 for odd f, 2 for f == 1) = [3][N]
-        forward_frontend(wavelet, d_rgb, reinterpret_cast<int16_t *>(d_scratch_), sym, hist, (int)d_.w, (int)d_.h,
-                         (int)d_.f, (int)d_.pw, (int)d_.ph, (int)d_.pf, 1, d_coef_, st_);
-    }
+    CU_TRY(cudaMemsetAsync(d_hist_ + (size_t)slot * 3 * 256, 0, 3 * 256 * sizeof(unsigned), st_));
+    int rc = frontend_one(slot, wavelet, d_rgb, sym, 1, d_coef_);   // at any step (1): only the coefficient dump is used
+    if (rc) return rc;
     const int bound = rate_value_bound(wavelet);
     CU_TRY(cudaMemsetAsync(d_vhist_, 0, 3 * (2 * (size_t)bound + 1) * sizeof(unsigned), st_));
     CU_TRY(cudaMemsetAsync(d_rate_out_ + kRateSteps, 0, sizeof(unsigned long long), st_));

@@ -144,20 +144,23 @@ public:
                    uint32_t slot = 0, uint8_t *d_work = nullptr);
 
     // staging buffers for host-pointer entry points
-    uint8_t *rgb_stage(uint32_t slot);          // device buffer of 3*n_pixels bytes, slot in [0, n_stage)
-    uint32_t n_stage() const { return (uint32_t)rgb_stage_.size(); }
+    uint8_t *rgb_stage(uint32_t slot);          // device buffer of 3*n_pixels bytes, allocated on first use
     const uint8_t *symbols_dev(uint32_t chunk) const { return sym_ptr_[chunk]; }
     EngineTimings timings;
-    uint8_t last_wavelet = 0;
-    uint32_t last_n = 0;
-    uint32_t submitted_ = 0;
 
 private:
     int run_rans_encode(uint32_t n);
     void build_encode_tables(uint32_t n);
+    bool overlaps(const uint8_t *sym, const uint8_t *rgb) const;
+    bool fused_frontend_ok(const uint8_t *d_rgb, const uint8_t *sym) const;
+    int frontend_one(uint32_t c, uint8_t wavelet, const uint8_t *d_rgb, uint8_t *sym, int step, int32_t *coef_dump);
     struct BackendHeader { uint8_t wavelet; int steps[3]; };   // what the back-end needs from a chunk's headers
+    bool fused_backend_ok(const uint8_t *sym, const uint8_t *d_rgb, const BackendHeader &hdr) const;
     int run_backend(uint32_t n, const BackendHeader *hdr, uint8_t *const *d_rgb_out);
     int backend_one(uint32_t c, const BackendHeader &hdr, uint8_t *d_rgb_out);
+    uint8_t last_wavelet = 0;
+    uint32_t last_n = 0;              // chunks of the last successful encode (fetch_chunk, decode_device_resident)
+    uint32_t submitted_ = 0;          // chunks whose front-end the current encode has enqueued
     uint32_t resident_decoded_ = 0;   // chunks whose symbol planes decode_resident_begin has queued
     int fetch_enqueue(uint32_t i, Chunk &out, bool &direct);
     Dims d_;
