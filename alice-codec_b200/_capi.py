@@ -120,6 +120,10 @@ SIGNATURES = {
     "alice_codec_rate_curve_device_ex": (cint, [u8, vp, u32, u32, u32, u64p, u32p, vp, u32]),
     "alice_codec_encode_to_size_ex": (vp, [u8, u8p, u64, u32, u32, u32, u64, u8p, u32]),
     "alice_codec_batch_encode_host_to_size": (cint, [vp, C.POINTER(vp), u32, u64, C.POINTER(vp), u8p]),
+    "alice_codec_psnr_curve": (cint, [u8, u8p, u64, u32, u32, u32, C.POINTER(dbl), u64p]),
+    "alice_codec_psnr_curve_device": (cint, [u8, vp, u32, u32, u32, C.POINTER(dbl), u64p, vp]),
+    "alice_codec_encode_to_psnr": (vp, [u8, u8p, u64, u32, u32, u32, dbl, u8p]),
+    "alice_codec_batch_encode_host_to_psnr": (cint, [vp, C.POINTER(vp), u32, dbl, C.POINTER(vp), u8p]),
     "alice_codec_synth_rgb_device": (cint, [cint, u32, u32, u32, u32, vp, vp]),
     "alice_codec_pinned_alloc": (vp, [u64]),
     "alice_codec_pinned_free": (None, [vp]),

@@ -54,6 +54,11 @@ def _curve_dict(sizes):
             for s in range(1, RATE_STEPS + 1)}
 
 
+def _psnr_dict(psnr):
+    """{quality: PSNR in dB} over the 64 steps (highest quality first), keyed as _curve_dict"""
+    return {quality_for_step(s): float(psnr[s - 1]) for s in range(1, RATE_STEPS + 1)}
+
+
 def _wavelet_byte(wavelet) -> int:
     if isinstance(wavelet, str):
         if wavelet not in WAVELET_NAMES:
@@ -502,6 +507,48 @@ class FrameEncoder:
             self._api._raise()
         return EncodedChunk(h, self._api), q.value
 
+    def _need_well_formed(self):
+        if not self.well_formed_tables:
+            raise ValueError("the PSNR curve describes the well-formed-tables encode only: "
+                             "make the encoder with well_formed_tables=True")
+
+    def psnr_curve(self, rgb_frames, width: int, height: int, frames: int, with_sse: bool = False):
+        """Exact PSNR of the decode of this encoder's encode at every quantiser step, without any rANS work:
+        {quality: dB}, one entry per step (the largest quality with that step), each equal to
+        psnr(rgb, FrameDecoder().decode(FrameEncoder(quality, wavelet, well_formed_tables=True).encode(rgb, ...))) bit
+        for bit; inf where the decode is exact.  Not monotone in the quality.  with_sse=True also returns the sums of
+        squared differences, uint64 [64] (index step - 1).  Well-formed-tables encoders only (DESIGN.md 4.9)."""
+        self._need_well_formed()
+        a, pa = _u8(rgb_frames)
+        psnr, sse = np.zeros(RATE_STEPS, np.float64), np.zeros(RATE_STEPS, np.uint64)
+        self._api._chk(self._api.lib.alice_codec_psnr_curve(
+            self.wavelet, pa, a.size, width, height, frames, psnr.ctypes.data_as(C.POINTER(C.c_double)),
+            sse.ctypes.data_as(_capi.u64p)))
+        return (_psnr_dict(psnr), sse) if with_sse else _psnr_dict(psnr)
+
+    def psnr_curve_device(self, d_rgb: int, width: int, height: int, frames: int, stream: int = 0,
+                          with_sse: bool = False):
+        """psnr_curve for RGB in device memory (raw device pointer); waits for the work enqueued on `stream` first"""
+        self._need_well_formed()
+        psnr, sse = np.zeros(RATE_STEPS, np.float64), np.zeros(RATE_STEPS, np.uint64)
+        self._api._chk(self._api.lib.alice_codec_psnr_curve_device(
+            self.wavelet, C.c_void_p(int(d_rgb)), width, height, frames, psnr.ctypes.data_as(C.POINTER(C.c_double)),
+            sse.ctypes.data_as(_capi.u64p), C.c_void_p(stream)))
+        return (_psnr_dict(psnr), sse) if with_sse else _psnr_dict(psnr)
+
+    def encode_to_psnr(self, rgb_frames, width: int, height: int, frames: int, min_psnr: float):
+        """The chunk at the lowest quality whose decode reaches min_psnr dB: (EncodedChunk, quality), the chunk
+        byte-identical to FrameEncoder(quality, wavelet, well_formed_tables=True).encode.  The encoder's quality is not
+        used.  Raises CodecError InvalidQuantStep if no quality reaches the target, or if it is NaN."""
+        self._need_well_formed()
+        a, pa = _u8(rgb_frames)
+        q = C.c_uint8()
+        h = self._api.lib.alice_codec_encode_to_psnr(self.wavelet, pa, a.size, width, height, frames, float(min_psnr),
+                                                     C.byref(q))
+        if not h:
+            self._api._raise()
+        return EncodedChunk(h, self._api), q.value
+
 
 class FrameDecoder:
     """python.rs:443-482: FrameDecoder().decode(chunk) -> 1-D uint8 RGB array."""
@@ -644,6 +691,20 @@ class ChunkBatch:
         out = (C.c_void_p * n)()
         q = np.zeros(max(n, 1), np.uint8)
         self._api._chk(self._api.lib.alice_codec_batch_encode_host_to_size(self._h, arr, n, int(max_bytes), out,
+                                                                           q.ctypes.data_as(_capi.u8p)))
+        return [EncodedChunk(C.c_void_p(out[i]), self._api) for i in range(n)], [int(x) for x in q[:n]]
+
+    def encode_host_to_psnr(self, h_rgb_ptrs, min_psnr: float):
+        """encode_host with every chunk at the lowest quality whose decode reaches min_psnr dB: (chunks, qualities).
+        Batches made with well_formed_tables=True only; the batch's quality is not used."""
+        if not self.well_formed_tables:
+            raise ValueError("the PSNR curve describes the well-formed-tables encode only: "
+                             "make the batch with well_formed_tables=True")
+        n = len(h_rgb_ptrs)
+        arr = self._ptr_array(h_rgb_ptrs)
+        out = (C.c_void_p * n)()
+        q = np.zeros(max(n, 1), np.uint8)
+        self._api._chk(self._api.lib.alice_codec_batch_encode_host_to_psnr(self._h, arr, n, float(min_psnr), out,
                                                                            q.ctypes.data_as(_capi.u8p)))
         return [EncodedChunk(C.c_void_p(out[i]), self._api) for i in range(n)], [int(x) for x in q[:n]]
 

@@ -5,6 +5,8 @@ concatenation of self-delimiting .alc blobs; `decode` and `info` accept such str
 (the whole input without --chunk-frames) is encoded at the highest quality whose .alc blob is at most N bytes; the chunk
 is byte-identical to an encode at that quality, and -q is not used.  With --well-formed-tables every chunk stores
 rANS tables that decode exactly on any decoder of the format (DESIGN.md 4.8); without it the output is the reference's.
+With --min-psnr DB (which needs --well-formed-tables) every chunk is encoded at the lowest quality whose decode reaches DB
+dB of PSNR against the input (DESIGN.md 4.9); the chunk is byte-identical to a well-formed encode at that quality.
 
     python -m alice_codec_b200.cli encode raw.rgb -W 1920 -H 1080 -f 64 -q 90 -w cdf53 -o out.alc
     (from the repo root: python alice-codec_b200/cli.py ...)
@@ -31,15 +33,23 @@ WAVELET_LABEL = {"cdf53": "CDF 5/3", "cdf97": "CDF 9/7", "haar": "Haar"}   # mai
 def cmd_encode(a) -> None:
     if a.wavelet not in pkg.WAVELET_NAMES:
         raise ValueError(f"unknown wavelet '{a.wavelet}'; expected cdf53, cdf97, or haar")     # main.rs:74-83
+    target = a.min_psnr
+    if target is not None and not a.well_formed_tables:
+        raise ValueError("--min-psnr needs --well-formed-tables (the PSNR curve describes that encode only)")
+    if target is not None and a.max_bytes is not None:
+        raise ValueError("--min-psnr and --max-bytes cannot be combined")
     rgb = np.fromfile(a.input, dtype=np.uint8)
     enc = pkg.FrameEncoder(a.quality, a.wavelet, well_formed_tables=a.well_formed_tables)
     budget = a.max_bytes
-    qualities = []                                  # --max-bytes: the quality chosen for each chunk
+    qualities = []                                  # --max-bytes / --min-psnr: the quality chosen for each chunk
 
     def one(part, nf):
-        if budget is None:
+        if budget is None and target is None:
             return enc.encode(part, a.width, a.height, nf).to_bytes()
-        chunk, q = enc.encode_to_size(part, a.width, a.height, nf, budget)
+        if budget is not None:
+            chunk, q = enc.encode_to_size(part, a.width, a.height, nf, budget)
+        else:
+            chunk, q = enc.encode_to_psnr(part, a.width, a.height, nf, target)
         qualities.append(q)
         return chunk.to_bytes()
 
@@ -55,11 +65,14 @@ def cmd_encode(a) -> None:
                                    well_formed_tables=a.well_formed_tables)
             cb = per * a.chunk_frames
             parts = [np.ascontiguousarray(rgb[i * cb:(i + 1) * cb]) for i in range(n_full)]
-            if budget is None:
-                chunks = batch.encode_host([p.ctypes.data for p in parts])
-            else:
+            if budget is not None:
                 chunks, qs = batch.encode_host_to_size([p.ctypes.data for p in parts], budget)
                 qualities.extend(qs)
+            elif target is not None:
+                chunks, qs = batch.encode_host_to_psnr([p.ctypes.data for p in parts], target)
+                qualities.extend(qs)
+            else:
+                chunks = batch.encode_host([p.ctypes.data for p in parts])
             blobs = [c.to_bytes() for c in chunks]
             batch.close()
         else:
@@ -73,8 +86,9 @@ def cmd_encode(a) -> None:
     with open(a.output, "wb") as f:
         f.write(data)
     ratio = len(data) / rgb.size if rgb.size else 0.0
-    setting = (f"quality={a.quality}" if budget is None else
-               f"max-bytes={budget} per chunk, quality={','.join(str(q) for q in qualities)}")
+    chosen = ",".join(str(q) for q in qualities)
+    setting = (f"max-bytes={budget} per chunk, quality={chosen}" if budget is not None else
+               f"min-psnr={target} dB per chunk, quality={chosen}" if target is not None else f"quality={a.quality}")
     tables = ", tables=well-formed" if a.well_formed_tables else ""
     sys.stderr.write(f"encoded {a.width}x{a.height}x{a.frames} ({rgb.size} bytes) -> {len(data)} bytes "
                      f"({ratio * 100:.1f}% ratio, {setting}, wavelet={a.wavelet}{tables})\n")
@@ -142,6 +156,9 @@ def main(argv=None) -> int:
     e.add_argument("--chunk-frames", type=int, default=0, help="cut the input into chunks of this many frames (0 = one chunk)")
     e.add_argument("--max-bytes", type=int, default=None,
                    help="byte budget per chunk: encode each chunk at the highest quality whose .alc fits (-q is not used)")
+    e.add_argument("--min-psnr", type=float, default=None, metavar="DB",
+                   help="PSNR target per chunk: encode each chunk at the lowest quality whose decode reaches DB dB "
+                        "(needs --well-formed-tables; -q is not used)")
     e.add_argument("--well-formed-tables", action="store_true",
                    help="store rANS tables that every .alc decoder decodes exactly (the header histograms become table "
                         "specifications instead of symbol counts)")

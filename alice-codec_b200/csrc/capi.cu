@@ -2,6 +2,7 @@
 // Part 1 mirrors src/ffi.rs of the reference symbol for symbol; Part 2 are the extensions.
 // Every compute entry point runs on the CUDA device; there is no CPU fallback.
 #include <cmath>
+#include <cstdio>
 #include <cstdlib>
 #include <cstring>
 #include <new>
@@ -217,6 +218,19 @@ bool encode_flags_ok(uint32_t flags) {
     return true;
 }
 
+// The input of a curve on a pooled engine: RGB on the device (the engine's stream waits for the work enqueued on
+// user_st), or host RGB copied to the engine's stage 0.  Null (error set) on failure.
+const uint8_t *curve_input(Engine *e, const uint8_t *rgb, bool device, uint64_t rgb_len, cudaStream_t user_st) {
+    if (!device) return stage_host_chunk(e, rgb, rgb_len);
+    cudaEvent_t ev = nullptr;
+    if (cudaEventCreateWithFlags(&ev, cudaEventDisableTiming) != cudaSuccess) { cudaGetLastError(); set_error(kErrCuda, "event creation failed"); return nullptr; }
+    cudaError_t ce = cudaEventRecord(ev, user_st);
+    if (ce == cudaSuccess) ce = cudaStreamWaitEvent(e->stream(), ev, 0);
+    cudaEventDestroy(ev);
+    if (ce != cudaSuccess) { cudaGetLastError(); set_error(kErrCuda, "stream ordering failed"); return nullptr; }
+    return rgb;
+}
+
 // Predicted .alc size of every step for one chunk whose RGB is on the host (device == false) or the device.
 int rate_curve_impl(uint8_t wavelet, const uint8_t *rgb, bool device, uint64_t rgb_len, uint32_t w, uint32_t h,
                     uint32_t f, uint64_t *bytes64, uint32_t *hist_out, cudaStream_t user_st, uint32_t flags) {
@@ -237,21 +251,8 @@ int rate_curve_impl(uint8_t wavelet, const uint8_t *rgb, bool device, uint64_t r
     if (!cuda_ready()) return kErrCuda;
     Engine *e = acquire_engine(d, (flags & ALICE_ENCODE_WELL_FORMED_TABLES) != 0);
     if (!e) return kErrCuda;
-    do {
-        const uint8_t *src = rgb;
-        if (device) {   // the engine's stream waits for the caller's work on the input
-            cudaEvent_t ev = nullptr;
-            if (cudaEventCreateWithFlags(&ev, cudaEventDisableTiming) != cudaSuccess) { cudaGetLastError(); set_error(kErrCuda, "event creation failed"); rc = kErrCuda; break; }
-            cudaError_t ce = cudaEventRecord(ev, user_st);
-            if (ce == cudaSuccess) ce = cudaStreamWaitEvent(e->stream(), ev, 0);
-            cudaEventDestroy(ev);
-            if (ce != cudaSuccess) { cudaGetLastError(); set_error(kErrCuda, "stream ordering failed"); rc = kErrCuda; break; }
-        } else {
-            src = stage_host_chunk(e, rgb, rgb_len);
-            if (!src) { rc = kErrCuda; break; }
-        }
-        rc = e->rate_curve(wavelet, src, bytes64, hist_out);
-    } while (0);
+    const uint8_t *src = curve_input(e, rgb, device, rgb_len, user_st);
+    rc = src ? e->rate_curve(wavelet, src, bytes64, hist_out) : kErrCuda;
     release_engine(e);
     return rc;
 }
@@ -307,6 +308,66 @@ EncodedChunk *encode_to_size_impl(uint8_t wavelet, const uint8_t *rgb, uint64_t 
     } while (0);
     release_engine(e);
     return out;
+}
+
+// ------------------------------------------------------------------------------ PSNR targets
+// alice_codec_psnr's closed form (metrics.rs:16-63) of an exact sum of squared differences over len bytes
+double psnr_of_sse(uint64_t sse, uint64_t len) {
+    if (len == 0) return INFINITY;
+    const double mse = (double)sse / (double)len;
+    return mse == 0.0 ? INFINITY : 10.0 * log10(255.0 * 255.0 / mse);
+}
+
+// the largest step whose PSNR reaches min_psnr_db (the lowest quality; PSNR is not monotone in the step), 0 if none
+int pick_psnr_step(const double psnr[kRateSteps], double min_psnr_db) {
+    for (int s = kRateSteps; s >= 1; s--)
+        if (psnr[s - 1] >= min_psnr_db) return s;
+    return 0;
+}
+
+void set_no_psnr_error(const double psnr[kRateSteps], double min_psnr_db) {
+    int best = kRateSteps;
+    for (int s = kRateSteps; s >= 1; s--)
+        if (psnr[s - 1] > psnr[best - 1]) best = s;
+    char msg[160];
+    snprintf(msg, sizeof msg, "no quality reaches %.17g dB: the best PSNR is %.17g dB, at quality %d", min_psnr_db,
+             psnr[best - 1], (int)quality_for_step(best));
+    set_error(kErrQuantStep, msg);
+}
+
+bool psnr_target_ok(double min_psnr_db) {
+    if (std::isnan(min_psnr_db)) { set_error(kErrQuantStep, "the PSNR target is NaN"); return false; }
+    return true;
+}
+
+void psnr_from_sse(const uint64_t sse[kRateSteps], uint64_t len, double *psnr64, uint64_t *sse64) {
+    for (int i = 0; i < kRateSteps; i++) {
+        psnr64[i] = psnr_of_sse(sse[i], len);
+        if (sse64) sse64[i] = sse[i];
+    }
+}
+
+// PSNR of the well-formed encode at every step for one chunk whose RGB is on the host (device == false) or the device.
+int psnr_curve_impl(uint8_t wavelet, const uint8_t *rgb, bool device, uint64_t rgb_len, uint32_t w, uint32_t h,
+                    uint32_t f, double *psnr64, uint64_t *sse64, cudaStream_t user_st) {
+    set_error(0, "");
+    if (!psnr64) { set_error(kErrNull, "null output"); return kErrNull; }
+    if (wavelet > 2) { set_error(kErrBitstream, "unknown wavelet type byte"); return kErrBitstream; }
+    Dims d;
+    bool empty;
+    int rc = validate_encode(rgb_len, w, h, f, d, empty);
+    if (rc) return rc;
+    uint64_t sse[kRateSteps] = {0};
+    if (empty) { psnr_from_sse(sse, 0, psnr64, sse64); return kOk; }
+    if (!rgb) { set_error(kErrNull, "null argument"); return kErrNull; }
+    if (!cuda_ready()) return kErrCuda;
+    Engine *e = acquire_engine(d, true);
+    if (!e) return kErrCuda;
+    const uint8_t *src = curve_input(e, rgb, device, rgb_len, user_st);
+    rc = src ? e->psnr_curve(wavelet, src, sse) : kErrCuda;
+    release_engine(e);
+    if (!rc) psnr_from_sse(sse, d.n_pixels * 3, psnr64, sse64);
+    return rc;
 }
 
 uint8_t *decode_impl(const EncodedChunk *chunk, uint64_t *out_len, uint8_t *symbols_out) {
@@ -1360,6 +1421,99 @@ int alice_codec_batch_encode_host_to_size(AliceBatch *b, const uint8_t *const *h
     return kOk;
 }
 
+// ------------------------------------------------------------------------------ PSNR targets
+int alice_codec_psnr_curve(uint8_t wavelet, const uint8_t *rgb, uint64_t rgb_len, uint32_t width, uint32_t height,
+                           uint32_t frames, double *psnr64, uint64_t *sse64) {
+    return psnr_curve_impl(wavelet, rgb, false, rgb_len, width, height, frames, psnr64, sse64, nullptr);
+}
+int alice_codec_psnr_curve_device(uint8_t wavelet, const uint8_t *d_rgb, uint32_t width, uint32_t height,
+                                  uint32_t frames, double *psnr64, uint64_t *sse64, void *cuda_stream) {
+    const unsigned __int128 len = (unsigned __int128)width * height * frames * 3;
+    if (len > (unsigned __int128)UINT64_MAX) { set_error(kErrOverflow, "dimensions overflow usize"); return kErrOverflow; }
+    return psnr_curve_impl(wavelet, d_rgb, true, (uint64_t)len, width, height, frames, psnr64, sse64,
+                           (cudaStream_t)cuda_stream);
+}
+// The PSNR curve picks the step, one well-formed encode at it follows: the curve is exact, so nothing is checked after.
+EncodedChunk *alice_codec_encode_to_psnr(uint8_t wavelet, const uint8_t *rgb, uint64_t rgb_len, uint32_t width,
+                                         uint32_t height, uint32_t frames, double min_psnr_db, uint8_t *quality_out) {
+    set_error(0, "");
+    if (!rgb || !quality_out) { set_error(kErrNull, "null argument"); return nullptr; }
+    if (wavelet > 2) { set_error(kErrBitstream, "unknown wavelet type byte"); return nullptr; }
+    if (!psnr_target_ok(min_psnr_db)) return nullptr;
+    Dims d;
+    bool empty;
+    if (validate_encode(rgb_len, width, height, frames, d, empty)) return nullptr;
+    if (empty) {   // +inf at every step: the largest one
+        EncodedChunk *out = new (std::nothrow) EncodedChunk();
+        if (!out) return nullptr;
+        out->c.width = width; out->c.height = height; out->c.frames = frames;
+        out->c.wavelet = wavelet;
+        *quality_out = quality_for_step(kRateSteps);
+        return out;
+    }
+    if (!cuda_ready()) return nullptr;
+    Engine *e = acquire_engine(d, true);
+    if (!e) return nullptr;
+    EncodedChunk *out = nullptr;
+    do {
+        const uint8_t *stage = stage_host_chunk(e, rgb, rgb_len);
+        if (!stage) break;
+        uint64_t sse[kRateSteps];
+        double psnr[kRateSteps];
+        if (e->psnr_curve(wavelet, stage, sse)) break;
+        psnr_from_sse(sse, d.n_pixels * 3, psnr, nullptr);
+        const int step = pick_psnr_step(psnr, min_psnr_db);
+        if (!step) { set_no_psnr_error(psnr, min_psnr_db); break; }
+        out = new (std::nothrow) EncodedChunk();
+        if (!out) break;
+        const uint8_t *ptrs[1] = {stage};
+        if (e->encode_device(quality_for_step(step), wavelet, ptrs, 1, nullptr) || e->fetch_chunk(0, out->c)) {
+            delete out; out = nullptr;
+            break;
+        }
+        *quality_out = quality_for_step(step);
+    } while (0);
+    release_engine(e);
+    return out;
+}
+// Per chunk, in stream order as alice_codec_batch_encode_host stages it: copy, PSNR curve, one host read of 64 sums, the
+// front-end at the chosen step; then one table build and one rANS launch for the whole batch.
+int alice_codec_batch_encode_host_to_psnr(AliceBatch *b, const uint8_t *const *h_rgb, uint32_t n, double min_psnr_db,
+                                          EncodedChunk **out_chunks, uint8_t *qualities_out) {
+    set_error(0, "");
+    if (!b || !h_rgb || !out_chunks || !qualities_out) { set_error(kErrNull, "null argument"); return kErrNull; }
+    Engine *e = b->eng;
+    if (!e->well_formed_tables()) { set_error(kErrDimensions, "batch was not created with ALICE_BATCH_WELL_FORMED_TABLES"); return kErrDimensions; }
+    if (!psnr_target_ok(min_psnr_db)) return kErrQuantStep;
+    if (n > e->cap_chunks()) { set_error(kErrBufferSize, "batch larger than capacity"); return kErrBufferSize; }
+    const size_t bytes = (size_t)e->dims().n_pixels * 3;
+    std::vector<int> steps(n);
+    int rc = e->encode_begin(100, b->wavelet);    // the batch's quality is not used: every chunk names its step
+    for (uint32_t i = 0; i < n && !rc; i++) {
+        if (!h_rgb[i]) { set_error(kErrNull, "null chunk pointer"); return kErrNull; }
+        uint8_t *s, *work;
+        if (!host_stage(e, i, s, work)) return kErrCuda;
+        CU_CHECK_RC(cudaMemcpyAsync(s, h_rgb[i], bytes, cudaMemcpyHostToDevice, e->stream()));
+        uint64_t sse[kRateSteps];
+        double psnr[kRateSteps];
+        rc = e->psnr_curve(b->wavelet, s, sse, i, work);
+        if (rc) return rc;
+        psnr_from_sse(sse, bytes, psnr, nullptr);
+        steps[i] = pick_psnr_step(psnr, min_psnr_db);
+        if (!steps[i]) {
+            set_no_psnr_error(psnr, min_psnr_db);
+            set_error(kErrQuantStep, "chunk " + std::to_string(i) + ": " + last_error_msg());
+            return kErrQuantStep;
+        }
+        rc = e->encode_submit(i, s, work, steps[i]);
+    }
+    if (!rc) rc = e->encode_finish(n);
+    if (!rc) rc = fetch_new_chunks(e, n, out_chunks);
+    if (rc) return rc;
+    for (uint32_t i = 0; i < n; i++) qualities_out[i] = quality_for_step(steps[i]);
+    return kOk;
+}
+
 int alice_codec_synth_rgb_device(int kind, uint32_t seed, uint32_t w, uint32_t h, uint32_t f, uint8_t *d_rgb,
                                  void *cuda_stream) {
     set_error(0, "");
@@ -1386,9 +1540,7 @@ int alice_codec_psnr_device(const uint8_t *d_a, const uint8_t *d_b, uint64_t len
     CU_CHECK_RC(cudaGetLastError());
     CU_CHECK_RC(cudaMemcpyAsync(h_acc, d_acc, 8, cudaMemcpyDeviceToHost, st));
     CU_CHECK_RC(cudaStreamSynchronize(st));
-    const unsigned long long sum = *h_acc;
-    const double mse = (double)sum / (double)len;
-    *psnr_out = mse == 0.0 ? INFINITY : 10.0 * log10(255.0 * 255.0 / mse);
+    *psnr_out = psnr_of_sse(*h_acc, len);
     return kOk;
 }
 void *alice_codec_pinned_alloc(uint64_t bytes) {

@@ -278,6 +278,9 @@ Engine::~Engine() {
     cudaFree(d_coef_); cudaFree(d_vhist_); cudaFree(d_rate_hist_); cudaFree(d_rate_wf_hist_); cudaFree(d_rate_enc_);
     cudaFree(d_rate_lut_); cudaFree(d_rate_aux_); cudaFree(d_rate_est_); cudaFree(d_rate_out_);
     if (h_rate_out_) cudaFreeHost(h_rate_out_);
+    cudaFree(d_sse_); cudaFree(d_sse_jobs_); cudaFree(d_sse_rgb_);
+    if (h_sse_) cudaFreeHost(h_sse_);
+    if (h_sse_jobs_) cudaFreeHost(h_sse_jobs_);
     for (auto &e : ev_) if (e) cudaEventDestroy(e);
     if (st_ && own_stream_) cudaStreamDestroy(st_);
     cudaGetLastError();
@@ -784,17 +787,24 @@ bool Engine::ensure_rate_buffers() {
     return true;
 }
 
-int Engine::rate_curve(uint8_t wavelet, const uint8_t *d_rgb, uint64_t bytes[kRateSteps], unsigned *h_hist_out,
-                       uint32_t slot, uint8_t *d_work) {
+// The front-end of one chunk with the coefficient dump into d_coef_ (the rate and PSNR curves): chunk slot `slot`'s
+// histogram and symbol planes, or d_work, are scratch until that chunk's real front-end; `sym` = those planes.
+int Engine::dump_frontend(uint8_t wavelet, const uint8_t *d_rgb, uint32_t slot, uint8_t *d_work, uint8_t *&sym) {
     if (slot >= cap_) { set_error(kErrBufferSize, "rate curve: chunk slot beyond the engine capacity"); return kErrBufferSize; }
-    uint8_t *sym = d_work ? d_work : sym_ptr_[slot];
+    sym = d_work ? d_work : sym_ptr_[slot];
     if (!sym) { set_error(kErrNull, "shared-workspace engine: workspace pointer required"); return kErrNull; }
     const uint64_t dev_before = dev_bytes_;
     if (!ensure_rate_buffers()) { dev_bytes_ = dev_before; return kErrCuda; }
-    const size_t N = (size_t)d_.padded;
     CU_TRY(cudaMemsetAsync(d_hist_ + (size_t)slot * 3 * 256, 0, 3 * 256 * sizeof(unsigned), st_));
-    int rc = frontend_one(slot, wavelet, d_rgb, sym, 1, d_coef_);   // at any step (1): only the coefficient dump is used
+    return frontend_one(slot, wavelet, d_rgb, sym, 1, d_coef_);   // at any step (1): only the coefficient dump is used
+}
+
+int Engine::rate_curve(uint8_t wavelet, const uint8_t *d_rgb, uint64_t bytes[kRateSteps], unsigned *h_hist_out,
+                       uint32_t slot, uint8_t *d_work) {
+    uint8_t *sym = nullptr;
+    int rc = dump_frontend(wavelet, d_rgb, slot, d_work, sym);
     if (rc) return rc;
+    const size_t N = (size_t)d_.padded;
     const int bound = rate_value_bound(wavelet);
     CU_TRY(cudaMemsetAsync(d_vhist_, 0, 3 * (2 * (size_t)bound + 1) * sizeof(unsigned), st_));
     CU_TRY(cudaMemsetAsync(d_rate_out_ + kRateSteps, 0, sizeof(unsigned long long), st_));
@@ -817,6 +827,59 @@ int Engine::rate_curve(uint8_t wavelet, const uint8_t *d_rgb, uint64_t bytes[kRa
         return kErrPanic;
     }
     for (int i = 0; i < kRateSteps; i++) bytes[i] = h_rate_out_[i];
+    return kOk;
+}
+
+// ------------------------------------------------------------------------------ PSNR curve
+bool Engine::ensure_psnr_buffers(bool rgb_scratch) {
+    const uint64_t dev_before = dev_bytes_;
+    bool a = true;
+    if (!d_sse_) {
+        a = a && dev_alloc(d_sse_, kRateSteps * sizeof(unsigned long long), dev_bytes_);
+        a = a && dev_alloc(d_sse_jobs_, kRateSteps * sizeof(InvSseJob), dev_bytes_);
+        a = a && cudaMallocHost((void **)&h_sse_, kRateSteps * sizeof(unsigned long long)) == cudaSuccess;
+        a = a && cudaMallocHost((void **)&h_sse_jobs_, kRateSteps * sizeof(InvSseJob)) == cudaSuccess;
+        if (!a) {   // leave the engine as it was: a later call retries
+            cudaFree(d_sse_); cudaFree(d_sse_jobs_);
+            if (h_sse_) cudaFreeHost(h_sse_);
+            if (h_sse_jobs_) cudaFreeHost(h_sse_jobs_);
+            d_sse_ = nullptr; d_sse_jobs_ = nullptr; h_sse_ = nullptr; h_sse_jobs_ = nullptr;
+        }
+    }
+    if (a && rgb_scratch && !d_sse_rgb_) a = dev_alloc(d_sse_rgb_, (size_t)d_.n_pixels * 3, dev_bytes_);
+    if (!a) {
+        cudaGetLastError();
+        dev_bytes_ = dev_before;
+        set_error(kErrCuda, "device or pinned memory allocation failed (PSNR curve)");
+    }
+    return a;
+}
+
+int Engine::psnr_curve(uint8_t wavelet, const uint8_t *d_rgb, uint64_t sse[kRateSteps], uint32_t slot, uint8_t *d_work) {
+    uint8_t *sym = nullptr;
+    int rc = dump_frontend(wavelet, d_rgb, slot, d_work, sym);
+    if (rc) return rc;
+    const int top[3] = {kRateSteps, kRateSteps, kRateSteps};   // the largest step of the curve bounds them all
+    const bool fused = !small_smem_ && inverse_fused_eligible(nullptr, d_rgb, (int)d_.w, (int)d_.h, (int)d_.f, top);
+    if (!ensure_psnr_buffers(!fused)) return kErrCuda;
+    CU_TRY(cudaMemsetAsync(d_sse_, 0, kRateSteps * sizeof(unsigned long long), st_));
+    if (fused) {
+        for (int i = 0; i < kRateSteps; i++) h_sse_jobs_[i] = InvSseJob{d_coef_, d_rgb, d_sse_ + i, i + 1};
+        CU_TRY(cudaMemcpyAsync(d_sse_jobs_, h_sse_jobs_, kRateSteps * sizeof(InvSseJob), cudaMemcpyHostToDevice, st_));
+        inverse_sse_fused(wavelet, d_sse_jobs_, (int)d_.w, (int)d_.h, device_sm_count(), st_);
+    } else {
+        for (int s = 1; s <= kRateSteps; s++) {
+            const int steps[3] = {s, s, s};
+            coef_symbols(d_coef_, 3 * d_.padded, s, sym, st_);
+            inverse_backend(wavelet, sym, reinterpret_cast<int32_t *>(d_scratch_), d_sse_rgb_, (int)d_.w, (int)d_.h,
+                            (int)d_.f, (int)d_.pw, (int)d_.ph, (int)d_.pf, steps, st_);
+            sq_diff_sum_u8(d_sse_rgb_, d_rgb, (size_t)d_.n_pixels * 3, d_sse_ + s - 1, st_);
+        }
+    }
+    CU_TRY(cudaMemcpyAsync(h_sse_, d_sse_, kRateSteps * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st_));
+    CU_TRY(cudaStreamSynchronize(st_));
+    CU_TRY(cudaGetLastError());
+    for (int i = 0; i < kRateSteps; i++) sse[i] = h_sse_[i];
     return kOk;
 }
 

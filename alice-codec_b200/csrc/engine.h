@@ -142,6 +142,15 @@ public:
     // pixel of coefficients + the tables of 192 pseudo-streams) are allocated on the first call.
     int rate_curve(uint8_t wavelet, const uint8_t *d_rgb, uint64_t bytes[kRateSteps], unsigned *h_hist_out,
                    uint32_t slot = 0, uint8_t *d_work = nullptr);
+    // PSNR curve of one chunk (DESIGN.md 4.9): sse[i] = the sum over the chunk's 3*w*h*f bytes of (input - decode)^2,
+    // where the decode is that of a well-formed-tables encode at step i + 1 (such a chunk decodes to exactly the symbols
+    // quant_symbol gives, so this is the decode of the quantised coefficient dump; the default encode has no such
+    // curve).  Runs the front-end with the coefficient dump as rate_curve does (same slot and d_work rules), then, for
+    // the fused back-end's shapes, one launch of its SSE mode over all 64 steps, otherwise per step the symbols, the
+    // two-kernel back-end into an RGB scratch and a squared-difference sum; one synchronisation.  Allocates on the first
+    // call the rate curve's coefficient buffer, 64 sums, and for the general path an RGB scratch of 3 B per pixel.
+    int psnr_curve(uint8_t wavelet, const uint8_t *d_rgb, uint64_t sse[kRateSteps], uint32_t slot = 0,
+                   uint8_t *d_work = nullptr);
 
     // staging buffers for host-pointer entry points
     uint8_t *rgb_stage(uint32_t slot);          // device buffer of 3*n_pixels bytes, allocated on first use
@@ -197,6 +206,7 @@ private:
     int begin_step_ = 1;                       // encode_begin's step, for submits that name none
     // rate curve (allocated by the first rate_curve call)
     bool ensure_rate_buffers();
+    int dump_frontend(uint8_t wavelet, const uint8_t *d_rgb, uint32_t slot, uint8_t *d_work, uint8_t *&sym);
     int32_t *d_coef_ = nullptr;                // i32 [3][N] coefficients
     unsigned *d_vhist_ = nullptr;              // [3][2*bound+1] value histogram (largest bound of the three wavelets)
     unsigned *d_rate_hist_ = nullptr;          // [64][3][256]
@@ -206,6 +216,11 @@ private:
     DecAux *d_rate_aux_ = nullptr;             // [192]
     unsigned long long *d_rate_est_ = nullptr; // [192]
     unsigned long long *d_rate_out_ = nullptr, *h_rate_out_ = nullptr;   // [64] sizes + [1] out-of-range count
+    // PSNR curve (allocated by the first psnr_curve call)
+    bool ensure_psnr_buffers(bool rgb_scratch);
+    unsigned long long *d_sse_ = nullptr, *h_sse_ = nullptr;             // [64]
+    InvSseJob *d_sse_jobs_ = nullptr, *h_sse_jobs_ = nullptr;             // [64] (fused path)
+    uint8_t *d_sse_rgb_ = nullptr;                                       // decode of one step, 3 B per pixel (general path)
     // pinned host mirrors
     unsigned long long *h_results_ = nullptr;
     unsigned *h_hist_ = nullptr;

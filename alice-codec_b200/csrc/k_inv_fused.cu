@@ -21,10 +21,20 @@
 //             of the t buffer, lane-parallel inverse x lifting (warp shuffles, lanes 0/15 of a half-warp are halo lanes, so
 //             the t phase also produces the two halo lanes' columns), i16 truncation, inverse colour transform, clamp,
 //             12-byte RGB stores.
+//
+// SSE mode (SSE = true, PSNR curve of a chunk, DESIGN.md 4.9): the same decode of the coefficient dump at one quantiser
+// step per job, compared with the chunk's input instead of stored.  Only two points differ: the t phase reads the i32
+// coefficients at the symbols' index and maps each through quant_symbol (quant.cuh) and sym_to_coef_narrow with the
+// job's step, and emit_row loads the 12 input bytes it would have stored to and sums the squared differences (a warp
+// reduction and one atomicAdd per warp at the end).  A launch runs the kRateSteps jobs of one tile next to each other
+// (block = tile * kRateSteps + job), so the 64 decodes of a tile read its coefficients from L2.
 #include <stdlib.h>
+
+#include <type_traits>
 
 #include "kernels.h"
 #include "lifting.cuh"
+#include "quant.cuh"
 
 namespace alice {
 
@@ -47,19 +57,21 @@ ALICE_D uint32_t clamp_u8_i16(int v) {
     return t < 0 ? 0u : (t > 255 ? 255u : (uint32_t)t);
 }
 
-template <int WT>
+template <int WT, bool SSE>
 __global__ void ALICE_LAUNCH_BOUNDS(kIfNT, 1)
-k_inv_fused(const InvFusedJob *__restrict__ jobs, int w, int h, int n_strips, int seg_pairs, int step0, int step1, int step2) {
+k_inv_fused(const std::conditional_t<SSE, InvSseJob, InvFusedJob> *__restrict__ jobs, int w, int h, int n_strips,
+            int seg_pairs, int step0, int step1, int step2) {
     constexpr int NST = WaveletTraits<WT>::NST;
     constexpr int Q = kIfQ;
     ALICE_DYN_SMEM(smem);
     int16_t *tbuf = reinterpret_cast<int16_t *>(smem);
 
-    const InvFusedJob job = jobs[blockIdx.y];
+    const auto job = jobs[SSE ? blockIdx.x % (unsigned)kRateSteps : blockIdx.y];
+    const unsigned tile = SSE ? blockIdx.x / (unsigned)kRateSteps : blockIdx.x;
     const int tid = threadIdx.x, lane = tid & 31, wv = tid >> 5;
-    const int s = (int)(blockIdx.x % (unsigned)n_strips);
-    const int twin = (int)((blockIdx.x / (unsigned)n_strips) & 1u);
-    const int seg = (int)(blockIdx.x / (2u * (unsigned)n_strips));
+    const int s = (int)(tile % (unsigned)n_strips);
+    const int twin = (int)((tile / (unsigned)n_strips) & 1u);
+    const int seg = (int)(tile / (2u * (unsigned)n_strips));
     const int halfx = w >> 1, halfy = h >> 1;
     const uint32_t fs32 = (uint32_t)w * (uint32_t)h;
     const int i0 = seg * seg_pairs, i1 = min(halfy, i0 + seg_pairs);
@@ -68,11 +80,16 @@ k_inv_fused(const InvFusedJob *__restrict__ jobs, int w, int h, int n_strips, in
     const int xl = lane & 15;
     const int p0 = kIfVP * s - 2 + 2 * xl;        // first of this lane's two pairs
     const bool lane_ok = xl >= 1 && xl <= 14 && p0 < halfx;
-    uint8_t *out_frame = job.rgb + (size_t)(32 * twin + fi) * fs32 * 3;
+    // this half-warp's frame of the output (decode) or of the input (SSE mode)
+    auto *const out_frame = [&] { if constexpr (SSE) return job.ref_rgb; else return job.rgb; }() +
+                            (size_t)(32 * twin + fi) * fs32 * 3;
+    unsigned long long sse = 0;   // SSE mode: this thread's sum of squared differences
 
     // ---- t phase: row pairs [jg, jg + nq) -> t-buffer slots 0 .. nq-1
     auto t_phase = [&](int jg, int nq) {
         const int n_items = nq * kIfLines;
+        QuantDev qd;
+        if constexpr (SSE) qd = make_quant_dev(job.step);
         for (int item = tid; item < n_items; item += kIfNT) {
             const int qq = item / kIfLines, r = item - qq * kIfLines;
             const int ch = r / (2 * kIfCols), rr = r - ch * (2 * kIfCols);
@@ -85,19 +102,30 @@ k_inv_fused(const InvFusedJob *__restrict__ jobs, int w, int h, int n_strips, in
                 continue;
             }
             const int j = jg + qq;
-            const int step = ch == 0 ? step0 : (ch == 1 ? step1 : step2);
+            int step;
+            if constexpr (SSE) step = job.step;
+            else step = ch == 0 ? step0 : (ch == 1 ? step1 : step2);
             const uint32_t pos = (uint32_t)(row ? halfy + j : j) * (uint32_t)w + (uint32_t)(xh ? halfx + pair : pair);
             const int tp0 = twin ? 16 - NST : 0;                                   // first t-pair pushed
-            const uint8_t *pl = job.symbols + ((uint32_t)ch * 64u + (uint32_t)tp0) * fs32 + pos;   // low-t symbol of the next pair
             const uint32_t hi_delta = 32u * fs32;                                  // its high-t symbol
             // Every symbol of the line first (2 * (16 + NST) one-byte loads in flight per thread: the phase was bound by
             // the latency of these loads when they were issued four pairs at a time), then the lifting.
             constexpr int NP = 16 + NST;
             uint32_t sl[NP], sh[NP];
+            if constexpr (SSE) {
+                const int32_t *pl = job.coef + ((uint32_t)ch * 64u + (uint32_t)tp0) * fs32 + pos;
 #pragma unroll
-            for (int jt = 0; jt < NP; jt++) {
-                sl[jt] = __ldg(pl + (uint32_t)jt * fs32);
-                sh[jt] = __ldg(pl + hi_delta + (uint32_t)jt * fs32);
+                for (int jt = 0; jt < NP; jt++) {
+                    sl[jt] = quant_symbol(__ldg(pl + (uint32_t)jt * fs32), qd);
+                    sh[jt] = quant_symbol(__ldg(pl + hi_delta + (uint32_t)jt * fs32), qd);
+                }
+            } else {
+                const uint8_t *pl = job.symbols + ((uint32_t)ch * 64u + (uint32_t)tp0) * fs32 + pos;   // low-t symbol of the next pair
+#pragma unroll
+                for (int jt = 0; jt < NP; jt++) {
+                    sl[jt] = __ldg(pl + (uint32_t)jt * fs32);
+                    sh[jt] = __ldg(pl + hi_delta + (uint32_t)jt * fs32);
+                }
             }
             InvLift<WT, false> T;
             int ev, od;
@@ -157,10 +185,25 @@ k_inv_fused(const InvFusedJob *__restrict__ jobs, int w, int h, int n_strips, in
             bytes[3 * i + 1] = clamp_u8_i16(g);
             bytes[3 * i + 2] = clamp_u8_i16(b);
         }
-        uint32_t *dst = reinterpret_cast<uint32_t *>(out_frame + ((size_t)y * w + 2 * p0) * 3);
+        if constexpr (SSE) {
+            const uint32_t *ref = reinterpret_cast<const uint32_t *>(out_frame + ((size_t)y * w + 2 * p0) * 3);
+            unsigned part = 0;   // at most 12 * 255^2
 #pragma unroll
-        for (int q4 = 0; q4 < 3; q4++)
-            dst[q4] = bytes[4 * q4] | (bytes[4 * q4 + 1] << 8) | (bytes[4 * q4 + 2] << 16) | (bytes[4 * q4 + 3] << 24);
+            for (int q4 = 0; q4 < 3; q4++) {
+                const uint32_t r = __ldg(ref + q4);
+#pragma unroll
+                for (int b = 0; b < 4; b++) {
+                    const int d = (int)((r >> (8 * b)) & 0xffu) - (int)bytes[4 * q4 + b];
+                    part += (unsigned)(d * d);
+                }
+            }
+            sse += part;
+        } else {
+            uint32_t *dst = reinterpret_cast<uint32_t *>(out_frame + ((size_t)y * w + 2 * p0) * 3);
+#pragma unroll
+            for (int q4 = 0; q4 < 3; q4++)
+                dst[q4] = bytes[4 * q4] | (bytes[4 * q4 + 1] << 8) | (bytes[4 * q4 + 2] << 16) | (bytes[4 * q4 + 3] << 24);
+        }
     };
     auto emit_pair = [&](int jo, int (&ev)[3][4], int (&od)[3][4]) {
         const bool active = jo >= i0 && jo < i1;
@@ -222,6 +265,11 @@ k_inv_fused(const InvFusedJob *__restrict__ jobs, int w, int h, int n_strips, in
             if (has) emit_pair(halfy - NST + which, ev, od);
         }
     }
+    if constexpr (SSE) {
+#pragma unroll
+        for (int d = 16; d > 0; d >>= 1) sse += __shfl_xor_sync(kFullMask, sse, d);
+        if (lane == 0 && sse) atomicAdd(job.sse, sse);
+    }
 }
 
 bool inverse_fused_eligible(const uint8_t *d_symbols, const uint8_t *d_rgb, int w, int h, int f, const int steps[3]) {
@@ -234,8 +282,10 @@ bool inverse_fused_eligible(const uint8_t *d_symbols, const uint8_t *d_rgb, int 
     return f == 64 && (h & 1) == 0 && h >= 2 && (w & 15) == 0 && w >= 80 && (reinterpret_cast<uintptr_t>(d_rgb) & 3) == 0;
 }
 
-template <int WT>
-static void launch_inv_fused(const InvFusedJob *d_jobs, int n_jobs, int w, int h, const int steps[3], int n_sms, cudaStream_t st) {
+// SSE = true: n_jobs == kRateSteps, one block per (tile, job), the jobs of a tile adjacent
+template <int WT, bool SSE>
+static void launch_inv_fused(const std::conditional_t<SSE, InvSseJob, InvFusedJob> *d_jobs, int n_jobs, int w, int h,
+                             const int steps[3], int n_sms, cudaStream_t st) {
     constexpr int NST = WaveletTraits<WT>::NST;
     const int halfx = w / 2, halfy = h / 2;
     const int n_strips = (halfx + kIfVP - 1) / kIfVP;
@@ -250,8 +300,9 @@ static void launch_inv_fused(const InvFusedJob *d_jobs, int n_jobs, int w, int h
     }
     const int seg_pairs = (halfy + best_segs - 1) / best_segs;
     const int n_segs = (halfy + seg_pairs - 1) / seg_pairs;
-    const dim3 grid((unsigned)(2 * n_strips * n_segs), (unsigned)n_jobs);
-    auto kf = k_inv_fused<WT>;
+    const unsigned tiles = (unsigned)(2 * n_strips * n_segs);
+    const dim3 grid = SSE ? dim3(tiles * (unsigned)n_jobs) : dim3(tiles, (unsigned)n_jobs);
+    auto kf = k_inv_fused<WT, SSE>;
 #ifndef ALICE_EMUL
     static unsigned long long done = 0;
     int dev = 0;
@@ -268,9 +319,18 @@ void inverse_backend_fused(int wavelet, const InvFusedJob *d_jobs, int n_jobs, i
                            cudaStream_t st) {
     if (n_jobs <= 0) return;
     switch (wavelet) {
-    case WT_CDF53: launch_inv_fused<WT_CDF53>(d_jobs, n_jobs, w, h, steps, n_sms, st); break;
-    case WT_CDF97: launch_inv_fused<WT_CDF97>(d_jobs, n_jobs, w, h, steps, n_sms, st); break;
-    default:       launch_inv_fused<WT_HAAR>(d_jobs, n_jobs, w, h, steps, n_sms, st); break;
+    case WT_CDF53: launch_inv_fused<WT_CDF53, false>(d_jobs, n_jobs, w, h, steps, n_sms, st); break;
+    case WT_CDF97: launch_inv_fused<WT_CDF97, false>(d_jobs, n_jobs, w, h, steps, n_sms, st); break;
+    default:       launch_inv_fused<WT_HAAR, false>(d_jobs, n_jobs, w, h, steps, n_sms, st); break;
+    }
+}
+
+void inverse_sse_fused(int wavelet, const InvSseJob *d_jobs, int w, int h, int n_sms, cudaStream_t st) {
+    const int steps[3] = {0, 0, 0};   // each job names its own
+    switch (wavelet) {
+    case WT_CDF53: launch_inv_fused<WT_CDF53, true>(d_jobs, kRateSteps, w, h, steps, n_sms, st); break;
+    case WT_CDF97: launch_inv_fused<WT_CDF97, true>(d_jobs, kRateSteps, w, h, steps, n_sms, st); break;
+    default:       launch_inv_fused<WT_HAAR, true>(d_jobs, kRateSteps, w, h, steps, n_sms, st); break;
     }
 }
 

@@ -132,6 +132,21 @@ void step_hists(const unsigned *d_vhist, int bound, unsigned long long n, unsign
     ALICE_LAUNCH(k_step_hists, dim3(kRateSteps, 3), dim3(256), 0, st, d_vhist, bound, n, d_hist);
 }
 
+// ------------------------------------------------------------------------------------ PSNR curve, general shapes
+// The symbols of one step from the coefficient dump (the front-end's own quantiser), for inverse_backend.
+__global__ void k_coef_symbols(const int32_t *__restrict__ coef, unsigned long long n, QuantDev q, uint8_t *__restrict__ sym) {
+    const unsigned long long nth = (unsigned long long)gridDim.x * blockDim.x;
+    for (unsigned long long i = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += nth)
+        sym[i] = (uint8_t)quant_symbol(__ldg(coef + i), q);
+}
+
+void coef_symbols(const int32_t *d_coef, unsigned long long n, int step, uint8_t *d_sym, cudaStream_t st) {
+    if (n == 0) return;
+    const unsigned gx = (unsigned)std::max<long long>(1, std::min<long long>((long long)((n + 255) / 256),
+                                                                          (long long)device_sm_count() * 8));
+    ALICE_LAUNCH(k_coef_symbols, dim3(gx), dim3(256), 0, st, d_coef, n, make_quant_dev(step), d_sym);
+}
+
 // ------------------------------------------------------------------------------------------- chunk sizes
 // bytes[i] = header_bytes + the three channels' predicted stream bytes at step i + 1, or UINT64_MAX where a used symbol
 // has frequency 0 (EncSym.cmpl == 4096: the reference divides by zero there and the encoder reports ALICE_ERR_PANIC).

@@ -107,6 +107,20 @@ void step_hists(const unsigned *d_vhist, int bound, unsigned long long n, unsign
 void rate_sizes(const unsigned *d_hist, const EncSym *d_enc, const unsigned long long *d_est, unsigned long long n,
                 unsigned long long header_bytes, unsigned long long *d_bytes, cudaStream_t st);
 
+// ---- PSNR curve (DESIGN.md 4.9): the squared error of the decode at every step, from the front-end's coefficient dump
+// sym [n] = quant_symbol(coef[i], step): the symbols a front-end at that step writes (k_rate.cu)
+void coef_symbols(const int32_t *d_coef, unsigned long long n, int step, uint8_t *d_sym, cudaStream_t st);
+// The SSE mode of the fused back-end (k_inv_fused.cu): kRateSteps jobs in one launch, each decodes the coefficient dump
+// at its step and adds sum((ref - decode)^2) over the chunk to *sse (zeroed by the caller).  The shapes, alignment and
+// bound of inverse_fused_eligible (with ref_rgb in place of the output).
+struct InvSseJob {
+    const int32_t *coef;       // [3][64][h][w] coefficient dump of the front-end
+    const uint8_t *ref_rgb;    // [64][h][w][3] the chunk's input
+    unsigned long long *sse;
+    int step;
+};
+void inverse_sse_fused(int wavelet, const InvSseJob *d_jobs, int w, int h, int n_sms, cudaStream_t st);
+
 // ---- generic element-wise / line kernels behind the public stage API (k_generic.cu) -----
 void lift_axis(int32_t *d_data, int32_t *d_tmp, int wavelet, bool inverse, int axis, long long w, long long h,
                long long d, cudaStream_t st);  // one 1-D transform along `axis` (0=x,1=y,2=t) of every line

@@ -320,6 +320,33 @@ EncodedChunk *alice_codec_encode_to_size_ex(uint8_t wavelet, const uint8_t *rgb,
 int alice_codec_batch_encode_host_to_size(AliceBatch *b, const uint8_t *const *h_rgb, uint32_t n, uint64_t max_bytes,
                                           EncodedChunk **out_chunks, uint8_t *qualities_out);
 
+/* ---- PSNR-target encoding (DESIGN.md 4.9), for ALICE_ENCODE_WELL_FORMED_TABLES encodes only: such a chunk decodes to
+ * exactly the symbols it encodes, so the decode at every step follows from one transform pass, without rANS work.  The
+ * default encode has no such curve.  sse64[i] = the sum over the chunk's 3*w*h*f bytes of (input - decode)^2 for the
+ * well-formed encode at step i+1 (an exact integer), psnr64[i] = 10 log10(255^2 / (sse / len)), +inf where sse == 0:
+ * bit for bit what alice_codec_psnr gives for the input and that decode.  PSNR is not monotone in the step (small steps
+ * wrap symbols mod 256), so the curve holds every step.  An empty input (a zero dimension) gives +inf and 0 at every
+ * step.  These calls take no flags: they always mean the well-formed encode. */
+/* sse64 may be null */
+int alice_codec_psnr_curve(uint8_t wavelet, const uint8_t *rgb, uint64_t rgb_len, uint32_t width, uint32_t height,
+                           uint32_t frames, double *psnr64, uint64_t *sse64);
+/* the same for RGB in device memory; the call waits for the work enqueued on cuda_stream before it reads d_rgb */
+int alice_codec_psnr_curve_device(uint8_t wavelet, const uint8_t *d_rgb, uint32_t width, uint32_t height,
+                                  uint32_t frames, double *psnr64, uint64_t *sse64, void *cuda_stream);
+/* the lowest quality that reaches min_psnr_db: the largest step s with psnr64[s-1] >= min_psnr_db, encoded at
+ * *quality_out = the largest quality with that step; the chunk is byte-identical to an encode with
+ * ALICE_ENCODE_WELL_FORMED_TABLES at that quality.  No step reaches the target, or the target is NaN: null,
+ * ALICE_ERR_QUANT_STEP, and the message names the best PSNR of the curve and its quality.  An empty input gives the empty
+ * chunk at the quality of step 64. */
+EncodedChunk *alice_codec_encode_to_psnr(uint8_t wavelet, const uint8_t *rgb, uint64_t rgb_len, uint32_t width,
+                                         uint32_t height, uint32_t frames, double min_psnr_db, uint8_t *quality_out);
+/* host-buffer batch form (the batch must have ALICE_BATCH_WELL_FORMED_TABLES, else ALICE_ERR_DIMENSIONS): every chunk at
+ * its own lowest quality that reaches min_psnr_db, all 3n rANS streams concurrently.  The batch's own quality is not
+ * used.  The first call allocates what the rate curve allocates, and for shapes the fused back-end does not take (or
+ * batches with ALICE_BATCH_SMALL_SMEM_KERNELS) an RGB scratch of 3 B per pixel. */
+int alice_codec_batch_encode_host_to_psnr(AliceBatch *b, const uint8_t *const *h_rgb, uint32_t n, double min_psnr_db,
+                                          EncodedChunk **out_chunks, uint8_t *qualities_out);
+
 /* synthetic RGB volumes generated on the device (SURVEY.md Appendix D): kind 0=G0, 1=G1, 2=G2 */
 int alice_codec_synth_rgb_device(int kind, uint32_t seed, uint32_t width, uint32_t height, uint32_t frames,
                                  uint8_t *d_rgb, void *cuda_stream);

@@ -4,9 +4,9 @@
 # compiled with AddressSanitizer and driven through the same parity checks as tests/test_emul_parity.py.
 set -e
 ROOT=$(cd "$(dirname "$0")/.." && pwd)
-OUT=${TMPDIR:-/tmp}/alice_asan
+OUT=$ROOT/tests/emul/_build/asan   # under tests/emul/_build: parity.device_of treats it as an emulator build
 mkdir -p "$OUT"
-for f in k_forward k_fwd_fused k_inv_fused k_inverse k_rans k_generic k_wavelet_i32 k_rdo k_synth engine lossless capi; do
+for f in k_forward k_fwd_fused k_inv_fused k_inverse k_rans k_generic k_wavelet_i32 k_rdo k_rate k_synth engine lossless capi; do
   g++ -O1 -g -std=c++17 -fPIC -fwrapv -DALICE_EMUL -x c++ -Wno-unknown-pragmas -I "$ROOT/tests/emul" \
       -fsanitize=address -fno-omit-frame-pointer -c "$ROOT/alice-codec_b200/csrc/$f.cu" -o "$OUT/$f.o" &
 done
@@ -51,6 +51,10 @@ parity.check_payload_arena(api)
 parity.check_submit_collect(api)
 parity.check_stream_device(api)
 parity.check_shifted_in_place(api)
+# the PSNR curve: the SSE mode of the fused back-end (80x2x64) and the general path (24x10x6)
+for shape in [(24, 10, 6), (80, 2, 64)]:
+    for wv in (0, 1, 2):
+        parity.pkg.FrameEncoder(80, parity.WV[wv], api=api, well_formed_tables=True).psnr_curve(O.generate(O.G1, *shape), *shape)
 print("ASAN RUN OK")
 PY
 LD_PRELOAD=$(gcc -print-file-name=libasan.so) ASAN_OPTIONS=detect_leaks=0:detect_stack_use_after_return=0 python "$OUT/run.py"
