@@ -48,15 +48,11 @@ def quality_for_step(step: int) -> int:
     return max(q for q in range(101) if quality_to_step(q) == step)
 
 
-def _curve_dict(sizes):
-    """{quality: predicted .alc bytes} over the 64 steps (highest quality first); None where the reference aborts"""
-    return {quality_for_step(s): (None if int(sizes[s - 1]) == UINT64_MAX else int(sizes[s - 1]))
-            for s in range(1, RATE_STEPS + 1)}
-
-
-def _psnr_dict(psnr):
-    """{quality: PSNR in dB} over the 64 steps (highest quality first), keyed as _curve_dict"""
-    return {quality_for_step(s): float(psnr[s - 1]) for s in range(1, RATE_STEPS + 1)}
+def _by_quality(curve):
+    """{quality: curve[step - 1]} over the 64 steps (highest quality first): a rate curve's predicted .alc bytes (None
+    where the reference aborts) or a PSNR curve's dB"""
+    return {quality_for_step(s): None if curve.dtype == np.uint64 and int(v) == UINT64_MAX else v.item()
+            for s, v in enumerate(curve, 1)}
 
 
 def _wavelet_byte(wavelet) -> int:
@@ -478,34 +474,18 @@ class FrameEncoder:
         where the reference aborts.  The encoder's wavelet and table mode are used, its quality is not.  with_hist=True
         also returns the symbol histograms, uint32 [64][3][256] (row step - 1): what the headers of default encodes hold.
         With well_formed_tables the sizes bound the well-formed encodes, and no step is None."""
-        a, pa = _u8(rgb_frames)
-        sizes = np.zeros(RATE_STEPS, np.uint64)
-        hist = np.zeros((RATE_STEPS, 3, 256), np.uint32) if with_hist else None
-        self._api._chk(self._api.lib.alice_codec_rate_curve_ex(
-            self.wavelet, pa, a.size, width, height, frames, sizes.ctypes.data_as(_capi.u64p),
-            hist.ctypes.data_as(_capi.u32p) if with_hist else None, self._flags))
-        return (_curve_dict(sizes), hist) if with_hist else _curve_dict(sizes)
+        return self._curve(False, rgb_frames, width, height, frames, with_hist)
 
     def rate_curve_device(self, d_rgb: int, width: int, height: int, frames: int, stream: int = 0, with_hist: bool = False):
         """rate_curve for RGB in device memory (raw device pointer); waits for the work enqueued on `stream` first"""
-        sizes = np.zeros(RATE_STEPS, np.uint64)
-        hist = np.zeros((RATE_STEPS, 3, 256), np.uint32) if with_hist else None
-        self._api._chk(self._api.lib.alice_codec_rate_curve_device_ex(
-            self.wavelet, C.c_void_p(int(d_rgb)), width, height, frames, sizes.ctypes.data_as(_capi.u64p),
-            hist.ctypes.data_as(_capi.u32p) if with_hist else None, C.c_void_p(stream), self._flags))
-        return (_curve_dict(sizes), hist) if with_hist else _curve_dict(sizes)
+        return self._curve(False, d_rgb, width, height, frames, with_hist, device=True, stream=stream)
 
     def encode_to_size(self, rgb_frames, width: int, height: int, frames: int, max_bytes: int):
         """The chunk at the highest quality whose .alc (to_bytes) is at most max_bytes: (EncodedChunk, quality), the
         chunk byte-identical to FrameEncoder(quality, wavelet, well_formed_tables=...).encode.  The encoder's quality is
         not used.  Raises CodecError InvalidBufferSize if no quality fits."""
-        a, pa = _u8(rgb_frames)
-        q = C.c_uint8()
-        h = self._api.lib.alice_codec_encode_to_size_ex(self.wavelet, pa, a.size, width, height, frames, int(max_bytes),
-                                                        C.byref(q), self._flags)
-        if not h:
-            self._api._raise()
-        return EncodedChunk(h, self._api), q.value
+        return self._encode_to(self._api.lib.alice_codec_encode_to_size_ex, rgb_frames, width, height, frames,
+                               int(max_bytes), self._flags)
 
     def _need_well_formed(self):
         if not self.well_formed_tables:
@@ -518,33 +498,48 @@ class FrameEncoder:
         psnr(rgb, FrameDecoder().decode(FrameEncoder(quality, wavelet, well_formed_tables=True).encode(rgb, ...))) bit
         for bit; inf where the decode is exact.  Not monotone in the quality.  with_sse=True also returns the sums of
         squared differences, uint64 [64] (index step - 1).  Well-formed-tables encoders only (DESIGN.md 4.9)."""
-        self._need_well_formed()
-        a, pa = _u8(rgb_frames)
-        psnr, sse = np.zeros(RATE_STEPS, np.float64), np.zeros(RATE_STEPS, np.uint64)
-        self._api._chk(self._api.lib.alice_codec_psnr_curve(
-            self.wavelet, pa, a.size, width, height, frames, psnr.ctypes.data_as(C.POINTER(C.c_double)),
-            sse.ctypes.data_as(_capi.u64p)))
-        return (_psnr_dict(psnr), sse) if with_sse else _psnr_dict(psnr)
+        return self._curve(True, rgb_frames, width, height, frames, with_sse)
 
     def psnr_curve_device(self, d_rgb: int, width: int, height: int, frames: int, stream: int = 0,
                           with_sse: bool = False):
         """psnr_curve for RGB in device memory (raw device pointer); waits for the work enqueued on `stream` first"""
-        self._need_well_formed()
-        psnr, sse = np.zeros(RATE_STEPS, np.float64), np.zeros(RATE_STEPS, np.uint64)
-        self._api._chk(self._api.lib.alice_codec_psnr_curve_device(
-            self.wavelet, C.c_void_p(int(d_rgb)), width, height, frames, psnr.ctypes.data_as(C.POINTER(C.c_double)),
-            sse.ctypes.data_as(_capi.u64p), C.c_void_p(stream)))
-        return (_psnr_dict(psnr), sse) if with_sse else _psnr_dict(psnr)
+        return self._curve(True, d_rgb, width, height, frames, with_sse, device=True, stream=stream)
 
     def encode_to_psnr(self, rgb_frames, width: int, height: int, frames: int, min_psnr: float):
         """The chunk at the lowest quality whose decode reaches min_psnr dB: (EncodedChunk, quality), the chunk
         byte-identical to FrameEncoder(quality, wavelet, well_formed_tables=True).encode.  The encoder's quality is not
         used.  Raises CodecError InvalidQuantStep if no quality reaches the target, or if it is NaN."""
         self._need_well_formed()
+        return self._encode_to(self._api.lib.alice_codec_encode_to_psnr, rgb_frames, width, height, frames,
+                               float(min_psnr))
+
+    def _curve(self, psnr, rgb, width, height, frames, with_extra, device=False, stream=0):
+        """The rate curve, or (psnr=True) the PSNR curve, of host RGB or (device=True) of the RGB at device pointer rgb:
+        {quality: value}, and with_extra the histograms or the sums of squared differences."""
+        L = self._api.lib
+        if psnr:
+            self._need_well_formed()
+            curve, extra = np.zeros(RATE_STEPS, np.float64), np.zeros(RATE_STEPS, np.uint64)
+            fn = L.alice_codec_psnr_curve_device if device else L.alice_codec_psnr_curve
+            outs, flags = (curve.ctypes.data_as(C.POINTER(C.c_double)), extra.ctypes.data_as(_capi.u64p)), ()
+        else:
+            curve = np.zeros(RATE_STEPS, np.uint64)
+            extra = np.zeros((RATE_STEPS, 3, 256), np.uint32) if with_extra else None
+            fn = L.alice_codec_rate_curve_device_ex if device else L.alice_codec_rate_curve_ex
+            outs = (curve.ctypes.data_as(_capi.u64p), extra.ctypes.data_as(_capi.u32p) if with_extra else None)
+            flags = (self._flags,)
+        if device:
+            self._api._chk(fn(self.wavelet, C.c_void_p(int(rgb)), width, height, frames, *outs, C.c_void_p(stream), *flags))
+        else:
+            a, pa = _u8(rgb)
+            self._api._chk(fn(self.wavelet, pa, a.size, width, height, frames, *outs, *flags))
+        return (_by_quality(curve), extra) if with_extra else _by_quality(curve)
+
+    def _encode_to(self, fn, rgb_frames, width, height, frames, target, *flags):
+        """the chunk and quality that alice_codec_encode_to_size_ex or _to_psnr (fn) choose for target"""
         a, pa = _u8(rgb_frames)
         q = C.c_uint8()
-        h = self._api.lib.alice_codec_encode_to_psnr(self.wavelet, pa, a.size, width, height, frames, float(min_psnr),
-                                                     C.byref(q))
+        h = fn(self.wavelet, pa, a.size, width, height, frames, target, C.byref(q), *flags)
         if not h:
             self._api._raise()
         return EncodedChunk(h, self._api), q.value
@@ -686,13 +681,7 @@ class ChunkBatch:
     def encode_host_to_size(self, h_rgb_ptrs, max_bytes: int):
         """encode_host with every chunk at the highest quality whose .alc fits max_bytes: (chunks, qualities).  The
         batch's quality is not used."""
-        n = len(h_rgb_ptrs)
-        arr = self._ptr_array(h_rgb_ptrs)
-        out = (C.c_void_p * n)()
-        q = np.zeros(max(n, 1), np.uint8)
-        self._api._chk(self._api.lib.alice_codec_batch_encode_host_to_size(self._h, arr, n, int(max_bytes), out,
-                                                                           q.ctypes.data_as(_capi.u8p)))
-        return [EncodedChunk(C.c_void_p(out[i]), self._api) for i in range(n)], [int(x) for x in q[:n]]
+        return self._encode_host_to(self._api.lib.alice_codec_batch_encode_host_to_size, h_rgb_ptrs, int(max_bytes))
 
     def encode_host_to_psnr(self, h_rgb_ptrs, min_psnr: float):
         """encode_host with every chunk at the lowest quality whose decode reaches min_psnr dB: (chunks, qualities).
@@ -700,12 +689,15 @@ class ChunkBatch:
         if not self.well_formed_tables:
             raise ValueError("the PSNR curve describes the well-formed-tables encode only: "
                              "make the batch with well_formed_tables=True")
+        return self._encode_host_to(self._api.lib.alice_codec_batch_encode_host_to_psnr, h_rgb_ptrs, float(min_psnr))
+
+    def _encode_host_to(self, fn, h_rgb_ptrs, target):
+        """the chunks and qualities that alice_codec_batch_encode_host_to_size or _to_psnr (fn) choose for target"""
         n = len(h_rgb_ptrs)
         arr = self._ptr_array(h_rgb_ptrs)
         out = (C.c_void_p * n)()
         q = np.zeros(max(n, 1), np.uint8)
-        self._api._chk(self._api.lib.alice_codec_batch_encode_host_to_psnr(self._h, arr, n, float(min_psnr), out,
-                                                                           q.ctypes.data_as(_capi.u8p)))
+        self._api._chk(fn(self._h, arr, n, target, out, q.ctypes.data_as(_capi.u8p)))
         return [EncodedChunk(C.c_void_p(out[i]), self._api) for i in range(n)], [int(x) for x in q[:n]]
 
     def submit_host(self, i, h_rgb_ptr):

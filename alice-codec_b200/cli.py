@@ -40,16 +40,20 @@ def cmd_encode(a) -> None:
         raise ValueError("--min-psnr and --max-bytes cannot be combined")
     rgb = np.fromfile(a.input, dtype=np.uint8)
     enc = pkg.FrameEncoder(a.quality, a.wavelet, well_formed_tables=a.well_formed_tables)
-    budget = a.max_bytes
-    qualities = []                                  # --max-bytes / --min-psnr: the quality chosen for each chunk
+    # --max-bytes / --min-psnr: every chunk is encoded at the quality that these calls choose for `goal`
+    goal = None
+    if a.max_bytes is not None:
+        goal, single, batched, label = (a.max_bytes, enc.encode_to_size, pkg.ChunkBatch.encode_host_to_size,
+                                        f"max-bytes={a.max_bytes} per chunk")
+    elif target is not None:
+        goal, single, batched, label = (target, enc.encode_to_psnr, pkg.ChunkBatch.encode_host_to_psnr,
+                                        f"min-psnr={target} dB per chunk")
+    qualities = []                                  # the quality chosen for each chunk
 
     def one(part, nf):
-        if budget is None and target is None:
+        if goal is None:
             return enc.encode(part, a.width, a.height, nf).to_bytes()
-        if budget is not None:
-            chunk, q = enc.encode_to_size(part, a.width, a.height, nf, budget)
-        else:
-            chunk, q = enc.encode_to_psnr(part, a.width, a.height, nf, target)
+        chunk, q = single(part, a.width, a.height, nf, goal)
         qualities.append(q)
         return chunk.to_bytes()
 
@@ -65,14 +69,11 @@ def cmd_encode(a) -> None:
                                    well_formed_tables=a.well_formed_tables)
             cb = per * a.chunk_frames
             parts = [np.ascontiguousarray(rgb[i * cb:(i + 1) * cb]) for i in range(n_full)]
-            if budget is not None:
-                chunks, qs = batch.encode_host_to_size([p.ctypes.data for p in parts], budget)
-                qualities.extend(qs)
-            elif target is not None:
-                chunks, qs = batch.encode_host_to_psnr([p.ctypes.data for p in parts], target)
-                qualities.extend(qs)
-            else:
+            if goal is None:
                 chunks = batch.encode_host([p.ctypes.data for p in parts])
+            else:
+                chunks, qs = batched(batch, [p.ctypes.data for p in parts], goal)
+                qualities.extend(qs)
             blobs = [c.to_bytes() for c in chunks]
             batch.close()
         else:
@@ -86,9 +87,7 @@ def cmd_encode(a) -> None:
     with open(a.output, "wb") as f:
         f.write(data)
     ratio = len(data) / rgb.size if rgb.size else 0.0
-    chosen = ",".join(str(q) for q in qualities)
-    setting = (f"max-bytes={budget} per chunk, quality={chosen}" if budget is not None else
-               f"min-psnr={target} dB per chunk, quality={chosen}" if target is not None else f"quality={a.quality}")
+    setting = f"quality={a.quality}" if goal is None else f"{label}, quality={','.join(str(q) for q in qualities)}"
     tables = ", tables=well-formed" if a.well_formed_tables else ""
     sys.stderr.write(f"encoded {a.width}x{a.height}x{a.frames} ({rgb.size} bytes) -> {len(data)} bytes "
                      f"({ratio * 100:.1f}% ratio, {setting}, wavelet={a.wavelet}{tables})\n")

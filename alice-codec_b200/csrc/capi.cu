@@ -187,7 +187,7 @@ EncodedChunk *encode_impl(const FrameEncoder *enc, const uint8_t *rgb, uint64_t 
     return out;
 }
 
-// ------------------------------------------------------------------------------ rate control
+// ------------------------------------------------------------------------------ quality targets
 constexpr uint64_t kAlcHeaderBytes = kFixedHeaderBytes + 3 * kChannelHeaderBytes;   // 3138
 
 // the largest quality in 0..=100 whose step is s (every step has one: 63q/100 takes every integer 0..63)
@@ -197,26 +197,92 @@ uint8_t quality_for_step(int s) {
     return 100;
 }
 
-// the smallest step >= first whose prediction fits max_bytes (the highest quality; sizes are not assumed monotone in the
-// step), 0 if there is none
-int pick_step(const uint64_t pred[kRateSteps], uint64_t max_bytes, int first) {
-    for (int s = first; s <= kRateSteps; s++)
-        if (pred[s - 1] != UINT64_MAX && pred[s - 1] <= max_bytes) return s;
-    return 0;
-}
-
-void set_no_fit_error(const uint64_t pred[kRateSteps], uint64_t max_bytes) {
-    uint64_t best = UINT64_MAX;
-    for (int i = 0; i < kRateSteps; i++) best = std::min(best, pred[i]);
-    set_error(kErrBufferSize, "no quality fits " + std::to_string(max_bytes) + " bytes: the smallest predicted size is " +
-                                  (best == UINT64_MAX ? std::string("unbounded (the reference aborts at every step)")
-                                                      : std::to_string(best) + " bytes"));
-}
-
 bool encode_flags_ok(uint32_t flags) {
     if (flags & ~(uint32_t)ALICE_ENCODE_WELL_FORMED_TABLES) { set_error(kErrDimensions, "unknown encode flag"); return false; }
     return true;
 }
+
+// alice_codec_psnr's closed form (metrics.rs:16-63) of an exact sum of squared differences over len bytes
+double psnr_of_sse(uint64_t sse, uint64_t len) {
+    if (len == 0) return INFINITY;
+    const double mse = (double)sse / (double)len;
+    return mse == 0.0 ? INFINITY : 10.0 * log10(255.0 * 255.0 / mse);
+}
+
+// What a rate-controlled encode aims for, and one chunk's curve once run: a byte budget (the highest quality whose .alc
+// fits max_bytes, from the predicted sizes) or a PSNR floor (the lowest quality whose decode reaches min_db, from the
+// exact PSNRs of the well-formed encodes).  Neither curve is assumed monotone in the step.
+struct Target {
+    bool psnr;                      // a PSNR floor; false: a byte budget
+    uint64_t max_bytes = 0;
+    uint32_t flags = 0;             // a byte budget's encode flags
+    double min_db = 0;
+    uint64_t curve[kRateSteps];     // by step - 1: predicted .alc sizes, or sums of squared differences ...
+    double db[kRateSteps];          // ... and their PSNRs
+
+    Target(uint64_t max_bytes, uint32_t flags) : psnr(false), max_bytes(max_bytes), flags(flags) {}
+    explicit Target(double min_db) : psnr(true), min_db(min_db) {}
+    // the target's own input checks: error code (set), or kOk
+    int check() const {
+        if (!psnr && !encode_flags_ok(flags)) return kErrDimensions;
+        if (psnr && std::isnan(min_db)) { set_error(kErrQuantStep, "the PSNR target is NaN"); return kErrQuantStep; }
+        return kOk;
+    }
+    // whether the encodes, and so the engine, use well-formed tables (the PSNR curve describes those encodes only)
+    bool well_formed() const { return psnr || (flags & ALICE_ENCODE_WELL_FORMED_TABLES); }
+    // the curve of the RGB at d_rgb on engine slot `slot` (Engine::rate_curve's slot and d_work rules)
+    int run(Engine *e, uint8_t wavelet, const uint8_t *d_rgb, uint32_t slot, uint8_t *d_work, uint32_t *hist_out = nullptr) {
+        if (!psnr) return e->rate_curve(wavelet, d_rgb, curve, hist_out, slot, d_work);
+        const int rc = e->psnr_curve(wavelet, d_rgb, curve, slot, d_work);
+        if (rc) return rc;
+        for (int i = 0; i < kRateSteps; i++) db[i] = psnr_of_sse(curve[i], e->dims().n_pixels * 3);
+        return kOk;
+    }
+    // the curve of the empty chunk (three default headers, decoded exactly) at every step
+    void set_empty() {
+        for (int i = 0; i < kRateSteps; i++) {
+            curve[i] = psnr ? 0 : kAlcHeaderBytes;
+            db[i] = INFINITY;
+        }
+    }
+    bool meets(int s) const {
+        return psnr ? db[s - 1] >= min_db : curve[s - 1] != UINT64_MAX && curve[s - 1] <= max_bytes;
+    }
+    // The next step after `after` (0: the first) in preference order that meets the target, 0 if none.  A byte budget
+    // prefers the highest quality (step 1 upward), a PSNR floor the lowest (step 64 downward).
+    int next(int after) const {
+        const int dir = psnr ? -1 : 1;
+        for (int s = after ? after + dir : psnr ? kRateSteps : 1; s >= 1 && s <= kRateSteps; s += dir)
+            if (meets(s)) return s;
+        return 0;
+    }
+    // sets the error of a curve that no step meets, and returns its code
+    int miss() const {
+        if (!psnr) {
+            uint64_t best = UINT64_MAX;
+            for (int i = 0; i < kRateSteps; i++) best = std::min(best, curve[i]);
+            set_error(kErrBufferSize, "no quality fits " + std::to_string(max_bytes) + " bytes: the smallest predicted size is " +
+                                          (best == UINT64_MAX ? std::string("unbounded (the reference aborts at every step)")
+                                                              : std::to_string(best) + " bytes"));
+            return kErrBufferSize;
+        }
+        int best = kRateSteps;
+        for (int s = kRateSteps; s >= 1; s--)
+            if (db[s - 1] > db[best - 1]) best = s;
+        char msg[160];
+        snprintf(msg, sizeof msg, "no quality reaches %.17g dB: the best PSNR is %.17g dB, at quality %d", min_db,
+                 db[best - 1], (int)quality_for_step(best));
+        set_error(kErrQuantStep, msg);
+        return kErrQuantStep;
+    }
+    // Whether the real encode meets the target (the error is set if not).  A PSNR curve is exact; a predicted size bounds
+    // the real one, so an encode larger than its prediction is not expected either.
+    bool accepts(const Chunk &c) const {
+        if (psnr || kAlcHeaderBytes + c.data.size() <= max_bytes) return true;
+        set_error(kErrBufferSize, "no quality fits " + std::to_string(max_bytes) + " bytes");
+        return false;
+    }
+};
 
 // The input of a curve on a pooled engine: RGB on the device (the engine's stream waits for the work enqueued on
 // user_st), or host RGB copied to the engine's stage 0.  Null (error set) on failure.
@@ -231,143 +297,86 @@ const uint8_t *curve_input(Engine *e, const uint8_t *rgb, bool device, uint64_t 
     return rgb;
 }
 
-// Predicted .alc size of every step for one chunk whose RGB is on the host (device == false) or the device.
-int rate_curve_impl(uint8_t wavelet, const uint8_t *rgb, bool device, uint64_t rgb_len, uint32_t w, uint32_t h,
-                    uint32_t f, uint64_t *bytes64, uint32_t *hist_out, cudaStream_t user_st, uint32_t flags) {
-    set_error(0, "");
-    if (!bytes64) { set_error(kErrNull, "null output"); return kErrNull; }
+// The checks every target call makes after its null checks, then t's curve of one chunk whose RGB is on the host
+// (device == false) or the device.  kOk: *e is the pooled engine that ran the curve on its input *src (release it), or
+// null for the empty chunk, whose curve t then holds.  Otherwise the error code, and no engine is held.
+int run_curve(Target &t, uint8_t wavelet, const uint8_t *rgb, bool device, uint64_t rgb_len, uint32_t w, uint32_t h,
+              uint32_t f, uint32_t *hist_out, cudaStream_t user_st, Engine **e, const uint8_t **src) {
+    *e = nullptr;
     if (wavelet > 2) { set_error(kErrBitstream, "unknown wavelet type byte"); return kErrBitstream; }
-    if (!encode_flags_ok(flags)) return kErrDimensions;
+    int rc = t.check();
+    if (rc) return rc;
     Dims d;
     bool empty;
-    int rc = validate_encode(rgb_len, w, h, f, d, empty);
+    rc = validate_encode(rgb_len, w, h, f, d, empty);
     if (rc) return rc;
-    if (empty) {   // the empty chunk (three default headers) at every step
-        for (int i = 0; i < kRateSteps; i++) bytes64[i] = kAlcHeaderBytes;
+    if (empty) {
+        t.set_empty();
         if (hist_out) memset(hist_out, 0, (size_t)kRateSteps * 3 * 256 * sizeof(uint32_t));
         return kOk;
     }
     if (!rgb) { set_error(kErrNull, "null argument"); return kErrNull; }
     if (!cuda_ready()) return kErrCuda;
-    Engine *e = acquire_engine(d, (flags & ALICE_ENCODE_WELL_FORMED_TABLES) != 0);
-    if (!e) return kErrCuda;
-    const uint8_t *src = curve_input(e, rgb, device, rgb_len, user_st);
-    rc = src ? e->rate_curve(wavelet, src, bytes64, hist_out) : kErrCuda;
-    release_engine(e);
+    *e = acquire_engine(d, t.well_formed());
+    if (!*e) return kErrCuda;
+    *src = curve_input(*e, rgb, device, rgb_len, user_st);
+    rc = *src ? t.run(*e, wavelet, *src, 0, nullptr, hist_out) : kErrCuda;
+    if (rc) { release_engine(*e); *e = nullptr; }
     return rc;
 }
 
-// The highest quality whose chunk fits max_bytes, trying steps from first_step on: the rate curve picks the step, one
-// real encode checks it (an encode larger than its prediction, which the bound rules out, moves on to the next step).
-EncodedChunk *encode_to_size_impl(uint8_t wavelet, const uint8_t *rgb, uint64_t rgb_len, uint32_t w, uint32_t h,
-                                  uint32_t f, uint64_t max_bytes, int first_step, uint8_t *quality_out, uint32_t flags) {
+// The target's curve for one chunk (device: rgb_len is the shape's).  Outputs: curve_out gets t.curve, psnr_out t.db,
+// hist_out the rate curve's histograms; the one a target kind exists for (psnr_out for a PSNR floor, curve_out for a
+// byte budget) is required.  The target's value is not used.
+int target_curve(Target t, uint8_t wavelet, const uint8_t *rgb, bool device, uint64_t rgb_len, uint32_t w, uint32_t h,
+                 uint32_t f, uint64_t *curve_out, double *psnr_out, uint32_t *hist_out, cudaStream_t user_st) {
+    if (device) {
+        const unsigned __int128 len = (unsigned __int128)w * h * f * 3;
+        if (len > (unsigned __int128)UINT64_MAX) { set_error(kErrOverflow, "dimensions overflow usize"); return kErrOverflow; }
+        rgb_len = (uint64_t)len;
+    }
+    set_error(0, "");
+    if (t.psnr ? !psnr_out : !curve_out) { set_error(kErrNull, "null output"); return kErrNull; }
+    Engine *e;
+    const uint8_t *src;
+    const int rc = run_curve(t, wavelet, rgb, device, rgb_len, w, h, f, hist_out, user_st, &e, &src);
+    if (rc) return rc;
+    if (e) release_engine(e);
+    if (curve_out) memcpy(curve_out, t.curve, sizeof t.curve);
+    if (psnr_out) memcpy(psnr_out, t.db, sizeof t.db);
+    return kOk;
+}
+
+// The chunk at the target's preferred step after `after` (0: from the first) whose real encode the target accepts:
+// the curve picks the step, one encode at its quality checks it, and an encode the target rejects moves on to the next
+// step that meets it.  The empty chunk is three default headers at the step its curve picks.
+EncodedChunk *encode_to_target(Target &t, uint8_t wavelet, const uint8_t *rgb, uint64_t rgb_len, uint32_t w, uint32_t h,
+                               uint32_t f, int after, uint8_t *quality_out) {
     set_error(0, "");
     if (!rgb || !quality_out) { set_error(kErrNull, "null argument"); return nullptr; }
-    if (wavelet > 2) { set_error(kErrBitstream, "unknown wavelet type byte"); return nullptr; }
-    if (!encode_flags_ok(flags)) return nullptr;
-    Dims d;
-    bool empty;
-    if (validate_encode(rgb_len, w, h, f, d, empty)) return nullptr;
-    if (empty) {
-        uint64_t pred[kRateSteps];
-        for (int i = 0; i < kRateSteps; i++) pred[i] = kAlcHeaderBytes;
-        if (max_bytes < kAlcHeaderBytes) { set_no_fit_error(pred, max_bytes); return nullptr; }
-        EncodedChunk *out = new (std::nothrow) EncodedChunk();
-        if (!out) return nullptr;
+    Engine *e;
+    const uint8_t *stage;
+    if (run_curve(t, wavelet, rgb, false, rgb_len, w, h, f, nullptr, nullptr, &e, &stage)) return nullptr;
+    EncodedChunk *out = nullptr;
+    int step = t.next(after);
+    if (!step) t.miss();
+    for (; step; step = t.next(step)) {
+        out = new (std::nothrow) EncodedChunk();
+        if (!out) break;
         out->c.width = w; out->c.height = h; out->c.frames = f;
         out->c.wavelet = wavelet;
-        *quality_out = 100;
-        return out;
-    }
-    if (!cuda_ready()) return nullptr;
-    Engine *e = acquire_engine(d, (flags & ALICE_ENCODE_WELL_FORMED_TABLES) != 0);
-    if (!e) return nullptr;
-    EncodedChunk *out = nullptr;
-    do {
-        const uint8_t *stage = stage_host_chunk(e, rgb, rgb_len);
-        if (!stage) break;
-        uint64_t pred[kRateSteps];
-        if (e->rate_curve(wavelet, stage, pred, nullptr)) break;
-        const uint8_t *ptrs[1] = {stage};
-        int step = pick_step(pred, max_bytes, first_step);
-        if (!step) { set_no_fit_error(pred, max_bytes); break; }
-        for (; step; step = pick_step(pred, max_bytes, step + 1)) {
-            out = new (std::nothrow) EncodedChunk();
-            if (!out) break;
-            if (e->encode_device(quality_for_step(step), wavelet, ptrs, 1, nullptr) || e->fetch_chunk(0, out->c)) {
-                delete out; out = nullptr;
-                break;
-            }
-            if (kAlcHeaderBytes + out->c.data.size() <= max_bytes) {
-                *quality_out = quality_for_step(step);
-                break;
-            }
+        if (e && (e->encode_device(quality_for_step(step), wavelet, &stage, 1, nullptr) || e->fetch_chunk(0, out->c))) {
             delete out; out = nullptr;
-            set_error(kErrBufferSize, "no quality fits " + std::to_string(max_bytes) + " bytes");
+            break;
         }
-    } while (0);
-    release_engine(e);
-    return out;
-}
-
-// ------------------------------------------------------------------------------ PSNR targets
-// alice_codec_psnr's closed form (metrics.rs:16-63) of an exact sum of squared differences over len bytes
-double psnr_of_sse(uint64_t sse, uint64_t len) {
-    if (len == 0) return INFINITY;
-    const double mse = (double)sse / (double)len;
-    return mse == 0.0 ? INFINITY : 10.0 * log10(255.0 * 255.0 / mse);
-}
-
-// the largest step whose PSNR reaches min_psnr_db (the lowest quality; PSNR is not monotone in the step), 0 if none
-int pick_psnr_step(const double psnr[kRateSteps], double min_psnr_db) {
-    for (int s = kRateSteps; s >= 1; s--)
-        if (psnr[s - 1] >= min_psnr_db) return s;
-    return 0;
-}
-
-void set_no_psnr_error(const double psnr[kRateSteps], double min_psnr_db) {
-    int best = kRateSteps;
-    for (int s = kRateSteps; s >= 1; s--)
-        if (psnr[s - 1] > psnr[best - 1]) best = s;
-    char msg[160];
-    snprintf(msg, sizeof msg, "no quality reaches %.17g dB: the best PSNR is %.17g dB, at quality %d", min_psnr_db,
-             psnr[best - 1], (int)quality_for_step(best));
-    set_error(kErrQuantStep, msg);
-}
-
-bool psnr_target_ok(double min_psnr_db) {
-    if (std::isnan(min_psnr_db)) { set_error(kErrQuantStep, "the PSNR target is NaN"); return false; }
-    return true;
-}
-
-void psnr_from_sse(const uint64_t sse[kRateSteps], uint64_t len, double *psnr64, uint64_t *sse64) {
-    for (int i = 0; i < kRateSteps; i++) {
-        psnr64[i] = psnr_of_sse(sse[i], len);
-        if (sse64) sse64[i] = sse[i];
+        if (t.accepts(out->c)) {
+            *quality_out = quality_for_step(step);
+            break;
+        }
+        delete out; out = nullptr;
     }
-}
-
-// PSNR of the well-formed encode at every step for one chunk whose RGB is on the host (device == false) or the device.
-int psnr_curve_impl(uint8_t wavelet, const uint8_t *rgb, bool device, uint64_t rgb_len, uint32_t w, uint32_t h,
-                    uint32_t f, double *psnr64, uint64_t *sse64, cudaStream_t user_st) {
-    set_error(0, "");
-    if (!psnr64) { set_error(kErrNull, "null output"); return kErrNull; }
-    if (wavelet > 2) { set_error(kErrBitstream, "unknown wavelet type byte"); return kErrBitstream; }
-    Dims d;
-    bool empty;
-    int rc = validate_encode(rgb_len, w, h, f, d, empty);
-    if (rc) return rc;
-    uint64_t sse[kRateSteps] = {0};
-    if (empty) { psnr_from_sse(sse, 0, psnr64, sse64); return kOk; }
-    if (!rgb) { set_error(kErrNull, "null argument"); return kErrNull; }
-    if (!cuda_ready()) return kErrCuda;
-    Engine *e = acquire_engine(d, true);
-    if (!e) return kErrCuda;
-    const uint8_t *src = curve_input(e, rgb, device, rgb_len, user_st);
-    rc = src ? e->psnr_curve(wavelet, src, sse) : kErrCuda;
-    release_engine(e);
-    if (!rc) psnr_from_sse(sse, d.n_pixels * 3, psnr64, sse64);
-    return rc;
+    if (e) release_engine(e);
+    return out;
 }
 
 uint8_t *decode_impl(const EncodedChunk *chunk, uint64_t *out_len, uint8_t *symbols_out) {
@@ -1173,6 +1182,54 @@ int fetch_new_chunks(Engine *e, uint32_t n, EncodedChunk **out_chunks) {
         for (uint32_t k = 0; k < n; k++) { delete out_chunks[k]; out_chunks[k] = nullptr; }
     return rc;
 }
+
+// Per chunk, in stream order as alice_codec_batch_encode_host stages it: copy, curve, one host read of 64 values, the
+// front-end at the chosen step; then one table build and one rANS launch for the whole batch.  A chunk whose encode the
+// target rejects is encoded again on its own, from the next step on.
+int batch_encode_to_target(AliceBatch *b, Target &t, const uint8_t *const *h_rgb, uint32_t n, EncodedChunk **out_chunks,
+                           uint8_t *qualities_out) {
+    set_error(0, "");
+    if (!b || !h_rgb || !out_chunks || !qualities_out) { set_error(kErrNull, "null argument"); return kErrNull; }
+    Engine *e = b->eng;
+    if (t.well_formed() && !e->well_formed_tables()) { set_error(kErrDimensions, "batch was not created with ALICE_BATCH_WELL_FORMED_TABLES"); return kErrDimensions; }
+    int rc = t.check();
+    if (rc) return rc;
+    if (n > e->cap_chunks()) { set_error(kErrBufferSize, "batch larger than capacity"); return kErrBufferSize; }
+    const Dims &d = e->dims();
+    const size_t bytes = (size_t)d.n_pixels * 3;
+    std::vector<int> steps(n);
+    rc = e->encode_begin(100, b->wavelet);    // the batch's quality is not used: every chunk names its step
+    for (uint32_t i = 0; i < n && !rc; i++) {
+        if (!h_rgb[i]) { set_error(kErrNull, "null chunk pointer"); return kErrNull; }
+        uint8_t *s, *work;
+        if (!host_stage(e, i, s, work)) return kErrCuda;
+        CU_CHECK_RC(cudaMemcpyAsync(s, h_rgb[i], bytes, cudaMemcpyHostToDevice, e->stream()));
+        rc = t.run(e, b->wavelet, s, i, work);
+        if (rc) return rc;
+        steps[i] = t.next(0);
+        if (!steps[i]) {
+            rc = t.miss();
+            set_error(rc, "chunk " + std::to_string(i) + ": " + last_error_msg());
+            return rc;
+        }
+        rc = e->encode_submit(i, s, work, steps[i]);
+    }
+    if (!rc) rc = e->encode_finish(n);
+    if (!rc) rc = fetch_new_chunks(e, n, out_chunks);
+    if (rc) return rc;
+    for (uint32_t i = 0; i < n && !rc; i++) {
+        qualities_out[i] = quality_for_step(steps[i]);
+        if (t.accepts(out_chunks[i]->c)) continue;
+        delete out_chunks[i];
+        out_chunks[i] = encode_to_target(t, b->wavelet, h_rgb[i], bytes, d.w, d.h, d.f, steps[i], &qualities_out[i]);
+        if (!out_chunks[i]) rc = last_error_code() ? last_error_code() : kErrCuda;
+    }
+    if (rc) {
+        for (uint32_t k = 0; k < n; k++) { delete out_chunks[k]; out_chunks[k] = nullptr; }
+        return rc;
+    }
+    return kOk;
+}
 }  // namespace
 
 AliceBatch *alice_codec_batch_create(uint8_t quality, uint8_t wavelet, uint32_t w, uint32_t h, uint32_t f,
@@ -1343,14 +1400,15 @@ int alice_codec_batch_timings(AliceBatch *b, float *ms8) {
 }
 uint64_t alice_codec_batch_device_bytes(const AliceBatch *b) { return b ? b->eng->device_bytes() : 0; }
 
-// ------------------------------------------------------------------------------ rate control
+// ------------------------------------------------------------------------------ quality targets
 int alice_codec_rate_curve(uint8_t wavelet, const uint8_t *rgb, uint64_t rgb_len, uint32_t width, uint32_t height,
                            uint32_t frames, uint64_t *bytes64, uint32_t *hist_out) {
     return alice_codec_rate_curve_ex(wavelet, rgb, rgb_len, width, height, frames, bytes64, hist_out, 0);
 }
 int alice_codec_rate_curve_ex(uint8_t wavelet, const uint8_t *rgb, uint64_t rgb_len, uint32_t width, uint32_t height,
                               uint32_t frames, uint64_t *bytes64, uint32_t *hist_out, uint32_t flags) {
-    return rate_curve_impl(wavelet, rgb, false, rgb_len, width, height, frames, bytes64, hist_out, nullptr, flags);
+    return target_curve(Target(0, flags), wavelet, rgb, false, rgb_len, width, height, frames, bytes64,
+                        nullptr, hist_out, nullptr);
 }
 int alice_codec_rate_curve_device(uint8_t wavelet, const uint8_t *d_rgb, uint32_t width, uint32_t height,
                                   uint32_t frames, uint64_t *bytes64, uint32_t *hist_out, void *cuda_stream) {
@@ -1359,10 +1417,8 @@ int alice_codec_rate_curve_device(uint8_t wavelet, const uint8_t *d_rgb, uint32_
 int alice_codec_rate_curve_device_ex(uint8_t wavelet, const uint8_t *d_rgb, uint32_t width, uint32_t height,
                                      uint32_t frames, uint64_t *bytes64, uint32_t *hist_out, void *cuda_stream,
                                      uint32_t flags) {
-    const unsigned __int128 len = (unsigned __int128)width * height * frames * 3;
-    if (len > (unsigned __int128)UINT64_MAX) { set_error(kErrOverflow, "dimensions overflow usize"); return kErrOverflow; }
-    return rate_curve_impl(wavelet, d_rgb, true, (uint64_t)len, width, height, frames, bytes64, hist_out,
-                           (cudaStream_t)cuda_stream, flags);
+    return target_curve(Target(0, flags), wavelet, d_rgb, true, 0, width, height, frames, bytes64, nullptr,
+                        hist_out, (cudaStream_t)cuda_stream);
 }
 EncodedChunk *alice_codec_encode_to_size(uint8_t wavelet, const uint8_t *rgb, uint64_t rgb_len, uint32_t width,
                                          uint32_t height, uint32_t frames, uint64_t max_bytes, uint8_t *quality_out) {
@@ -1371,147 +1427,34 @@ EncodedChunk *alice_codec_encode_to_size(uint8_t wavelet, const uint8_t *rgb, ui
 EncodedChunk *alice_codec_encode_to_size_ex(uint8_t wavelet, const uint8_t *rgb, uint64_t rgb_len, uint32_t width,
                                             uint32_t height, uint32_t frames, uint64_t max_bytes, uint8_t *quality_out,
                                             uint32_t flags) {
-    return encode_to_size_impl(wavelet, rgb, rgb_len, width, height, frames, max_bytes, 1, quality_out, flags);
+    Target t(max_bytes, flags);
+    return encode_to_target(t, wavelet, rgb, rgb_len, width, height, frames, 0, quality_out);
 }
-// Per chunk, in stream order as alice_codec_batch_encode_host stages it: copy, rate curve, one host read of 64 sizes, the
-// front-end at the chosen step; then one table build and one rANS launch for the whole batch.
 int alice_codec_batch_encode_host_to_size(AliceBatch *b, const uint8_t *const *h_rgb, uint32_t n, uint64_t max_bytes,
                                           EncodedChunk **out_chunks, uint8_t *qualities_out) {
-    set_error(0, "");
-    if (!b || !h_rgb || !out_chunks || !qualities_out) { set_error(kErrNull, "null argument"); return kErrNull; }
-    Engine *e = b->eng;
-    if (n > e->cap_chunks()) { set_error(kErrBufferSize, "batch larger than capacity"); return kErrBufferSize; }
-    const Dims &d = e->dims();
-    const size_t bytes = (size_t)d.n_pixels * 3;
-    std::vector<int> steps(n);
-    int rc = e->encode_begin(100, b->wavelet);    // the batch's quality is not used: every chunk names its step
-    for (uint32_t i = 0; i < n && !rc; i++) {
-        if (!h_rgb[i]) { set_error(kErrNull, "null chunk pointer"); return kErrNull; }
-        uint8_t *s, *work;
-        if (!host_stage(e, i, s, work)) return kErrCuda;
-        CU_CHECK_RC(cudaMemcpyAsync(s, h_rgb[i], bytes, cudaMemcpyHostToDevice, e->stream()));
-        uint64_t pred[kRateSteps];
-        rc = e->rate_curve(b->wavelet, s, pred, nullptr, i, work);
-        if (rc) return rc;
-        steps[i] = pick_step(pred, max_bytes, 1);
-        if (!steps[i]) {
-            set_no_fit_error(pred, max_bytes);
-            set_error(kErrBufferSize, "chunk " + std::to_string(i) + ": " + last_error_msg());
-            return kErrBufferSize;
-        }
-        rc = e->encode_submit(i, s, work, steps[i]);
-    }
-    if (!rc) rc = e->encode_finish(n);
-    if (!rc) rc = fetch_new_chunks(e, n, out_chunks);
-    if (rc) return rc;
-    for (uint32_t i = 0; i < n && !rc; i++) {
-        qualities_out[i] = quality_for_step(steps[i]);
-        if (kAlcHeaderBytes + out_chunks[i]->c.data.size() <= max_bytes) continue;
-        // larger than its prediction (the bound rules this out): this chunk alone, from the next step on
-        delete out_chunks[i];
-        out_chunks[i] = encode_to_size_impl(b->wavelet, h_rgb[i], bytes, d.w, d.h, d.f, max_bytes, steps[i] + 1,
-                                            &qualities_out[i],
-                                            e->well_formed_tables() ? (uint32_t)ALICE_ENCODE_WELL_FORMED_TABLES : 0u);
-        if (!out_chunks[i]) rc = last_error_code() ? last_error_code() : kErrCuda;
-    }
-    if (rc) {
-        for (uint32_t k = 0; k < n; k++) { delete out_chunks[k]; out_chunks[k] = nullptr; }
-        return rc;
-    }
-    return kOk;
+    // the encodes use the batch's table mode
+    Target t(max_bytes, b && b->eng->well_formed_tables() ? (uint32_t)ALICE_ENCODE_WELL_FORMED_TABLES : 0u);
+    return batch_encode_to_target(b, t, h_rgb, n, out_chunks, qualities_out);
 }
-
-// ------------------------------------------------------------------------------ PSNR targets
 int alice_codec_psnr_curve(uint8_t wavelet, const uint8_t *rgb, uint64_t rgb_len, uint32_t width, uint32_t height,
                            uint32_t frames, double *psnr64, uint64_t *sse64) {
-    return psnr_curve_impl(wavelet, rgb, false, rgb_len, width, height, frames, psnr64, sse64, nullptr);
+    return target_curve(Target(0.0), wavelet, rgb, false, rgb_len, width, height, frames, sse64, psnr64,
+                        nullptr, nullptr);
 }
 int alice_codec_psnr_curve_device(uint8_t wavelet, const uint8_t *d_rgb, uint32_t width, uint32_t height,
                                   uint32_t frames, double *psnr64, uint64_t *sse64, void *cuda_stream) {
-    const unsigned __int128 len = (unsigned __int128)width * height * frames * 3;
-    if (len > (unsigned __int128)UINT64_MAX) { set_error(kErrOverflow, "dimensions overflow usize"); return kErrOverflow; }
-    return psnr_curve_impl(wavelet, d_rgb, true, (uint64_t)len, width, height, frames, psnr64, sse64,
-                           (cudaStream_t)cuda_stream);
+    return target_curve(Target(0.0), wavelet, d_rgb, true, 0, width, height, frames, sse64, psnr64, nullptr,
+                        (cudaStream_t)cuda_stream);
 }
-// The PSNR curve picks the step, one well-formed encode at it follows: the curve is exact, so nothing is checked after.
 EncodedChunk *alice_codec_encode_to_psnr(uint8_t wavelet, const uint8_t *rgb, uint64_t rgb_len, uint32_t width,
                                          uint32_t height, uint32_t frames, double min_psnr_db, uint8_t *quality_out) {
-    set_error(0, "");
-    if (!rgb || !quality_out) { set_error(kErrNull, "null argument"); return nullptr; }
-    if (wavelet > 2) { set_error(kErrBitstream, "unknown wavelet type byte"); return nullptr; }
-    if (!psnr_target_ok(min_psnr_db)) return nullptr;
-    Dims d;
-    bool empty;
-    if (validate_encode(rgb_len, width, height, frames, d, empty)) return nullptr;
-    if (empty) {   // +inf at every step: the largest one
-        EncodedChunk *out = new (std::nothrow) EncodedChunk();
-        if (!out) return nullptr;
-        out->c.width = width; out->c.height = height; out->c.frames = frames;
-        out->c.wavelet = wavelet;
-        *quality_out = quality_for_step(kRateSteps);
-        return out;
-    }
-    if (!cuda_ready()) return nullptr;
-    Engine *e = acquire_engine(d, true);
-    if (!e) return nullptr;
-    EncodedChunk *out = nullptr;
-    do {
-        const uint8_t *stage = stage_host_chunk(e, rgb, rgb_len);
-        if (!stage) break;
-        uint64_t sse[kRateSteps];
-        double psnr[kRateSteps];
-        if (e->psnr_curve(wavelet, stage, sse)) break;
-        psnr_from_sse(sse, d.n_pixels * 3, psnr, nullptr);
-        const int step = pick_psnr_step(psnr, min_psnr_db);
-        if (!step) { set_no_psnr_error(psnr, min_psnr_db); break; }
-        out = new (std::nothrow) EncodedChunk();
-        if (!out) break;
-        const uint8_t *ptrs[1] = {stage};
-        if (e->encode_device(quality_for_step(step), wavelet, ptrs, 1, nullptr) || e->fetch_chunk(0, out->c)) {
-            delete out; out = nullptr;
-            break;
-        }
-        *quality_out = quality_for_step(step);
-    } while (0);
-    release_engine(e);
-    return out;
+    Target t(min_psnr_db);
+    return encode_to_target(t, wavelet, rgb, rgb_len, width, height, frames, 0, quality_out);
 }
-// Per chunk, in stream order as alice_codec_batch_encode_host stages it: copy, PSNR curve, one host read of 64 sums, the
-// front-end at the chosen step; then one table build and one rANS launch for the whole batch.
 int alice_codec_batch_encode_host_to_psnr(AliceBatch *b, const uint8_t *const *h_rgb, uint32_t n, double min_psnr_db,
                                           EncodedChunk **out_chunks, uint8_t *qualities_out) {
-    set_error(0, "");
-    if (!b || !h_rgb || !out_chunks || !qualities_out) { set_error(kErrNull, "null argument"); return kErrNull; }
-    Engine *e = b->eng;
-    if (!e->well_formed_tables()) { set_error(kErrDimensions, "batch was not created with ALICE_BATCH_WELL_FORMED_TABLES"); return kErrDimensions; }
-    if (!psnr_target_ok(min_psnr_db)) return kErrQuantStep;
-    if (n > e->cap_chunks()) { set_error(kErrBufferSize, "batch larger than capacity"); return kErrBufferSize; }
-    const size_t bytes = (size_t)e->dims().n_pixels * 3;
-    std::vector<int> steps(n);
-    int rc = e->encode_begin(100, b->wavelet);    // the batch's quality is not used: every chunk names its step
-    for (uint32_t i = 0; i < n && !rc; i++) {
-        if (!h_rgb[i]) { set_error(kErrNull, "null chunk pointer"); return kErrNull; }
-        uint8_t *s, *work;
-        if (!host_stage(e, i, s, work)) return kErrCuda;
-        CU_CHECK_RC(cudaMemcpyAsync(s, h_rgb[i], bytes, cudaMemcpyHostToDevice, e->stream()));
-        uint64_t sse[kRateSteps];
-        double psnr[kRateSteps];
-        rc = e->psnr_curve(b->wavelet, s, sse, i, work);
-        if (rc) return rc;
-        psnr_from_sse(sse, bytes, psnr, nullptr);
-        steps[i] = pick_psnr_step(psnr, min_psnr_db);
-        if (!steps[i]) {
-            set_no_psnr_error(psnr, min_psnr_db);
-            set_error(kErrQuantStep, "chunk " + std::to_string(i) + ": " + last_error_msg());
-            return kErrQuantStep;
-        }
-        rc = e->encode_submit(i, s, work, steps[i]);
-    }
-    if (!rc) rc = e->encode_finish(n);
-    if (!rc) rc = fetch_new_chunks(e, n, out_chunks);
-    if (rc) return rc;
-    for (uint32_t i = 0; i < n; i++) qualities_out[i] = quality_for_step(steps[i]);
-    return kOk;
+    Target t(min_psnr_db);
+    return batch_encode_to_target(b, t, h_rgb, n, out_chunks, qualities_out);
 }
 
 int alice_codec_synth_rgb_device(int kind, uint32_t seed, uint32_t w, uint32_t h, uint32_t f, uint8_t *d_rgb,
